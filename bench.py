@@ -4,6 +4,7 @@ reference's nets on synthetic data of the datasets' shapes.
 
   python bench.py --gpus N --steps K --warmup W [--config C] [--batch B] [--precision bf16|fp32]
   python bench.py --impl reference ...      # CPU arm: the oracle port of the reference on the host cores
+  python bench.py ... --dump-outputs DIR    # also write what the last timed step computed, DIR/<name>.npy
 
 Headline workload = `cifar10-ac` (ac_chain, /root/reference/scripts/arch_and_hypers.py:76-139, experiment
 table scripts/train-nets:84-87) at --batch per GPU (default 4096; the reference trains at 128, reported in
@@ -185,7 +186,7 @@ def run_reference(args, rank, world, emit):
         return
     torch.set_num_threads(os.cpu_count() or 1)
     cfg = _configs()[args.config]
-    B, steps, warm = args.batch, max(1, args.steps), max(0, args.warmup)
+    B, steps, warm = args.batch, args.steps, max(0, args.warmup)
     o = _oracle(args.config)
     rng = np.random.default_rng(0)
     probe_B = min(B, 256)
@@ -240,6 +241,8 @@ class Run:
         self.kcs = [rng.choice(ah.k_cpts, B).astype(np.float32) for _ in range(4)] if self.cfg.get('dyn') else None
         self.plan = self.eng._plan(B, True, True)
         self.flop = train_flop_per_img(self.net)
+        # parameters, momentum and layer state as initialised (seeded): the last device-timed step starts from them
+        self.init = [t.clone() for t in (self.eng.theta, self.eng.accum, self.eng.state)]
 
     def feed(self, t):
         net = self.net
@@ -267,13 +270,22 @@ class Run:
         return float(tt.item())
 
     def device_timed(self, steps, warmup, flush):
-        """K steps with the batch resident in HBM, one CUDA event pair per step, L2 flushed in between"""
+        """K steps with the batch resident in HBM, one CUDA event pair per step, L2 flushed in between.  The last
+        step starts again from the initial parameters: the step's fp32 weight-gradient sums are unordered, so two
+        runs differ in the last bits, and consecutive steps on one batch amplify that to percents within 25 steps.
+        Restarting the last step from the seeded state keeps what it computes (--dump-outputs) reproducible to those
+        last bits; it runs the same kernels on the same shapes as the others.  The K end-to-end steps that follow
+        (e2e_timed, whose mean objective is the line's `loss`) therefore continue from the initial parameters plus
+        one step, not plus the warm-up and K steps."""
         eng, plan = self.eng, self.plan
         ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
         eng._feed(plan, self.feed(warmup), True)
         self.barrier()
         l0 = eng.L.launches
         for t in range(steps):
+            if t == steps - 1:
+                for buf, init in zip((eng.theta, eng.accum, eng.state), self.init):
+                    buf.copy_(init)
             flush.zero_()                                  # evict L2 between timed iterations
             ev[t][0].record()
             eng.run_resident(plan, True)
@@ -313,6 +325,41 @@ class Run:
             'tensor_frac_of_step': value / self.world * self.flop / (pk['bf16_tflops_sustained'] * 1e12),
             'hbm_frac_of_step': (self.hbm_bytes_per_step() / (pk['hbm_gbs'] * 1e9)) / (ms / steps * 1e-3),
             'loss': loss}
+
+
+DUMP_BYTES = 60 << 20          # leaves room for the .npy headers under 64 MB
+
+
+def dump_outputs(run, out_dir):
+    """What the last device-timed step (one training step from the initial parameters on the resident batch) left
+    for a caller, one float32 DIR/<name>.npy each: the updated parameters (`theta`), momentum and layer state, the
+    step's gradient buffer ([per-node TALR moments | gradients]), every leaf's logits / per-example error /
+    correctness and, for routed nets, the routing weights `p_tr`, decisions `p_ev` (nodes x batch) and per-example
+    objective `c_data`.  The inputs are seeded, so two builds run with the same arguments can be compared array for
+    array.  A batch whose arrays would pass 64 MB in all is cut to a fixed, seeded sample of examples (their indices
+    in `examples.npy`)."""
+    eng, plan = run.eng, run.plan
+    whole = {'theta': eng.theta, 'momentum': eng.accum, 'grad': eng.grad, 'state': eng.state[:eng.n_state]}
+    per_ex = {}                                   # name -> (tensor, batch axis)
+    for k, nd in enumerate(eng.regs):
+        r = plan.reg[nd.idx]
+        per_ex.update({'leaf%d_logits' % k: (r.Z, 0), 'leaf%d_c_err' % k: (r.c_err, 0), 'leaf%d_d_cor' % k: (r.d_cor, 0)})
+    if eng.dynamic:
+        per_ex.update(p_tr=(plan.p_tr, 1), p_ev=(plan.p_ev, 1), c_data=(plan.c_data, 0))
+    out = {k: t.detach().float().cpu().numpy() for k, t in whole.items()}
+    per_ex = {k: (t.detach().float().cpu().numpy(), ax) for k, (t, ax) in per_ex.items()}
+    B = plan.B
+    fixed = sum(a.nbytes for a in out.values())
+    per_example = sum(a.nbytes for a, _ in per_ex.values()) / B
+    keep = int((DUMP_BYTES - fixed - 8 * B) // per_example) if per_example else B
+    if keep < B:
+        idx = np.sort(np.random.default_rng(0).choice(B, max(keep, 1), replace=False))
+        per_ex = {k: (np.take(a, idx, axis=ax), ax) for k, (a, ax) in per_ex.items()}
+        out['examples'] = idx.astype(np.float64)
+    out.update({k: a for k, (a, _) in per_ex.items()})
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + '.npy'), a)
 
 
 def per_launch_profile(run):
@@ -404,7 +451,13 @@ def main():
     ap.add_argument('--no-graphs', action='store_true')
     ap.add_argument('--no-sweep', action='store_true', help='skip the `configs` array (other configs / batches)')
     ap.add_argument('--profile', action='store_true', help='print per-kernel-kind time shares')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step computed as DIR/<name>.npy (float32, at most 64 MB)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of --impl ours')
     # stdout carries exactly ONE JSON line: anything a library prints to fd 1 meanwhile (NCCL's version banner on
     # the first communicator) is sent to stderr, and the real stdout comes back for the final print
     sys.stdout.flush()
@@ -450,6 +503,8 @@ def main():
         clocks.mark = len(clocks.rows)                 # samples from here on fall inside the timed regions
     run.barrier()
     dev_ms, launches = run.device_timed(args.steps, args.warmup, flush)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(run, args.dump_outputs)
     e2e_s, loss = run.e2e_timed(args.steps, args.warmup)
     clk = clocks.stop() if rank == 0 else None
 
