@@ -411,6 +411,20 @@ int mpnn_route_compact(const float* R, int ldr, int ns, int n, const int* parent
  * (p_cor, p_inc, p_cor_by_cls, p_inc_by_cls of train-nets:121-124 summed over the batch; out is double). */
 int mpnn_leaf_stats(const float* Z, int ldz, int n_cls, const float* y, const int* pos, const int* orig,
                     const int* count, int n, double* out, void* stream);
+/* Routed inference: the results of the examples that exit at one classifier.  Rows pos[j] of the logits Z
+ * (row stride ldz) of the parent's compact batch, original ids orig[j], j < *count (count NULL -> j < n;
+ * pos / orig NULL -> identity; the grid covers n, so *count <= n):
+ *   prob[orig[j]][c] = softmax(Z[pos[j]])[c]     (c < n_cls <= 32; the same bits as mpnn_softmax_ce_fwd)
+ *   cls[orig[j]]     = first argmax of that row of prob
+ *   exit_id[orig[j]] = leaf,   ops[orig[j]] = path_ops
+ * n == 0 is a no-op. */
+int mpnn_leaf_emit(const float* Z, int ldz, int n_cls, const int* pos, const int* orig, const int* count, int n,
+                   int leaf, double path_ops, float* prob, int* cls, int* exit_id, double* ops, void* stream);
+/* The per-example router feature through the compaction: dst[j] = src[orig[j]] for j < *count (count NULL ->
+ * j < n; orig NULL -> identity; dst may be NULL), and, when col != NULL, the same value into the strided column
+ * col[j * col_stride] of dtype col_dtype (0 fp32, 1 bf16 rounded to nearest even, like torch's copy_). */
+int mpnn_gather_feature(const float* src, const int* orig, const int* count, int n, float* dst,
+                        void* col, int col_stride, int col_dtype, void* stream);
 
 /* ---- optimiser: minimize_expectation + MomentumOptimizer (lib/net_types.py:24-37) */
 /* For segment s covering theta[seg_start[s] : seg_start[s+1]):

@@ -206,6 +206,50 @@ extern "C" int mpnn_softmax_ce_fwd(const float* Z, int ldz, const float* y, int 
     return mpnn_check_launch("softmax_ce_fwd");
 }
 
+// ------------------------------------------------------ routed inference: results at one classifier
+// The softmax and first argmax of softmax_ce_fwd_kernel (same lane groups, same expressions, so prob is the same
+// bits as the dense path's for the same logits) on rows pos[j] of the parent's compact batch, written at the
+// examples' original ids orig[j].  The live count is read on the device; the grid covers the host bound.
+template <int LPR>
+__global__ void __launch_bounds__(128)
+leaf_emit_kernel(const float* __restrict__ Z, int ldz, int n, const int* __restrict__ pos,
+                 const int* __restrict__ orig, const int* __restrict__ count, int n_max, int leaf, double path_ops,
+                 float* __restrict__ prob, int* __restrict__ cls, int* __restrict__ exit_id, double* __restrict__ ops) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    const int b = t / LPR, j = t % LPR;
+    const int nb = count ? min(*count, n_max) : n_max;
+    const bool live = b < nb;
+    const bool on = live && j < n;
+    const int row = !live ? 0 : pos ? pos[b] : b;
+    const int o = !live ? 0 : orig ? orig[b] : b;
+    const float z = on ? Z[(size_t)row * ldz + j] : -INFINITY;
+    const float mx = grp_max<LPR>(z);
+    const float e = on ? expf(z - mx) : 0.f;
+    const float p = e * (1.f / grp_sum<LPR>(e));
+    if (on) prob[(size_t)o * n + j] = p;
+    const int am = grp_argmax<LPR>(on ? p : -INFINITY, j);
+    if (live && j == 0) {
+        cls[o] = am;
+        exit_id[o] = leaf;
+        ops[o] = path_ops;
+    }
+}
+
+extern "C" int mpnn_leaf_emit(const float* Z, int ldz, int n_cls, const int* pos, const int* orig, const int* count,
+                              int n, int leaf, double path_ops, float* prob, int* cls, int* exit_id, double* ops,
+                              void* stream) {
+    MPNN_REQUIRE(n >= 0 && n_cls >= 1 && n_cls <= CE_NMAX && ldz >= n_cls, "leaf_emit: n=%d n_cls=%d ldz=%d", n, n_cls, ldz);
+    if (n == 0) return MPNN_OK;
+    MPNN_REQUIRE(Z && prob && cls && exit_id && ops, "leaf_emit: NULL operand");
+    if (n_cls <= 16)
+        leaf_emit_kernel<16><<<ceil_div(n, 128 / 16), 128, 0, (cudaStream_t)stream>>>(
+            Z, ldz, n_cls, pos, orig, count, n, leaf, path_ops, prob, cls, exit_id, ops);
+    else
+        leaf_emit_kernel<32><<<ceil_div(n, 128 / 32), 128, 0, (cudaStream_t)stream>>>(
+            Z, ldz, n_cls, pos, orig, count, n, leaf, path_ops, prob, cls, exit_id, ops);
+    return mpnn_check_launch("leaf_emit");
+}
+
 // dZ in fp32 [B][n] and/or as two bf16 planes [2][Balloc][8] (columns >= n zero) for the
 // tcgen05 head GEMMs; dbias += column sums of dZ.  squared: the error layer is SquaredError on x = prob.
 template <int LPR>

@@ -599,6 +599,37 @@ extern "C" int mpnn_scatter_add_images(const void* src, int Bs, int Ps, const in
     return move_images<true>(src, Bs, Ps, idx, count, dst, Bd, Pd, C, H, W, G, dtype, stream);
 }
 
+// The per-example router feature alpha_cpt * k_cpt of the examples at one node of the compacted walk, in the
+// node's compact order: into the fp32 `extra` vector of the CUDA-core heads and / or into the feature column of
+// the tcgen05 heads (bf16 with round-to-nearest-even, the rounding of torch's fp32 -> bf16 copy_).
+__global__ void __launch_bounds__(256)
+gather_feature_kernel(const float* __restrict__ src, const int* __restrict__ orig, const int* __restrict__ count,
+                      int n_max, float* __restrict__ dst, void* __restrict__ col, int col_stride, int col_dtype) {
+    const int n = count ? min(*count, n_max) : n_max;
+    for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < n; j += gridDim.x * blockDim.x) {
+        const float v = src[orig ? orig[j] : j];
+        if (dst) dst[j] = v;
+        if (col) {
+            if (col_dtype == MPNN_BF16)
+                static_cast<__nv_bfloat16*>(col)[(size_t)j * col_stride] = __float2bfloat16_rn(v);
+            else
+                static_cast<float*>(col)[(size_t)j * col_stride] = v;
+        }
+    }
+}
+
+extern "C" int mpnn_gather_feature(const float* src, const int* orig, const int* count, int n, float* dst,
+                                   void* col, int col_stride, int col_dtype, void* stream) {
+    MPNN_REQUIRE(n >= 0 && (col == nullptr || (col_stride >= 1 && (col_dtype == MPNN_F32 || col_dtype == MPNN_BF16))),
+                 "gather_feature: n=%d col_stride=%d col_dtype=%d", n, col_stride, col_dtype);
+    if (n == 0 || (dst == nullptr && col == nullptr)) return MPNN_OK;
+    MPNN_REQUIRE(src, "gather_feature: NULL src");
+    int grid = ceil_div(n, 256);
+    if (grid > 148) grid = 148;
+    gather_feature_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(src, orig, count, n, dst, col, col_stride, col_dtype);
+    return mpnn_check_launch("gather_feature");
+}
+
 // ------------------------------------------------ per-switch compaction (compacted ev-mode evaluator)
 // The reference evaluates every node on the whole batch and weights statistics with the one-hot p_ev
 // (net_types.py:127-131, train-nets:117-130); in 'ev' mode an example only needs the nodes on its own

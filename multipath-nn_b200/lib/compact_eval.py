@@ -15,8 +15,14 @@ Exact for every p_ev-weighted statistic -- acc, moc, and per leaf p_cor, p_inc, 
 (what make-acc-eff-plots / make-nlds / make-routing-hists read).  The three entries of `state_tensors` that
 are NOT p_ev-weighted (per-leaf c_err and p_tr, per-switch x_rte; train-nets:125-128) are defined on examples
 a compacted pass never evaluates: they are absent from its result (use the dense `Engine.eval_stats` for them).
+
+The same walk serves routed inference (`predict`, behind `Net.predict`): at a classifier it writes each
+example's softmax, predicted class, exit leaf and path cost (mpnn_leaf_emit) instead of adding statistics.
+Nets with a per-example k_cpt carry the router feature alpha_cpt * k_cpt through the compaction by original
+example id (mpnn_gather_feature), so one batch may mix cost budgets.
 """
 import ctypes
+from types import SimpleNamespace as Ns
 
 import numpy as np
 import torch
@@ -26,21 +32,46 @@ from lib.engine import BF16, _RT_FWD, _ru, _vp
 __all__ = ['CompactEvaluator']
 
 
+def _node_ops(nd):
+    return nd.layer.n_ops + (nd.router.n_ops if nd.router is not None else 0)
+
+
 class CompactEvaluator:
     def __init__(self, eng, batch=4096):
-        if not eng.dynamic:
-            raise ValueError('compacted evaluation is for dynamically-routed nets (an SRNet has one path)')
         if eng.split:
             raise NotImplementedError('compacted evaluation runs in fp32 or bf16 precision (not the split modes bf16x3 / bf16x6)')
         if any(getattr(nd, 'maxpool', False) or getattr(nd, 'gmp', False) for nd in eng.nodes):
             raise NotImplementedError('compacted evaluation does not cover MaxPool / GlobalMaxPool blocks')
         if any(nd.loss != 'ce' for nd in eng.regs):
             raise NotImplementedError('compacted evaluation scores Softmax + CrossEntropyError classifiers only')
+        if any(getattr(nd, 'keep', 1.0) != 1.0 for nd in eng.nodes):
+            # the reference applies Dropout in every mode: an 'ev' pass through it is random, and this walk has no mask
+            raise NotImplementedError('compacted evaluation does not cover Dropout(λ < 1) blocks')
+        root = eng.nodes[0]
+        if root.kind != 'pyr' or getattr(root, 'lln', None) is not None:
+            raise NotImplementedError('compacted evaluation starts from a ToPyramid root without MultiscaleLLN')
         self.eng, self.L, self.B = eng, eng.L, int(batch)
         self.plan = plan = eng._plan(self.B, False, False)      # buffers, packed operands, BN constants
         self.n_cls = eng.net.hypers.y_shape[0]
         B = self.B
         dev = eng.dev
+        self.dyn_k = eng.dynamic and bool(eng.net.hypers.dyn_k_cpt)
+        # alpha_cpt * k_cpt of the chunk's examples by original id (the dense path's plan.kextra)
+        self.kfeat = torch.zeros(B, dtype=torch.float32, device=dev) if self.dyn_k else None
+        # per classifier: its index in `net.leaves` and the ops of the nodes on its root-to-leaf path, summed in node
+        # order like the dense `moc` (Engine.eval_stats) with a one-hot p_ev
+        self.leaf_no = {nd.idx: i for i, nd in enumerate(eng.leaves)}
+        self.path_ops = []
+        for nd in eng.leaves:
+            on_path, i = set(), nd.idx
+            while i is not None:
+                on_path.add(i)
+                i = eng.nodes[i].parent
+            tot = 0.0
+            for i in sorted(on_path):
+                tot += float(_node_ops(eng.nodes[i]))
+            self.path_ops.append(tot)
+        self._emit = None                     # None: the leaves add statistics; else the output arrays of predict
         zi = lambda *shape: torch.zeros(shape, dtype=torch.int32, device=dev)
         self.sw = {}
         for nd in eng.nodes:
@@ -53,8 +84,9 @@ class CompactEvaluator:
                     W2=P(rt.fc2, 'w'), bias2=P(rt.fc2, 'b'), g2=P(rt.bn2, 'γ'), b2=P(rt.bn2, 'β'),
                     m2=P(rt.bn2, 'm_avg'), v2=P(rt.bn2, 'v_avg'), W3=P(rt.fc3, 'w'), bias3=P(rt.fc3, 'b'),
                     Z2=rt.Z2, R=rt.R, save=rt.save, ns=ns)])
+                host = torch.zeros(ns, dtype=torch.int32)
                 self.sw[nd.idx] = dict(tab=tab, pos=zi(ns, B), orig=zi(ns, B), count=zi(ns),
-                                       host=torch.zeros(ns, dtype=torch.int32).pin_memory())
+                                       host=host if eng.dry else host.pin_memory())
         # compacted inputs of every conv stage below a switch: one planes tensor per scale it consumes
         self.cin = {}
         for nd in eng.nodes:
@@ -89,38 +121,93 @@ class CompactEvaluator:
         self._prepared = True
 
     # ------------------------------------------------------------------ #
-    def run_batch(self, x0, y, k_cpt=None):
-        """accumulate the statistics of one batch (n <= batch examples; host or device arrays)"""
+    def _k_feature(self, k_cpt, n):
+        """alpha_cpt * k_cpt per example as fp32 (the dense feed's arithmetic, Engine._feed), or None for nets with
+        a fixed k_cpt; k_cpt is a scalar, one value or n values"""
+        hy = self.eng.net.hypers
+        if not self.dyn_k:
+            if k_cpt is not None:
+                raise ValueError('k_cpt is fed to nets with a per-example k_cpt (dyn_k_cpt) only')
+            return None
+        if k_cpt is None:
+            raise ValueError('this net routes on a per-example k_cpt: pass k_cpt (a scalar, one value or n values)')
+        kc = np.asarray(k_cpt, dtype=np.float32).reshape(-1)
+        if kc.size == 1:
+            kc = np.full(n, kc[0], np.float32)
+        if kc.size != n:
+            raise ValueError('k_cpt: %d values for %d examples' % (kc.size, n))
+        return kc * np.float32(hy.α_cpt)
+
+    def _walk(self, x0, n, kf):
+        """run the chunk x0 (n <= batch examples, host or device) down the tree; kf: its router features or None"""
         eng, plan, L = self.eng, self.plan, self.L
+        hy = eng.net.hypers
+        plan.x0[:n].copy_(eng._to_dev(x0, (n,) + tuple(hy.x0_shape), 'x0'), non_blocking=True)
+        if kf is not None:
+            self.kfeat[:n].copy_(torch.as_tensor(kf), non_blocking=True)
+        root = eng.nodes[0]
+        st = plan.node[0]
+        H0, W0, C0 = hy.x0_shape
+        for i, slot in enumerate(st.out):
+            L.pack_input(_vp(plan.x0), n, H0, W0, C0, 2 ** i, _vp(slot.t), min(slot.C, (C0 + 7) // 8 * 8), slot.geo.G, slot.geo.P,
+                         eng.dtype, self._S())
+        self.visits[0] += n
+        for k in root.kids:
+            self._node(eng.nodes[k], n, None, None, None)
+
+    def run_batch(self, x0, y, k_cpt=None):
+        """accumulate the statistics of one batch (n <= batch examples; host or device arrays).  k_cpt (nets with a
+        per-example k_cpt only): a scalar, one value or one per example."""
+        eng, plan = self.eng, self.plan
+        if not eng.dynamic:
+            raise ValueError('compacted evaluation is for dynamically-routed nets (an SRNet has one path)')
+        n = int(x0.shape[0])
+        if n > self.B:
+            raise ValueError('batch %d > evaluator capacity %d' % (n, self.B))
+        kf = self._k_feature(k_cpt, n)
         with torch.cuda.device(eng.dev):
             if not self._prepared:
                 self._prepare()
-            n = int(x0.shape[0])
-            if n > self.B:
-                raise ValueError('batch %d > evaluator capacity %d' % (n, self.B))
-            hy = eng.net.hypers
-            x0 = eng._to_dev(x0, (n,) + tuple(hy.x0_shape), 'x0')
-            y = eng._to_dev(y, (n,) + tuple(hy.y_shape), 'y')
-            plan.x0[:n].copy_(x0, non_blocking=True)
+            y = eng._to_dev(y, (n,) + tuple(eng.net.hypers.y_shape), 'y')
             plan.y[:n].copy_(y, non_blocking=True)
-            if hy.dyn_k_cpt:
-                kc = np.unique(np.asarray(k_cpt, dtype=np.float32).reshape(-1))
-                if kc.size != 1:
-                    raise NotImplementedError('compacted evaluation needs one k_cpt for the whole batch '
-                                              '(the length-1 feed of train-adaptive-nets:102-105)')
-                plan.kextra.fill_(float(kc[0] * np.float32(hy.α_cpt)))
-                for col in plan.kplanes:
-                    col.fill_(float(kc[0] * np.float32(hy.α_cpt)))
             self.n_seen += n
-            root = eng.nodes[0]
-            st = plan.node[0]
-            H0, W0, C0 = hy.x0_shape
-            for i, slot in enumerate(st.out):
-                L.pack_input(_vp(plan.x0), n, H0, W0, C0, 2 ** i, _vp(slot.t), min(slot.C, (C0 + 7) // 8 * 8), slot.geo.G, slot.geo.P,
-                             eng.dtype, self._S())
-            self.visits[0] += n
-            for k in root.kids:
-                self._node(eng.nodes[k], n, None, None, None)
+            self._walk(x0, n, kf)
+
+    def predict(self, x0, k_cpt=None):
+        """Routed inference (see `Net.predict`): Ns(cls, prob, exit, ops) of numpy arrays, one row per example of x0
+        (any n, host or device), run in chunks of `batch` examples."""
+        eng, hy = self.eng, self.eng.net.hypers
+        n = int(x0.shape[0])
+        if tuple(x0.shape[1:]) != tuple(hy.x0_shape):
+            raise ValueError('x0: shape %s, expected (n,) + %s' % (tuple(x0.shape), tuple(hy.x0_shape)))
+        kf = self._k_feature(k_cpt, n)
+        nc = self.n_cls
+        # one byte buffer holds the four outputs, so that one device-to-host copy returns them
+        o_prob = 8 * n
+        o_cls = o_prob + 4 * n * nc
+        o_exit = o_cls + 4 * n
+        nbytes = o_exit + 4 * n
+        if n == 0:
+            host = np.zeros(nbytes, np.uint8)
+        else:
+            with torch.cuda.device(eng.dev):
+                self._prepare()                      # every call: the current parameters and running moments
+                buf = torch.empty(nbytes, dtype=torch.uint8, device=eng.dev)
+                kfd = torch.from_numpy(kf).to(eng.dev, non_blocking=True) if kf is not None else None
+                base_ptr = buf.data_ptr()
+                visits = self.visits.copy()          # node visits belong to the statistics of the data set
+                try:
+                    for b0 in range(0, n, self.B):
+                        m = min(self.B, n - b0)
+                        self._emit = Ns(prob=base_ptr + o_prob + 4 * nc * b0, cls=base_ptr + o_cls + 4 * b0,
+                                        exit=base_ptr + o_exit + 4 * b0, ops=base_ptr + 8 * b0)
+                        self._walk(x0[b0:b0 + m], m, kfd[b0:b0 + m] if kfd is not None else None)
+                finally:
+                    self._emit = None
+                    self.visits[:] = visits
+                host = buf.cpu().numpy()
+        return Ns(cls=host[o_cls:o_exit].view(np.int32), prob=host[o_prob:o_cls].view(np.float32).reshape(n, nc),
+                  exit=host[o_exit:nbytes].view(np.int32), ops=host[:o_prob].view(np.float64))
 
     # ------------------------------------------------------------------ #
     def _node(self, nd, n, orig, pos, count_dev):
@@ -138,8 +225,15 @@ class CompactEvaluator:
                 # logits of the parent's compact batch (rows of the examples that exit here are read through pos)
                 L.fc_fwd(_vp(pst.feat), pst.F, plan.Balloc, self._n_parent, eng.tptr(r.fc.params.w),
                          eng.tptr(r.fc.params.b), None, self.n_cls, _vp(r.Zbuf), eng.dtype, self._S())
-            L.leaf_stats(_vp(r.Zbuf), r.ldz, self.n_cls, _vp(plan.y), _vp(pos), _vp(orig), _vp(count_dev), n,
-                         _vp(self.acc[nd.err]), self._S())
+            o = self._emit
+            if o is None:
+                L.leaf_stats(_vp(r.Zbuf), r.ldz, self.n_cls, _vp(plan.y), _vp(pos), _vp(orig), _vp(count_dev), n,
+                             _vp(self.acc[nd.err]), self._S())
+            else:
+                V = ctypes.c_void_p
+                L.leaf_emit(_vp(r.Zbuf), r.ldz, self.n_cls, _vp(pos), _vp(orig), _vp(count_dev), n,
+                            self.leaf_no[nd.idx], self.path_ops[self.leaf_no[nd.idx]],
+                            V(o.prob), V(o.cls), V(o.exit), V(o.ops), self._S())
             return
         st = plan.node[nd.idx]
         dt, impl = eng.dtype, eng.impl
@@ -150,6 +244,13 @@ class CompactEvaluator:
                 L.gather_images(_vp(slot.t), self._n_parent, g.P, _vp(pos), _vp(count_dev), _vp(dst), n, g.P,
                                 slot.C, g.H, g.W, g.G, dt, self._S())
             ins = self.cin[nd.idx]
+        rt = plan.rtr.get(nd.idx)
+        if self.dyn_k and rt is not None:           # the router's k_cpt feature, in this node's compact order
+            if plan.umma_heads:                      # channel 0 of the extra planes of the head GEMM's input
+                L.gather_feature(_vp(self.kfeat), _vp(orig), _vp(count_dev), n, None, _vp(st.feat[st.F // 8, :, 0]), 8,
+                                 dt, self._S())
+            else:
+                L.gather_feature(_vp(self.kfeat), _vp(orig), _vp(count_dev), n, _vp(plan.kextra), None, 0, 0, self._S())
         for k, sc in enumerate(st.sc):
             g = sc.geo
             prev = st.sc[k - 1] if k > 0 else None
@@ -162,8 +263,6 @@ class CompactEvaluator:
                                    _vp(sc.feat), plan.Balloc, dt, self._S())
         if not nd.kids:
             return
-        dyn_k = bool(eng.net.hypers.dyn_k_cpt)
-        rt = plan.rtr.get(nd.idx)
         if plan.umma_heads and nd.idx in plan.heads:
             hd = plan.heads[nd.idx]
             outs = ([(hd.Z16, 16)] if hd.leaf_off is not None else []) + ([(rt.Z1, 16)] if rt is not None else [])
@@ -173,7 +272,7 @@ class CompactEvaluator:
                            n, 0, 0, 0, plan.Balloc, None, 0, None, BF16, 2, 1, self._S())
         elif rt is not None:
             L.fc_fwd(_vp(st.feat), st.F, plan.Balloc, n, eng.tptr(rt.fc1.params.w), eng.tptr(rt.fc1.params.b),
-                     _vp(plan.kextra) if dyn_k else None, 16, _vp(rt.Z1), dt, self._S())
+                     _vp(plan.kextra) if self.dyn_k else None, 16, _vp(rt.Z1), dt, self._S())
         if len(nd.kids) == 1:                       # no switch: the only sink sees every example of this node
             self._n_parent = n
             self._node(eng.nodes[nd.kids[0]], n, orig, None, None)

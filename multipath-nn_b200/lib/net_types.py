@@ -127,6 +127,19 @@ class Net:
             cache[batch] = CompactEvaluator(self._get_engine(), batch)
         return cache[batch]
 
+    def predict(self, x0, k_cpt=None, batch=4096):
+        """Routed inference: run every example of x0 (numpy or torch, host or device, any n) only along its own
+        path in 'ev' mode, in chunks of `batch` on the cached `compact_evaluator(batch)`.  No labels.  Returns
+        Ns of numpy arrays:
+            cls  int32 (n,)            predicted class (first argmax of prob)
+            prob float32 (n, n_cls)    softmax of the classifier the example exits at
+            exit int32 (n,)            that classifier's index in list(net.leaves)
+            ops  float64 (n,)          ops of the nodes and routers on the example's path (the dense `moc`)
+        k_cpt: required for nets with a per-example k_cpt (dyn_k_cpt) -- a scalar, one value or n values --
+        and None for the others.  The weights are packed and the BatchNorm moments finalised on every call, so a
+        call between training steps sees the current parameters."""
+        return self.compact_evaluator(batch).predict(x0, k_cpt)
+
     def eval_stats(self, feed_dict):
         """Per-example `state_tensors` (train-nets:111-130) for one batch, as a
         dict {(net|layer, name): ndarray}; `mode` defaults to 'ev'."""

@@ -1,0 +1,109 @@
+"""Routed inference (`net.predict`) against the dense 'ev' forward (`Engine.forward` on an eval plan) on cifar10-ac at
+the real architecture in bf16, for three router settings and B in {128, 4096, 16384}:
+
+  (a) fresh net: the zero-initialised last router layer ties, every example exits at stage 0;
+  (b) every switch biased to continue: every example runs the whole chain (worst case for the compaction);
+  (c) randomized routers (tests/util.py::randomize_routers).
+
+CUDA events around each call, warm-up first, the two paths alternated in one process, and a 256 MB buffer
+rewritten before every timed call so that neither path reads its inputs or weights from L2 (126 MB).  Reports
+ms per call (median of the repeats), images/s, mean ops as a fraction of the whole tree, the exit histogram and
+the host synchronisations of one predict call (one per switch visited per chunk, plus the final read-back)."""
+import os
+import subprocess
+import sys
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path[:0] = [ROOT, os.path.join(ROOT, 'multipath-nn_b200'), os.path.join(ROOT, 'tests')]
+import numpy as np  # noqa: E402
+import torch  # noqa: E402
+
+import arch_and_hypers as ah  # noqa: E402
+from lib import layer_types  # noqa: E402
+from util import randomize_routers  # noqa: E402
+
+BATCHES = [int(b) for b in os.environ.get('BATCHES', '128,4096,16384').split(',')]
+REPS = int(os.environ.get('REPS', 10))
+
+
+def card():
+    q = subprocess.run(['nvidia-smi', '--query-gpu=name,power.limit,clocks.max.sm', '--format=csv,noheader'],
+                       capture_output=True, text=True)
+    return q.stdout.strip().splitlines()[torch.cuda.current_device()] if q.returncode == 0 else 'nvidia-smi failed'
+
+
+def make_net(setting):
+    layer_types.seed(0)
+    net = ah.ac_chain(k_cpt=4e-9)((32, 32, 3), (10,))
+    if setting == 'continue':
+        for l in net.layers:
+            if l.router is not None:
+                last = l.router.comps[-1]
+                last.params.w.assign(np.zeros(last.params.w.shape, np.float32))
+                b = np.zeros(last.params.b.shape, np.float32)
+                b[1:] = 1.0                                 # sink 0 is the stage's classifier, sink 1 the next stage
+                last.params.b.assign(b)
+    elif setting == 'random':
+        randomize_routers(net)
+    return net.configure(precision='bf16')
+
+
+def switches_visited(eng, exit_, B):
+    """host synchronisations of one predict call: per chunk, every switch that some example of the chunk reaches"""
+    below = {}
+    for i, leaf in enumerate(eng.leaves):
+        j = eng.nodes[leaf.idx].parent
+        while j is not None:
+            below.setdefault(j, set()).add(i)
+            j = eng.nodes[j].parent
+    n = 0
+    for b0 in range(0, len(exit_), B):
+        seen = set(exit_[b0:b0 + B].tolist())
+        n += sum(1 for sw in eng.switches if below[sw.idx] & seen)
+    return n + 1
+
+
+def main():
+    torch.cuda.init()
+    print('card (name, power limit, max SM clock): %s' % card())
+    rng = np.random.default_rng(0)
+    flush = torch.empty(256 << 20, dtype=torch.uint8, device='cuda')
+    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    print('%-9s %6s %12s %12s %12s %12s %7s %8s %6s  %s' % ('routers', 'B', 'dense ms', 'predict ms', 'dense im/s',
+                                                           'predict im/s', 'speedup', 'ops frac', 'syncs', 'exits'))
+    for setting in ('fresh', 'continue', 'random'):
+        net = make_net(setting)
+        eng = net._get_engine()
+        ops_tree = float(sum(l.n_ops + (l.router.n_ops if l.router is not None else 0) for l in net.layers))
+        for B in BATCHES:
+            x0 = torch.from_numpy(rng.random((B, 32, 32, 3), dtype=np.float32)).cuda()
+            y = torch.from_numpy(np.eye(10, dtype=np.float32)[rng.integers(0, 10, B)]).cuda()
+            feed = {net.x0: x0, net.y: y, net.τ: 0.5}
+            dense = lambda: eng.forward(feed, 'ev')
+            routed = lambda: net.predict(x0, batch=B)
+
+            def timed(fn):
+                flush.fill_(1)
+                ev0.record()
+                r = fn()
+                ev1.record()
+                ev1.synchronize()
+                return ev0.elapsed_time(ev1), r
+            for _ in range(3):                                # warm-up: plans, packing, module loads
+                timed(dense), timed(routed)
+            t_d, t_p = [], []
+            for _ in range(REPS):                             # alternated
+                t_d.append(timed(dense)[0])
+                t, r = timed(routed)
+                t_p.append(t)
+            md, mp = float(np.median(t_d)), float(np.median(t_p))
+            hist = np.bincount(r.exit, minlength=len(eng.leaves))
+            print('%-9s %6d %12.3f %12.3f %12.0f %12.0f %7.2f %8.3f %6d  %s' % (
+                setting, B, md, mp, B / md * 1e3, B / mp * 1e3, md / mp, r.ops.mean() / ops_tree,
+                switches_visited(eng, r.exit, B), hist.tolist()), flush=True)
+        del net, eng
+        torch.cuda.empty_cache()
+
+
+if __name__ == '__main__':
+    main()
