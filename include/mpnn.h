@@ -490,6 +490,35 @@ int mpnn_allreduce_talr_p2p(const mpnn_p2p_desc* d /* host */, const int* seg_st
                             const float* seg_mult, const float* seg_l2, int n_seg, int use_stats, int talr,
                             const float* hyp, int write_back, int lo, int hi, int channel, void* stream);
 
+/* ---- counted launches: the live batch in device memory ------------------------------------------------------
+ * Each entry point below is the one named without `_counted`, plus `count`: a DEVICE int holding the live batch m.
+ * The batch argument B (n for mpnn_route_compact) becomes the capacity the grid is sized for; the call processes
+ * the first min(*count, B) examples exactly as the uncounted call with batch m would (bit for bit: the launch
+ * variants are chosen from the capacity and do the same per-row arithmetic), and writes nothing at or past them.
+ * m = 0 is valid.  count == NULL is the uncounted call.  A stream-ordered walk whose batch sizes are produced on
+ * the device (mpnn_route_compact's count) can so be launched, and captured into a CUDA graph, without reading
+ * them back to the host.
+ *   mpnn_stencil_gemm_counted: no statistics (stats == NULL).  Rows are pixels: q < m * (H+1)(W+1).
+ *   mpnn_router_tail_fwd_batched_counted: train == 0 only (train-mode moments are batch statistics).
+ *   mpnn_route_compact_counted: n_count is the count of the parent's compact batch (its `count` is the output). */
+int mpnn_pack_input_counted(const float* x0, int B, int H0, int W0, int C0, int step,
+                            void* planes, int Cpad, int G, int P, int dtype, const int* count, void* stream);
+int mpnn_stencil_gemm_counted(const void* A0, int K0, const void* A1, int K1,
+                              const void* Wp, int ntaps, const float* bias,
+                              void* out0, int N0, int acc0, void* out1, int N1, int acc1,
+                              int B, int H, int W, int G, int P,
+                              float* stats, int stats_cap, int* n_parts,
+                              int dtype, int out_dtype, int impl, const int* count, void* stream);
+int mpnn_bn_relu_pool_fwd_counted(const void* lin, int C, int B, int H, int W, int G, int P,
+                                  const float* ss, void* act, void* pooled, int Pp,
+                                  void* feat, int Balloc, int dtype, const int* count, void* stream);
+int mpnn_fc_fwd_counted(const void* X, int F, int Balloc, int B, const float* W, const float* bias,
+                        const float* extra, int n, float* Z, int dtype, const int* count, void* stream);
+int mpnn_router_tail_fwd_batched_counted(const mpnn_router_fwd_desc* descs, int n, int B, int C,
+                                         float d, float eps, int train, const int* count, void* stream);
+int mpnn_route_compact_counted(const float* R, int ldr, int ns, int n, const int* parent_orig, int cap,
+                               int* dec, int* pos, int* orig, int* count, const int* n_count, void* stream);
+
 /* ---- tcgen05 bring-up probe (tests only) -------------------------------- */
 /* D[128][N] = A[128][K] * B[N][K]^T through one CTA of tcgen05.mma; all
  * operands in the interleaved (no-swizzle) core-matrix layout. */

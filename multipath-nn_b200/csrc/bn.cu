@@ -64,17 +64,20 @@ extern "C" int mpnn_bn_finalize(const float* partials, int n_parts, int C, doubl
 // load and store instruction is fully coalesced; the 2x2 maximum is taken in-thread
 // over the row pair and across the lane pair (w, w^1) with one shuffle per channel.
 // grid.y = plane, so the per-channel constants are loaded once per thread.
-template <typename T, bool POOL>
+// CNT: only the first min(*count, g.B) images are read and written (g.B: the capacity the grid was sized for).
+template <typename T, bool POOL, bool CNT = false>
 __global__ void __launch_bounds__(256)
 bn_relu_pool_fwd_kernel(const T* __restrict__ lin, int C, Geom g,
                         const float* __restrict__ ss, T* __restrict__ act,
                         T* __restrict__ pooled, Geom gp,
-                        T* __restrict__ feat, int Balloc, const mpnn_bn_fuse bn) {
+                        T* __restrict__ feat, int Balloc, const mpnn_bn_fuse bn, const int* __restrict__ count) {
     pdl_launch_dependents();
     pdl_wait();
     const int KG = C / 8, kg = blockIdx.y;
     const int HH = POOL ? g.H / 2 : g.H;
-    const unsigned total = (unsigned)g.B * HH * g.W;          // host guarantees < 2^31
+    const int nb = CNT ? min(max(*count, 0), g.B) : g.B;
+    const unsigned total = (unsigned)nb * HH * g.W;           // host guarantees < 2^31
+    if (CNT && total == 0) return;
     float a[8], c[8];
     const bool affine = (ss || bn.acc) && (act || feat);
     if (bn.acc) {
@@ -146,8 +149,9 @@ bn_relu_pool_fwd_kernel(const T* __restrict__ lin, int C, Geom g,
 
 static int bn_relu_pool_fwd_impl(const void* lin, int C, int B, int H, int W, int G, int P,
                                  const float* ss, const mpnn_bn_fuse* bnp, void* act, void* pooled, int Pp,
-                                 void* feat, int Balloc, int dtype, void* stream) {
+                                 void* feat, int Balloc, int dtype, void* stream, const int* count = nullptr) {
     MPNN_REQUIRE(C % 8 == 0, "bn_relu_pool_fwd: C=%d", C);
+    MPNN_REQUIRE(!count || !bnp, "bn_relu_pool_fwd_counted: no train-mode statistics");
     MPNN_REQUIRE(!(pooled && feat), "bn_relu_pool_fwd: pooled and feat are exclusive");
     MPNN_REQUIRE(pooled || ss || bnp, "bn_relu_pool_fwd: nothing to do");
     MPNN_REQUIRE(!pooled || (H % 2 == 0 && W % 2 == 0), "bn_relu_pool_fwd: odd size");
@@ -166,13 +170,14 @@ static int bn_relu_pool_fwd_impl(const void* lin, int C, int B, int H, int W, in
     cudaStream_t st = (cudaStream_t)stream;
     mpnn_bn_fuse bn = {};
     if (bnp) bn = *bnp;
+#define GO(POOL, CNT) MPNN_DISPATCH_DTYPE(dtype, (mpnn_launch_pdl(bn_relu_pool_fwd_kernel<T, POOL, CNT>, grid, dim3(256), \
+        0, st, (const T*)lin, C, g, ss, (T*)act, (T*)pooled, gp, (T*)feat, Balloc, bn, count)))
     if (pooled) {
-        MPNN_DISPATCH_DTYPE(dtype, (mpnn_launch_pdl(bn_relu_pool_fwd_kernel<T, true>, grid, dim3(256), 0, st,
-            (const T*)lin, C, g, ss, (T*)act, (T*)pooled, gp, (T*)feat, Balloc, bn)));
+        if (count) GO(true, true); else GO(true, false);
     } else {
-        MPNN_DISPATCH_DTYPE(dtype, (mpnn_launch_pdl(bn_relu_pool_fwd_kernel<T, false>, grid, dim3(256), 0, st,
-            (const T*)lin, C, g, ss, (T*)act, (T*)pooled, gp, (T*)feat, Balloc, bn)));
+        if (count) GO(false, true); else GO(false, false);
     }
+#undef GO
     return mpnn_check_launch("bn_relu_pool_fwd");
 }
 
@@ -180,6 +185,13 @@ extern "C" int mpnn_bn_relu_pool_fwd(const void* lin, int C, int B, int H, int W
                                      const float* ss, void* act, void* pooled, int Pp,
                                      void* feat, int Balloc, int dtype, void* stream) {
     return bn_relu_pool_fwd_impl(lin, C, B, H, W, G, P, ss, nullptr, act, pooled, Pp, feat, Balloc, dtype, stream);
+}
+
+extern "C" int mpnn_bn_relu_pool_fwd_counted(const void* lin, int C, int B, int H, int W, int G, int P,
+                                             const float* ss, void* act, void* pooled, int Pp,
+                                             void* feat, int Balloc, int dtype, const int* count, void* stream) {
+    return bn_relu_pool_fwd_impl(lin, C, B, H, W, G, P, ss, nullptr, act, pooled, Pp, feat, Balloc, dtype, stream,
+                                 count);
 }
 
 extern "C" int mpnn_bn_relu_pool_fwd_acc(const void* lin, int C, int B, int H, int W, int G, int P,

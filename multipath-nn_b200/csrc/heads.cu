@@ -9,14 +9,17 @@
 #define FC_NMAX 16
 
 // ---------------------------------------------------------------- fc forward
-template <typename T>
+// CNT: only the rows b < min(*count, B) are stored (B: the capacity the grid was sized for)
+template <typename T, bool CNT = false>
 __global__ void __launch_bounds__(256)
 fc_fwd_kernel(const T* __restrict__ X, int F, int Balloc, int B, const float* __restrict__ W,
               const float* __restrict__ bias, const float* __restrict__ extra, int n,
-              float* __restrict__ Z) {
+              float* __restrict__ Z, const int* __restrict__ count) {
     const int lane = threadIdx.x, ky = threadIdx.y;   // 32 x 8
     const int b = blockIdx.x * 32 + lane;
     const int bl = b < B ? b : B - 1;
+    const int Bn = CNT ? min(max(*count, 0), B) : B;
+    if (CNT && (int)blockIdx.x * 32 >= Bn) return;
     float acc[FC_NMAX];
 #pragma unroll
     for (int j = 0; j < FC_NMAX; ++j) acc[j] = 0.f;
@@ -42,7 +45,7 @@ fc_fwd_kernel(const T* __restrict__ X, int F, int Balloc, int B, const float* __
         for (int s = 0; s < 8; ++s) t += red[s][lane][j];
         if (extra) t = fmaf(extra[bl], __ldg(W + (size_t)F * n + j), t);
         t += bias ? bias[j] : 0.f;
-        if (b < B) Z[(size_t)b * n + j] = t;
+        if (b < Bn) Z[(size_t)b * n + j] = t;
     }
 }
 
@@ -52,8 +55,19 @@ extern "C" int mpnn_fc_fwd(const void* X, int F, int Balloc, int B, const float*
     MPNN_REQUIRE(B >= 1 && Balloc >= B, "fc_fwd: B=%d Balloc=%d", B, Balloc);
     dim3 block(32, 8), grid(ceil_div(B, 32));
     MPNN_DISPATCH_DTYPE(dtype, (fc_fwd_kernel<T><<<grid, block, 0, (cudaStream_t)stream>>>(
-        (const T*)X, F, Balloc, B, W, bias, extra, n, Z)));
+        (const T*)X, F, Balloc, B, W, bias, extra, n, Z, nullptr)));
     return mpnn_check_launch("fc_fwd");
+}
+
+extern "C" int mpnn_fc_fwd_counted(const void* X, int F, int Balloc, int B, const float* W, const float* bias,
+                                   const float* extra, int n, float* Z, int dtype, const int* count, void* stream) {
+    if (!count) return mpnn_fc_fwd(X, F, Balloc, B, W, bias, extra, n, Z, dtype, stream);
+    MPNN_REQUIRE(F % 8 == 0 && n >= 1 && n <= FC_NMAX, "fc_fwd: F=%d n=%d (n<=%d)", F, n, FC_NMAX);
+    MPNN_REQUIRE(B >= 1 && Balloc >= B, "fc_fwd: B=%d Balloc=%d", B, Balloc);
+    dim3 block(32, 8), grid(ceil_div(B, 32));
+    MPNN_DISPATCH_DTYPE(dtype, (fc_fwd_kernel<T, true><<<grid, block, 0, (cudaStream_t)stream>>>(
+        (const T*)X, F, Balloc, B, W, bias, extra, n, Z, count)));
+    return mpnn_check_launch("fc_fwd_counted");
 }
 
 // ---------------------------------------------------------- fc backward data

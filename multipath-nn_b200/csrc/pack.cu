@@ -29,10 +29,12 @@ extern "C" int mpnn_version(void) { return 100; }
 // ToPyramid: strided subsample of NHWC fp32 into padded planes.
 // One thread per (plane kg, valid pixel); 8 channels each.
 // --------------------------------------------------------------------------- //
-template <typename T>
+// CNT: the first min(*count, g.B) images only (g.B: the capacity the grid was sized for)
+template <typename T, bool CNT = false>
 __global__ void pack_input_kernel(const float* __restrict__ x0, int H0, int W0, int C0, int step,
-                                  T* __restrict__ planes, int Cpad, Geom g) {
+                                  T* __restrict__ planes, int Cpad, Geom g, const int* __restrict__ count) {
     const int KG = Cpad / 8;
+    if (CNT) g.B = min(max(*count, 0), g.B);
     const long long total = (long long)KG * g.B * g.H * g.W;
     for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total;
          i += (long long)gridDim.x * blockDim.x) {
@@ -52,8 +54,8 @@ __global__ void pack_input_kernel(const float* __restrict__ x0, int H0, int W0, 
     }
 }
 
-extern "C" int mpnn_pack_input(const float* x0, int B, int H0, int W0, int C0, int step,
-                               void* planes, int Cpad, int G, int P, int dtype, void* stream) {
+static int pack_input_impl(const float* x0, int B, int H0, int W0, int C0, int step,
+                           void* planes, int Cpad, int G, int P, int dtype, const int* count, void* stream) {
     MPNN_REQUIRE(step >= 1 && H0 % step == 0 && W0 % step == 0, "pack_input: bad step %d", step);
     MPNN_REQUIRE(Cpad % 8 == 0 && Cpad >= C0, "pack_input: Cpad=%d C0=%d", Cpad, C0);
     Geom g = make_geom(B, H0 / step, W0 / step, G, P);
@@ -62,9 +64,25 @@ extern "C" int mpnn_pack_input(const float* x0, int B, int H0, int W0, int C0, i
     int grid = (int)((total + 255) / 256);
     if (grid > 148 * 16) grid = 148 * 16;
     if (grid < 1) grid = 1;
-    MPNN_DISPATCH_DTYPE(dtype, (pack_input_kernel<T><<<grid, 256, 0, (cudaStream_t)stream>>>(
-        x0, H0, W0, C0, step, (T*)planes, Cpad, g)));
+    if (count) {
+        MPNN_DISPATCH_DTYPE(dtype, (pack_input_kernel<T, true><<<grid, 256, 0, (cudaStream_t)stream>>>(
+            x0, H0, W0, C0, step, (T*)planes, Cpad, g, count)));
+    } else {
+        MPNN_DISPATCH_DTYPE(dtype, (pack_input_kernel<T><<<grid, 256, 0, (cudaStream_t)stream>>>(
+            x0, H0, W0, C0, step, (T*)planes, Cpad, g, nullptr)));
+    }
     return mpnn_check_launch("pack_input");
+}
+
+extern "C" int mpnn_pack_input(const float* x0, int B, int H0, int W0, int C0, int step,
+                               void* planes, int Cpad, int G, int P, int dtype, void* stream) {
+    return pack_input_impl(x0, B, H0, W0, C0, step, planes, Cpad, G, P, dtype, nullptr, stream);
+}
+
+extern "C" int mpnn_pack_input_counted(const float* x0, int B, int H0, int W0, int C0, int step,
+                                       void* planes, int Cpad, int G, int P, int dtype, const int* count,
+                                       void* stream) {
+    return pack_input_impl(x0, B, H0, W0, C0, step, planes, Cpad, G, P, dtype, count, stream);
 }
 
 // --------------------------------------------------------------------------- //

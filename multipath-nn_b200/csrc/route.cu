@@ -637,9 +637,10 @@ extern "C" int mpnn_gather_feature(const float* src, const int* orig, const int*
 // switch, and for every sink the ascending list of positions (rows of the parent's compact batch) and
 // of original example ids that chose it -- ballot + prefix scan, order preserving, one CTA.
 __global__ void __launch_bounds__(1024)
-route_compact_kernel(const float* __restrict__ R, int ldr, int ns, int n, const int* __restrict__ parent_orig,
+route_compact_kernel(const float* __restrict__ R, int ldr, int ns, int n_max, const int* __restrict__ parent_orig,
                      int cap, int* __restrict__ dec, int* __restrict__ pos, int* __restrict__ orig,
-                     int* __restrict__ count) {
+                     int* __restrict__ count, const int* __restrict__ n_count) {
+    const int n = n_count ? min(max(*n_count, 0), n_max) : n_max;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     __shared__ int wcount[8][32];
     __shared__ int base_s[8];
@@ -685,8 +686,18 @@ extern "C" int mpnn_route_compact(const float* R, int ldr, int ns, int n, const 
                                   int* dec, int* pos, int* orig, int* count, void* stream) {
     MPNN_REQUIRE(R && pos && orig && count && ns >= 1 && ns <= 8 && n >= 0 && cap >= n && ldr >= ns,
                  "route_compact: ns=%d n=%d cap=%d ldr=%d", ns, n, cap, ldr);
-    route_compact_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(R, ldr, ns, n, parent_orig, cap, dec, pos, orig, count);
+    route_compact_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(R, ldr, ns, n, parent_orig, cap, dec, pos, orig, count,
+                                                               nullptr);
     return mpnn_check_launch("route_compact");
+}
+
+extern "C" int mpnn_route_compact_counted(const float* R, int ldr, int ns, int n, const int* parent_orig, int cap,
+                                          int* dec, int* pos, int* orig, int* count, const int* n_count, void* stream) {
+    MPNN_REQUIRE(R && pos && orig && count && ns >= 1 && ns <= 8 && n >= 0 && cap >= n && ldr >= ns,
+                 "route_compact: ns=%d n=%d cap=%d ldr=%d", ns, n, cap, ldr);
+    route_compact_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(R, ldr, ns, n, parent_orig, cap, dec, pos, orig, count,
+                                                               n_count);
+    return mpnn_check_launch("route_compact_counted");
 }
 
 // Leaf statistics of the examples routed to one classifier (train-nets:117-130 with p_ev one-hot):

@@ -242,8 +242,12 @@ __device__ __forceinline__ void cluster_channel_sum(cg::cluster_group& cluster, 
     cluster.sync();          // everyone has read `part` before it is reused
 }
 
+// CNT (eval mode only): the rows b < min(*count, B) are computed and stored; the batch is split over the cluster by
+// the capacity B, so every row sees the arithmetic of an uncounted launch at batch B
+template <bool CNT = false>
 __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(T)
-router_tail_fwd_cluster_kernel(const mpnn_router_fwd_desc* __restrict__ descs, int B, float d, float eps, int train) {
+router_tail_fwd_cluster_kernel(const mpnn_router_fwd_desc* __restrict__ descs, int B, float d, float eps, int train,
+                               const int* __restrict__ count) {
     cg::cluster_group cluster = cg::this_cluster();
     const int rank = (int)cluster.block_rank();
     const mpnn_router_fwd_desc r = descs[blockIdx.x / CL];
@@ -256,7 +260,7 @@ router_tail_fwd_cluster_kernel(const mpnn_router_fwd_desc* __restrict__ descs, i
     if (tid < C) sb2[tid] = r.bias2[tid];
     if (tid < ns) sb3[tid] = r.bias3[tid];
     const int Bc = (B + CL - 1) / CL;
-    const int b_lo = rank * Bc, b_hi = min(B, b_lo + Bc);
+    const int b_lo = rank * Bc, b_hi = min(CNT ? min(max(*count, 0), B) : B, b_lo + Bc);
     for (int layer = 0; layer < 2; ++layer) {
         const float* Zin = layer == 0 ? r.Z1 : r.Z2;
         const float* gg = layer == 0 ? r.g1 : r.g2;
@@ -390,9 +394,10 @@ __device__ __forceinline__ void cta_colsum16(float (&v)[C], float* wpart, float*
     }
 }
 
-template <int RPT>
+template <int RPT, bool CNT = false>
 __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(T)
-router_tail_fwd_fast_kernel(const mpnn_router_fwd_desc* __restrict__ descs, int B, float d, float eps, int train) {
+router_tail_fwd_fast_kernel(const mpnn_router_fwd_desc* __restrict__ descs, int B, float d, float eps, int train,
+                            const int* __restrict__ count) {
     cg::cluster_group cluster = cg::this_cluster();
     const int rank = (int)cluster.block_rank();
     const mpnn_router_fwd_desc r = descs[blockIdx.x / CL];
@@ -404,7 +409,7 @@ router_tail_fwd_fast_kernel(const mpnn_router_fwd_desc* __restrict__ descs, int 
     if (tid < C) sb2[tid] = r.bias2[tid];
     if (tid < ns) sb3[tid] = r.bias3[tid];
     const int Bc = (B + CL - 1) / CL;
-    const int b_lo = rank * Bc, b_hi = min(B, b_lo + Bc);
+    const int b_lo = rank * Bc, b_hi = min(CNT ? min(max(*count, 0), B) : B, b_lo + Bc);
     float z[RPT][C];
     bool ok[RPT];
 #pragma unroll
@@ -713,14 +718,28 @@ extern "C" int mpnn_router_tail_bwd_batched(const mpnn_router_bwd_desc* descs, i
     return mpnn_check_launch("router_tail_bwd_batched");
 }
 
+template <bool CNT>
+static int router_tail_fwd_launch(const mpnn_router_fwd_desc* descs, int n, int B, float d, float eps, int train,
+                                  const int* count, cudaStream_t st) {
+    static const int fast = getenv("MPNN_ROUTER_FAST") ? atoi(getenv("MPNN_ROUTER_FAST")) : 1;
+    const int per_cta = ceil_div(B, CL);
+    if (fast && per_cta <= T) router_tail_fwd_fast_kernel<1, CNT><<<n * CL, T, 0, st>>>(descs, B, d, eps, train, count);
+    else if (fast && per_cta <= 2 * T) router_tail_fwd_fast_kernel<2, CNT><<<n * CL, T, 0, st>>>(descs, B, d, eps, train, count);
+    else if (fast && per_cta <= 4 * T) router_tail_fwd_fast_kernel<4, CNT><<<n * CL, T, 0, st>>>(descs, B, d, eps, train, count);
+    else router_tail_fwd_cluster_kernel<CNT><<<n * CL, T, 0, st>>>(descs, B, d, eps, train, count);
+    return mpnn_check_launch("router_tail_fwd_batched");
+}
+
 extern "C" int mpnn_router_tail_fwd_batched(const mpnn_router_fwd_desc* descs, int n, int B, int Cw,
                                             float d, float eps, int train, void* stream) {
     MPNN_REQUIRE(Cw == C && n >= 1, "router_tail_fwd_batched: C=%d n=%d", Cw, n);
-    static const int fast = getenv("MPNN_ROUTER_FAST") ? atoi(getenv("MPNN_ROUTER_FAST")) : 1;
-    const int per_cta = ceil_div(B, CL);
-    if (fast && per_cta <= T) router_tail_fwd_fast_kernel<1><<<n * CL, T, 0, (cudaStream_t)stream>>>(descs, B, d, eps, train);
-    else if (fast && per_cta <= 2 * T) router_tail_fwd_fast_kernel<2><<<n * CL, T, 0, (cudaStream_t)stream>>>(descs, B, d, eps, train);
-    else if (fast && per_cta <= 4 * T) router_tail_fwd_fast_kernel<4><<<n * CL, T, 0, (cudaStream_t)stream>>>(descs, B, d, eps, train);
-    else router_tail_fwd_cluster_kernel<<<n * CL, T, 0, (cudaStream_t)stream>>>(descs, B, d, eps, train);
-    return mpnn_check_launch("router_tail_fwd_batched");
+    return router_tail_fwd_launch<false>(descs, n, B, d, eps, train, nullptr, (cudaStream_t)stream);
+}
+
+extern "C" int mpnn_router_tail_fwd_batched_counted(const mpnn_router_fwd_desc* descs, int n, int B, int Cw,
+                                                    float d, float eps, int train, const int* count, void* stream) {
+    MPNN_REQUIRE(Cw == C && n >= 1, "router_tail_fwd_batched: C=%d n=%d", Cw, n);
+    if (!count) return mpnn_router_tail_fwd_batched(descs, n, B, Cw, d, eps, train, stream);
+    MPNN_REQUIRE(!train, "router_tail_fwd_batched_counted: eval mode only (train-mode moments need the whole batch)");
+    return router_tail_fwd_launch<true>(descs, n, B, d, eps, train, count, (cudaStream_t)stream);
 }

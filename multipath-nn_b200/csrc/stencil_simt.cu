@@ -9,7 +9,7 @@
 int mpnn_stencil_gemm_umma(const void* A0, int K0, const void* A1, int K1, const void* Wp, int ntaps,
                            const float* bias, void* out0, int N0, int acc0, void* out1, int N1, int acc1,
                            Geom g, float* stats, int stats_cap, int* n_parts, int out_dtype,
-                           const mpnn_bn_fuse* bn, const mpnn_bn_bwd_epi* bwd, cudaStream_t st);
+                           const mpnn_bn_fuse* bn, const mpnn_bn_bwd_epi* bwd, const int* count, cudaStream_t st);
 int mpnn_stencil_wgrad_umma(const void* A0, int K0, int K0real, float* dW0, const void* A1, int K1,
                             int K1real, float* dW1, const void* Gd, int N, int Nreal, float* dbias,
                             int ntaps, Geom g, cudaStream_t st);
@@ -18,13 +18,19 @@ __device__ __forceinline__ int tap_offset(int ntaps, int tap, int Wp) {
     return ntaps == 9 ? (tap / 3 - 1) * Wp + (tap % 3 - 1) : 0;
 }
 
-template <typename T, typename TO, int NB>
+// CNT: the live batch is min(*count, g.B) (g.B: the capacity the grid was sized for); only its rows are stored.
+template <typename T, typename TO, int NB, bool CNT = false>
 __global__ void __launch_bounds__(128)
 stencil_gemm_simt(const T* __restrict__ A0, int K0, const T* __restrict__ A1, int K1,
                   const T* __restrict__ Wp, int ntaps, const float* __restrict__ bias,
                   TO* __restrict__ out0, int N0, int acc0, TO* __restrict__ out1, int N1, int acc1,
-                  Geom g, int n_tiles, float* __restrict__ stats, const mpnn_bn_fuse bn) {
+                  Geom g, int n_tiles, float* __restrict__ stats, const mpnn_bn_fuse bn, const int* __restrict__ count) {
     const int N = N0 + N1;
+    int row_end = g.rows + 128 - 1;              // the tiles' pad rows beyond the batch are stored too (unspecified)
+    if (CNT) {
+        row_end = min(max(*count, 0), g.B) * g.S;
+        n_tiles = (row_end + 127) >> 7;
+    }
     const int n0 = blockIdx.y * NB;
     const int KG0 = K0 / 8, KG = (K0 + K1) / 8;
     float ssum[NB], ssq[NB];
@@ -55,7 +61,7 @@ stencil_gemm_simt(const T* __restrict__ A0, int K0, const T* __restrict__ A1, in
         }
         int n_, h_, w_;
         const bool valid = row_valid(g, q, n_, h_, w_);
-        if (q < g.rows + 128 - 1 && p < g.P) {
+        if (q < row_end && p < g.P) {
 #pragma unroll
             for (int j8 = 0; j8 < NB / 8; ++j8) {
                 int col = n0 + j8 * 8;
@@ -103,11 +109,11 @@ stencil_gemm_simt(const T* __restrict__ A0, int K0, const T* __restrict__ A1, in
     }
 }
 
-template <typename T, typename TO>
+template <typename T, typename TO, bool CNT>
 static int launch_gemm_simt(const void* A0, int K0, const void* A1, int K1, const void* Wp, int ntaps,
                             const float* bias, void* out0, int N0, int acc0, void* out1, int N1, int acc1,
                             Geom g, float* stats, int stats_cap, int* n_parts, const mpnn_bn_fuse* bnp,
-                            cudaStream_t st) {
+                            const int* count, cudaStream_t st) {
     const int N = N0 + N1;
     mpnn_bn_fuse bn = {};
     if (bnp) bn = *bnp;
@@ -119,16 +125,16 @@ static int launch_gemm_simt(const void* A0, int K0, const void* A1, int K1, cons
     if (n_parts) *n_parts = stats ? gx : 0;
     if (N % 32 == 0 && N0 % 32 == 0) {
         dim3 grid(gx, N / 32);
-        stencil_gemm_simt<T, TO, 32><<<grid, 128, 0, st>>>((const T*)A0, K0, (const T*)A1, K1, (const T*)Wp,
-            ntaps, bias, (TO*)out0, N0, acc0, (TO*)out1, N1, acc1, g, n_tiles, stats, bn);
+        stencil_gemm_simt<T, TO, 32, CNT><<<grid, 128, 0, st>>>((const T*)A0, K0, (const T*)A1, K1, (const T*)Wp,
+            ntaps, bias, (TO*)out0, N0, acc0, (TO*)out1, N1, acc1, g, n_tiles, stats, bn, count);
     } else if (N % 16 == 0 && N0 % 16 == 0) {
         dim3 grid(gx, N / 16);
-        stencil_gemm_simt<T, TO, 16><<<grid, 128, 0, st>>>((const T*)A0, K0, (const T*)A1, K1, (const T*)Wp,
-            ntaps, bias, (TO*)out0, N0, acc0, (TO*)out1, N1, acc1, g, n_tiles, stats, bn);
+        stencil_gemm_simt<T, TO, 16, CNT><<<grid, 128, 0, st>>>((const T*)A0, K0, (const T*)A1, K1, (const T*)Wp,
+            ntaps, bias, (TO*)out0, N0, acc0, (TO*)out1, N1, acc1, g, n_tiles, stats, bn, count);
     } else {
         dim3 grid(gx, N / 8);
-        stencil_gemm_simt<T, TO, 8><<<grid, 128, 0, st>>>((const T*)A0, K0, (const T*)A1, K1, (const T*)Wp,
-            ntaps, bias, (TO*)out0, N0, acc0, (TO*)out1, N1, acc1, g, n_tiles, stats, bn);
+        stencil_gemm_simt<T, TO, 8, CNT><<<grid, 128, 0, st>>>((const T*)A0, K0, (const T*)A1, K1, (const T*)Wp,
+            ntaps, bias, (TO*)out0, N0, acc0, (TO*)out1, N1, acc1, g, n_tiles, stats, bn, count);
     }
     return mpnn_check_launch("stencil_gemm_simt");
 }
@@ -139,7 +145,7 @@ static int stencil_gemm_impl(const void* A0, int K0, const void* A1, int K1,
                              int B, int H, int W, int G, int P,
                              float* stats, int stats_cap, int* n_parts, const mpnn_bn_fuse* bn,
                              int dtype, int out_dtype, int impl, void* stream,
-                             const mpnn_bn_bwd_epi* bwd = nullptr) {
+                             const mpnn_bn_bwd_epi* bwd = nullptr, const int* count = nullptr) {
     MPNN_REQUIRE(ntaps == 9 || ntaps == 1, "stencil_gemm: ntaps=%d", ntaps);
     MPNN_REQUIRE(!bwd || impl == 1, "conv_dgrad_bn_reduce: only the tcgen05 path fuses the BN-backward sums");
     MPNN_REQUIRE(K0 % 8 == 0 && K1 % 8 == 0 && K0 > 0, "stencil_gemm: K0=%d K1=%d", K0, K1);
@@ -150,16 +156,19 @@ static int stencil_gemm_impl(const void* A0, int K0, const void* A1, int K1,
     MPNN_REQUIRE(G >= halo, "stencil_gemm: front guard %d < %d", G, halo);
     MPNN_REQUIRE(P >= G + ceil_div(g.rows, 128) * 128 + halo, "stencil_gemm: back guard too small (P=%d)", P);
     MPNN_REQUIRE(!stats || stats_cap > 0, "stencil_gemm: stats_cap");
+    MPNN_REQUIRE(!count || (!stats && !bn && !bwd), "stencil_gemm_counted: a counted launch computes no statistics");
     MPNN_REQUIRE(!bn || (bn->acc && bn->gamma && bn->beta && bn->ss && bn->mr && bn->count > 0),
                  "conv_bn_stats: incomplete mpnn_bn_fuse");
     cudaStream_t st = (cudaStream_t)stream;
     if (impl == 1) {
         MPNN_REQUIRE(dtype == MPNN_BF16, "stencil_gemm: tcgen05 path needs bf16 operands");
         return mpnn_stencil_gemm_umma(A0, K0, A1, K1, Wp, ntaps, bias, out0, N0, acc0, out1, N1, acc1,
-                                      g, stats, stats_cap, n_parts, out_dtype, bn, bwd, st);
+                                      g, stats, stats_cap, n_parts, out_dtype, bn, bwd, count, st);
     }
-#define GO(T, TO) return launch_gemm_simt<T, TO>(A0, K0, A1, K1, Wp, ntaps, bias, out0, N0, acc0, out1, N1, \
-                                                 acc1, g, stats, stats_cap, n_parts, bn, st)
+#define GO(T, TO) return count ? launch_gemm_simt<T, TO, true>(A0, K0, A1, K1, Wp, ntaps, bias, out0, N0, acc0, out1,  \
+                                                               N1, acc1, g, stats, stats_cap, n_parts, bn, count, st) \
+                           : launch_gemm_simt<T, TO, false>(A0, K0, A1, K1, Wp, ntaps, bias, out0, N0, acc0, out1,  \
+                                                            N1, acc1, g, stats, stats_cap, n_parts, bn, nullptr, st)
     if (dtype == MPNN_F32 && out_dtype == MPNN_F32) GO(float, float);
     if (dtype == MPNN_BF16 && out_dtype == MPNN_BF16) GO(__nv_bfloat16, __nv_bfloat16);
     if (dtype == MPNN_BF16 && out_dtype == MPNN_F32) GO(__nv_bfloat16, float);
@@ -176,6 +185,16 @@ extern "C" int mpnn_stencil_gemm(const void* A0, int K0, const void* A1, int K1,
                                  int dtype, int out_dtype, int impl, void* stream) {
     return stencil_gemm_impl(A0, K0, A1, K1, Wp, ntaps, bias, out0, N0, acc0, out1, N1, acc1, B, H, W, G, P,
                              stats, stats_cap, n_parts, nullptr, dtype, out_dtype, impl, stream);
+}
+
+extern "C" int mpnn_stencil_gemm_counted(const void* A0, int K0, const void* A1, int K1,
+                                         const void* Wp, int ntaps, const float* bias,
+                                         void* out0, int N0, int acc0, void* out1, int N1, int acc1,
+                                         int B, int H, int W, int G, int P,
+                                         float* stats, int stats_cap, int* n_parts,
+                                         int dtype, int out_dtype, int impl, const int* count, void* stream) {
+    return stencil_gemm_impl(A0, K0, A1, K1, Wp, ntaps, bias, out0, N0, acc0, out1, N1, acc1, B, H, W, G, P,
+                             stats, stats_cap, n_parts, nullptr, dtype, out_dtype, impl, stream, nullptr, count);
 }
 
 extern "C" int mpnn_conv_bn_stats(const void* A0, int K0, const void* A1, int K1,

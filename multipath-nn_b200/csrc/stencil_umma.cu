@@ -51,6 +51,7 @@ struct GemmArgs {
     int dbg;           // tuning aid (MPNN_TUNE_DBG): 1 skip MMAs, 2 skip stores, 4 skip loads; timing probes of the
                        // MMA phase (results wrong by construction): 8 all taps read the unshifted tile, 16 the taps
                        // alternate between the two accumulators, 32 three MMAs of 3x the width instead of nine
+    const int* count;  // CNT instantiations: live batch in device memory (g.B is the capacity the grid was sized for)
 };
 
 constexpr int kThreads = 192;
@@ -84,7 +85,8 @@ __device__ __forceinline__ void unpack_bf16x8(const uint4& u, float* v) {
 // accumulation into the outputs, forward BN moments or no sums (stores without the read-modify-write and
 // output-mode dispatch); 2: the same with the fused BN-backward sums (separate instantiation: the two kinds
 // of sums have different register footprints and the accumulators must not spill).
-template <int NBT, int KS, int EPI>
+// CNT: the live batch is min(*count, g.B); only its rows are computed and stored (counted entry point, inference).
+template <int NBT, int KS, int EPI, bool CNT = false>
 // (32-wide slices at two CTAs per SM: at three the 64 register accumulators of the BN sums spilled -- 96 registers,
 //  16-48 bytes of stack -- and H16 32->32 ran at 53 us instead of 49)
 __global__ void __launch_bounds__(kThreads, NBT == 16 ? (EPI == 2 ? 3 : 4) : (NBT == 32 ? 2 : 1))
@@ -109,6 +111,15 @@ stencil_gemm_umma_kernel(const GemmArgs a) {
     const uint32_t ncols = tmem_cols_pow2(((a.dbg & 32) && NBT ? 6 : 2) * NB);
     constexpr bool FAST = EPI != 0;
     const int stats_mode = EPI == 2 ? 2 : (EPI == 1 ? (a.stats_mode == 1 ? 1 : 0) : a.stats_mode);
+    int n_tiles = a.n_tiles, rows = a.g.rows;
+    if (CNT) {
+        // the count is written by an earlier kernel: wait for it before anything else, and let a CTA without tiles
+        // leave before it sets up barriers or allocates tensor memory (a zero count costs one early return)
+        pdl_wait();
+        rows = min(max(*a.count, 0), a.g.B) * a.g.S;
+        n_tiles = (rows + 127) >> 7;
+        if ((int)blockIdx.x >= n_tiles) return;
+    }
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < a.nstage; ++s) { mbar_init(full0 + 8 * s, 1); mbar_init(empty0 + 8 * s, 1); }
@@ -154,7 +165,7 @@ stencil_gemm_umma_kernel(const GemmArgs a) {
             const __nv_bfloat16* src0 = a.A0 + (size_t)(a.g.G - a.halo) * 8;
             const __nv_bfloat16* src1 = a.A1 ? a.A1 + (size_t)(a.g.G - a.halo) * 8 : nullptr;
             const size_t plane = (size_t)a.g.P * 8;
-            for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x) {
+            for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
                 const size_t toff = (size_t)tile * (128 * 8);
                 for (int ci = 0; ci < a.n_kc; ++ci) {
                     const int kg0 = ci * a.KC, kgn = min(a.KC, KG - kg0);
@@ -192,7 +203,7 @@ stencil_gemm_umma_kernel(const GemmArgs a) {
             const bool skip = (a.dbg & 1) != 0;
             mbar_wait(wbar, 0);
             int s = 0, tl = 0; uint32_t ph = 0;
-            for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x, ++tl) {
+            for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++tl) {
                 const int acc = tl & 1;
                 const uint32_t aph = (uint32_t)(tl >> 1) & 1u;
                 mbar_wait(tempty0 + 8 * acc, aph ^ 1u);
@@ -360,7 +371,7 @@ stencil_gemm_umma_kernel(const GemmArgs a) {
         int dr = 0, rq = 0, qrun = (int)blockIdx.x * 128 + m;
         auto valid_of = [&](int q_, int r_) {
             const int hr = (int)__umulhi((uint32_t)r_, a.g.mWp);     // exact: r < S << 2^32 / Wp
-            return q_ < a.g.rows && r_ >= Wp_ && r_ != hr * Wp_;
+            return q_ < rows && r_ >= Wp_ && r_ != hr * Wp_;
         };
         uint4 lnext[NR / 8 ? NR / 8 : 1];
         auto fetch_lin = [&](int q_, bool v_) {
@@ -381,13 +392,13 @@ stencil_gemm_umma_kernel(const GemmArgs a) {
             if (EPI == 2) fetch_lin(qrun, vrun);
         }
         int it = 0;
-        for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x, ++it) {
+        for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
             const int acc = it & 1;
             const uint32_t aph = (uint32_t)(it >> 1) & 1u;
             const int q = tile * 128 + m;
             const int p = a.g.G + q;
             const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)acc * NB;
-            bool valid, inrange = q < a.g.rows && !(a.dbg & 2);
+            bool valid, inrange = q < rows && !(a.dbg & 2);
             if (FAST && NBT) {
                 valid = vrun;
                 uint4 lrow[NR / 8 ? NR / 8 : 1];
@@ -579,7 +590,7 @@ umma_selftest_kernel(const uint8_t* __restrict__ A, int a_bytes, int a_off, cons
 int mpnn_stencil_gemm_umma(const void* A0, int K0, const void* A1, int K1, const void* Wp, int ntaps,
                            const float* bias, void* out0, int N0, int acc0, void* out1, int N1, int acc1,
                            Geom g, float* stats, int stats_cap, int* n_parts, int out_dtype,
-                           const mpnn_bn_fuse* bn, const mpnn_bn_bwd_epi* bwd, cudaStream_t st) {
+                           const mpnn_bn_fuse* bn, const mpnn_bn_bwd_epi* bwd, const int* count, cudaStream_t st) {
     const int N = N0 + N1;
     MPNN_REQUIRE(K0 % 16 == 0 && K1 % 16 == 0, "stencil_gemm(tcgen05): K0=%d K1=%d must be multiples of 16", K0, K1);
     MPNN_REQUIRE(N % 16 == 0 && N0 % 16 == 0, "stencil_gemm(tcgen05): N0=%d N1=%d must be multiples of 16", N0, N1);
@@ -588,6 +599,7 @@ int mpnn_stencil_gemm_umma(const void* A0, int K0, const void* A1, int K1, const
                  "stencil_gemm(tcgen05): fused BN-backward sums need a plain 9-tap bf16 data gradient");
     MPNN_REQUIRE(!bwd || (bwd->lin && bwd->ss && bwd->mr && bwd->f.acc && bwd->f.sums),
                  "stencil_gemm(tcgen05): incomplete mpnn_bn_bwd_epi");
+    MPNN_REQUIRE(!count || (!bwd && !bn && !stats), "stencil_gemm(tcgen05): a counted launch computes no statistics");
     const int KG = (K0 + K1) / 8;
     static const int tune_halo8 = getenv("MPNN_TUNE_HALO8") ? atoi(getenv("MPNN_TUNE_HALO8")) : 0;
     static const int tune_per_sm = getenv("MPNN_TUNE_PER_SM") ? atoi(getenv("MPNN_TUNE_PER_SM")) : 0;
@@ -674,46 +686,59 @@ int mpnn_stencil_gemm_umma(const void* A0, int K0, const void* A1, int K1, const
     a.ld0 = N0; a.ld1 = N1;
     a.n_tiles = ceil_div(g.rows, 128); a.nstage = nstage;
     a.rowsA = rowsA; a.halo = halo; a.KC = KC; a.n_kc = ceil_div(KG, KC);
+    a.count = count;
     MPNN_REQUIRE(a.out_mode != 2 || (!acc0 && !acc1 && !stats && !bn), "stencil_gemm: row-major output cannot accumulate");
     int gx = 148 * per_sm / split;
     if (gx > a.n_tiles) gx = a.n_tiles;
     if (stats && gx > stats_cap) gx = stats_cap;
     if (gx < 1) gx = 1;
     if (n_parts) *n_parts = stats ? gx : 0;
-    // kernel table: [slice width 16 / 32 / generic][K steps 0 (generic loop), 1..4][epilogue kind]
+    // kernel table: [slice width 16 / 32 / generic][K steps 0 (generic loop), 1..4][epilogue kind]; the counted
+    // instantiations (live batch from device memory) exist for the epilogues without sums only
     typedef void (*Kern)(const GemmArgs);
-    static const Kern generic[3] = {stencil_gemm_umma_kernel<16, 0, 0>, stencil_gemm_umma_kernel<32, 0, 0>,
-                                    stencil_gemm_umma_kernel<0, 0, 0>};
-    static const Kern fast16[2][2] = {{stencil_gemm_umma_kernel<16, 1, 1>, stencil_gemm_umma_kernel<16, 2, 1>},
-                                      {stencil_gemm_umma_kernel<16, 1, 2>, stencil_gemm_umma_kernel<16, 2, 2>}};
-    static const Kern fast32[2][4] = {{stencil_gemm_umma_kernel<32, 1, 1>, stencil_gemm_umma_kernel<32, 2, 1>,
+    static const Kern generic[2][3] = {{stencil_gemm_umma_kernel<16, 0, 0>, stencil_gemm_umma_kernel<32, 0, 0>,
+                                        stencil_gemm_umma_kernel<0, 0, 0>},
+                                       {stencil_gemm_umma_kernel<16, 0, 0, true>, stencil_gemm_umma_kernel<32, 0, 0, true>,
+                                        stencil_gemm_umma_kernel<0, 0, 0, true>}};
+    // [0] forward, [1] fused BN-backward sums, [2] forward, counted
+    static const Kern fast16[3][2] = {{stencil_gemm_umma_kernel<16, 1, 1>, stencil_gemm_umma_kernel<16, 2, 1>},
+                                      {stencil_gemm_umma_kernel<16, 1, 2>, stencil_gemm_umma_kernel<16, 2, 2>},
+                                      {stencil_gemm_umma_kernel<16, 1, 1, true>, stencil_gemm_umma_kernel<16, 2, 1, true>}};
+    static const Kern fast32[3][4] = {{stencil_gemm_umma_kernel<32, 1, 1>, stencil_gemm_umma_kernel<32, 2, 1>,
                                        stencil_gemm_umma_kernel<32, 3, 1>, stencil_gemm_umma_kernel<32, 4, 1>},
                                       {stencil_gemm_umma_kernel<32, 1, 2>, stencil_gemm_umma_kernel<32, 2, 2>,
-                                       stencil_gemm_umma_kernel<32, 3, 2>, stencil_gemm_umma_kernel<32, 4, 2>}};
+                                       stencil_gemm_umma_kernel<32, 3, 2>, stencil_gemm_umma_kernel<32, 4, 2>},
+                                      {stencil_gemm_umma_kernel<32, 1, 1, true>, stencil_gemm_umma_kernel<32, 2, 1, true>,
+                                       stencil_gemm_umma_kernel<32, 3, 1, true>, stencil_gemm_umma_kernel<32, 4, 1, true>}};
     // generic slice width (N >= 48), generic epilogue, unrolled issue loop for the K of the 32..128-channel layers
-    static const Kern wide[5] = {stencil_gemm_umma_kernel<0, 2, 0>, stencil_gemm_umma_kernel<0, 3, 0>,
-                                 stencil_gemm_umma_kernel<0, 4, 0>, stencil_gemm_umma_kernel<0, 6, 0>,
-                                 stencil_gemm_umma_kernel<0, 8, 0>};
-    const int e = bwd ? 1 : 0;
-    Kern kern = generic[NB == 16 ? 0 : (NB == 32 ? 1 : 2)];
+    static const Kern wide[2][5] = {{stencil_gemm_umma_kernel<0, 2, 0>, stencil_gemm_umma_kernel<0, 3, 0>,
+                                     stencil_gemm_umma_kernel<0, 4, 0>, stencil_gemm_umma_kernel<0, 6, 0>,
+                                     stencil_gemm_umma_kernel<0, 8, 0>},
+                                    {stencil_gemm_umma_kernel<0, 2, 0, true>, stencil_gemm_umma_kernel<0, 3, 0, true>,
+                                     stencil_gemm_umma_kernel<0, 4, 0, true>, stencil_gemm_umma_kernel<0, 6, 0, true>,
+                                     stencil_gemm_umma_kernel<0, 8, 0, true>}};
+    const int c = count ? 1 : 0;
+    const int e = bwd ? 1 : 2 * c;
+    Kern kern = generic[c][NB == 16 ? 0 : (NB == 32 ? 1 : 2)];
     if (fast_ok && NB == 16 && ks >= 1 && ks <= 2) kern = fast16[e][ks - 1];
     if (fast_ok && NB == 32 && ks >= 1 && ks <= 4) kern = fast32[e][ks - 1];
     if (!tune_generic && NB != 16 && NB != 32) {
         const int wi = ks == 2 ? 0 : ks == 3 ? 1 : ks == 4 ? 2 : ks == 6 ? 3 : ks == 8 ? 4 : -1;
-        if (wi >= 0) kern = wide[wi];
+        if (wi >= 0) kern = wide[c][wi];
     }
     // the > 48 KB dynamic shared memory opt-in is a per-device function attribute
     static bool attr_set[64] = {};
     int dev = 0;
     cudaGetDevice(&dev);
     if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-        Kern all[20] = {generic[0], generic[1], generic[2]};
-        for (int i = 0; i < 2; ++i) {
-            for (int j = 0; j < 2; ++j) all[3 + 2 * i + j] = fast16[i][j];
-            for (int j = 0; j < 4; ++j) all[7 + 4 * i + j] = fast32[i][j];
-        }
-        for (int j = 0; j < 5; ++j) all[15 + j] = wide[j];
-        for (int i = 0; i < 20; ++i) {
+        constexpr int nk = 6 + 3 * 2 + 3 * 4 + 2 * 5;
+        Kern all[nk];
+        int k = 0;
+        for (int i = 0; i < 2; ++i) for (int j = 0; j < 3; ++j) all[k++] = generic[i][j];
+        for (int i = 0; i < 3; ++i) for (int j = 0; j < 2; ++j) all[k++] = fast16[i][j];
+        for (int i = 0; i < 3; ++i) for (int j = 0; j < 4; ++j) all[k++] = fast32[i][j];
+        for (int i = 0; i < 2; ++i) for (int j = 0; j < 5; ++j) all[k++] = wide[i][j];
+        for (int i = 0; i < nk; ++i) {
             cudaError_t e2 = cudaFuncSetAttribute(all[i], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMax);   // + static smem stays under 227 KB
             if (e2 != cudaSuccess) { mpnn_set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e2)); return MPNN_ERR_CUDA; }
             // without this the driver picks the L1 / shared-memory split heuristically and may leave room for fewer

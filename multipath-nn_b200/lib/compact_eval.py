@@ -20,6 +20,12 @@ The same walk serves routed inference (`predict`, behind `Net.predict`): at a cl
 example's softmax, predicted class, exit leaf and path cost (mpnn_leaf_emit) instead of adding statistics.
 Nets with a per-example k_cpt carry the router feature alpha_cpt * k_cpt through the compaction by original
 example id (mpnn_gather_feature), so one batch may mix cost budgets.
+
+The walk above reads every switch's child batch sizes back to the host, because they are launch parameters of the
+kernels below it.  `RoutedPredictor` (behind `Net.predictor`) runs the same tables through the counted entry points
+instead: every node of the tree is launched in a static order at the capacity `batch`, and each kernel reads its live
+batch from the parent switch's device-side count (zero for the subtrees no example takes).  That walk has no host
+round trip, so it is captured once as a CUDA graph and replayed per call.
 """
 import ctypes
 from types import SimpleNamespace as Ns
@@ -29,7 +35,7 @@ import torch
 
 from lib.engine import BF16, _RT_FWD, _ru, _vp
 
-__all__ = ['CompactEvaluator']
+__all__ = ['CompactEvaluator', 'RoutedPredictor']
 
 
 def _node_ops(nd):
@@ -93,6 +99,10 @@ class CompactEvaluator:
             if nd.kind == 'rcm' and len(eng.nodes[nd.parent].kids) > 1:
                 st = plan.node[nd.idx]
                 self.cin[nd.idx] = [plan.planes(s.C, s.geo) for s in st.pin]
+        # the counted walk runs sibling subtrees concurrently: each router of the CUDA-core heads gets its own k_cpt
+        # feature vector instead of the plan's shared `kextra`
+        self._kext = {i: torch.zeros(B, dtype=torch.float32, device=dev) for i in plan.rtr} \
+            if self.dyn_k and not plan.umma_heads else {}
         n_leaf = len(eng.regs)
         self.acc = torch.zeros((n_leaf, 2 + 2 * self.n_cls), dtype=torch.float64, device=dev)
         self.visits = np.zeros(len(eng.nodes), np.int64)
@@ -131,6 +141,13 @@ class CompactEvaluator:
             return None
         if k_cpt is None:
             raise ValueError('this net routes on a per-example k_cpt: pass k_cpt (a scalar, one value or n values)')
+        if isinstance(k_cpt, torch.Tensor) and k_cpt.is_cuda:      # stays on the device (no host round trip)
+            kc = k_cpt.to(torch.float32).reshape(-1)
+            if kc.numel() == 1:
+                kc = kc.expand(n)
+            if kc.numel() != n:
+                raise ValueError('k_cpt: %d values for %d examples' % (kc.numel(), n))
+            return kc * float(np.float32(hy.α_cpt))                 # fp32 product, as below
         kc = np.asarray(k_cpt, dtype=np.float32).reshape(-1)
         if kc.size == 1:
             kc = np.full(n, kc[0], np.float32)
@@ -173,13 +190,17 @@ class CompactEvaluator:
             self.n_seen += n
             self._walk(x0, n, kf)
 
+    def _check_x0(self, x0):
+        hy = self.eng.net.hypers
+        if tuple(x0.shape[1:]) != tuple(hy.x0_shape):
+            raise ValueError('x0: shape %s, expected (n,) + %s' % (tuple(x0.shape), tuple(hy.x0_shape)))
+        return int(x0.shape[0])
+
     def predict(self, x0, k_cpt=None):
         """Routed inference (see `Net.predict`): Ns(cls, prob, exit, ops) of numpy arrays, one row per example of x0
         (any n, host or device), run in chunks of `batch` examples."""
-        eng, hy = self.eng, self.eng.net.hypers
-        n = int(x0.shape[0])
-        if tuple(x0.shape[1:]) != tuple(hy.x0_shape):
-            raise ValueError('x0: shape %s, expected (n,) + %s' % (tuple(x0.shape), tuple(hy.x0_shape)))
+        eng = self.eng
+        n = self._check_x0(x0)
         kf = self._k_feature(k_cpt, n)
         nc = self.n_cls
         # one byte buffer holds the four outputs, so that one device-to-host copy returns them
@@ -193,7 +214,7 @@ class CompactEvaluator:
             with torch.cuda.device(eng.dev):
                 self._prepare()                      # every call: the current parameters and running moments
                 buf = torch.empty(nbytes, dtype=torch.uint8, device=eng.dev)
-                kfd = torch.from_numpy(kf).to(eng.dev, non_blocking=True) if kf is not None else None
+                kfd = torch.as_tensor(kf).to(eng.dev, non_blocking=True) if kf is not None else None
                 base_ptr = buf.data_ptr()
                 visits = self.visits.copy()          # node visits belong to the statistics of the data set
                 try:
@@ -290,6 +311,98 @@ class CompactEvaluator:
             self._node(eng.nodes[kid], counts[s], sw['orig'][s], sw['pos'][s], sw['count'][s:s + 1])
 
     # ------------------------------------------------------------------ #
+    def _counted_walk(self, n_dev, out, fork):
+        """The whole tree at capacity B with the live batch sizes on the device: n_dev (int32 [1]) is the chunk's count,
+        every switch writes its sinks' counts, and every kernel takes its batch from one of them.  No host read.
+        out: Ns of the output pointers (leaf_emit).  fork(key) -> a side stream for the subtree of one sink."""
+        eng, plan, L, B = self.eng, self.plan, self.L, self.B
+        hy = eng.net.hypers
+        H0, W0, C0 = hy.x0_shape
+        main = torch.cuda.current_stream(eng.dev)
+        S = ctypes.c_void_p(main.cuda_stream)
+        for i, slot in enumerate(plan.node[0].out):
+            L.pack_input_counted(_vp(plan.x0), B, H0, W0, C0, 2 ** i, _vp(slot.t), min(slot.C, (C0 + 7) // 8 * 8),
+                                 slot.geo.G, slot.geo.P, eng.dtype, _vp(n_dev), S)
+        joins = []
+        for k in eng.nodes[0].kids:
+            self._cnode(eng.nodes[k], n_dev, None, None, None, main, out, fork, joins)
+        for st in joins:                             # every side stream rejoins the origin (required under capture)
+            main.wait_stream(st)
+
+    def _cnode(self, nd, cnt, orig, pos, pcnt, stream, out, fork, joins):
+        """node `nd` on `stream` with its live count at cnt (device int32 [1]); orig / pos: the examples' original ids
+        and rows in the parent's compact batch (None = identity, no switch above); pcnt: the parent's count"""
+        eng, plan, L, B = self.eng, self.plan, self.L, self.B
+        dt = eng.dtype
+        S = ctypes.c_void_p(stream.cuda_stream)
+        if nd.kind == 'reg':
+            par = eng.nodes[nd.parent]
+            r = plan.reg[nd.idx]
+            if not plan.umma_heads:
+                pst = plan.node[par.idx]
+                L.fc_fwd_counted(_vp(pst.feat), pst.F, plan.Balloc, B, eng.tptr(r.fc.params.w), eng.tptr(r.fc.params.b),
+                                 None, self.n_cls, _vp(r.Zbuf), dt, _vp(pcnt if pcnt is not None else cnt), S)
+            no = self.leaf_no[nd.idx]
+            L.leaf_emit(_vp(r.Zbuf), r.ldz, self.n_cls, _vp(pos), _vp(orig), _vp(cnt), B, no, self.path_ops[no],
+                        ctypes.c_void_p(out.prob), ctypes.c_void_p(out.cls), ctypes.c_void_p(out.exit),
+                        ctypes.c_void_p(out.ops), S)
+            return
+        st = plan.node[nd.idx]
+        ins = [s.t for s in st.pin]
+        if pos is not None:
+            for slot, dst in zip(st.pin, self.cin[nd.idx]):
+                g = slot.geo
+                L.gather_images(_vp(slot.t), B, g.P, _vp(pos), _vp(cnt), _vp(dst), B, g.P, slot.C, g.H, g.W, g.G, dt, S)
+            ins = self.cin[nd.idx]
+        rt = plan.rtr.get(nd.idx)
+        if self.dyn_k and rt is not None:
+            if plan.umma_heads:
+                L.gather_feature(_vp(self.kfeat), _vp(orig), _vp(cnt), B, None, _vp(st.feat[st.F // 8, :, 0]), 8, dt, S)
+            else:                                    # a vector per router: sibling subtrees run concurrently
+                L.gather_feature(_vp(self.kfeat), _vp(orig), _vp(cnt), B, _vp(self._kext[nd.idx]), None, 0, 0, S)
+        for k, sc in enumerate(st.sc):
+            g = sc.geo
+            prev = st.sc[k - 1] if k > 0 else None
+            L.stencil_gemm_counted(_vp(ins[k]), sc.K0, _vp(prev.pooled) if prev is not None else None, sc.K1, _vp(sc.Wf),
+                                   9, eng.tptr(sc.bk), _vp(sc.lin), sc.N, 0, None, 0, 0, B, g.H, g.W, g.G, g.P,
+                                   None, 0, None, dt, dt, eng.impl, _vp(cnt), S)
+            if sc.live or sc.pooled is not None:
+                L.bn_relu_pool_fwd_counted(_vp(sc.lin), sc.N, B, g.H, g.W, g.G, g.P, _vp(sc.ss) if sc.live else None,
+                                           _vp(sc.act), _vp(sc.pooled), sc.geo_p.P if sc.pooled is not None else 0,
+                                           _vp(sc.feat), plan.Balloc, dt, _vp(cnt), S)
+        if not nd.kids:
+            return
+        if plan.umma_heads and nd.idx in plan.heads:
+            hd = plan.heads[nd.idx]
+            outs = ([(hd.Z16, 16)] if hd.leaf_off is not None else []) + ([(rt.Z1, 16)] if rt is not None else [])
+            outs.append((None, 0))
+            (o0, n0), (o1, n1) = outs[0], outs[1]
+            L.stencil_gemm_counted(_vp(st.feat), st.Fext, None, 0, _vp(hd.Wfc), 1, _vp(hd.bias), _vp(o0), n0, 0,
+                                   _vp(o1), n1, 0, B, 0, 0, 0, plan.Balloc, None, 0, None, BF16, 2, 1, _vp(cnt), S)
+        elif rt is not None:
+            L.fc_fwd_counted(_vp(st.feat), st.F, plan.Balloc, B, eng.tptr(rt.fc1.params.w), eng.tptr(rt.fc1.params.b),
+                             _vp(self._kext[nd.idx]) if self.dyn_k else None, 16, _vp(rt.Z1), dt, _vp(cnt), S)
+        if len(nd.kids) == 1:
+            self._cnode(eng.nodes[nd.kids[0]], cnt, orig, None, cnt, stream, out, fork, joins)
+            return
+        sw = self.sw[nd.idx]
+        ns = len(nd.kids)
+        L.router_tail_fwd_batched_counted(_vp(sw['tab']), 1, B, 16, float(rt.bn1.hypers.d), float(rt.bn1.hypers.ε), 0,
+                                          _vp(cnt), S)
+        L.route_compact_counted(_vp(rt.R), ns, ns, B, _vp(orig), B, None, _vp(sw['pos']), _vp(sw['orig']),
+                                _vp(sw['count']), _vp(cnt), S)
+        # sink 0 continues on this stream, the others fork: the graph's critical path is one root-to-leaf chain
+        ev = torch.cuda.Event()
+        ev.record(stream)
+        for s, kid in enumerate(nd.kids):
+            st2 = stream
+            if s > 0:
+                st2 = fork((nd.idx, s))
+                st2.wait_event(ev)
+                joins.append(st2)
+            self._cnode(eng.nodes[kid], sw['count'][s:s + 1], sw['orig'][s], sw['pos'][s], cnt, st2, out, fork, joins)
+
+    # ------------------------------------------------------------------ #
     def result(self):
         """{(object, name): mean over the data set} in `mean_net_state`'s form (desc.py:10-22) for the exact keys"""
         eng = self.eng
@@ -313,3 +426,82 @@ class CompactEvaluator:
         out[(eng.net, 'acc')] = acc
         out[(eng.net, 'moc')] = moc / n
         return out
+
+
+class RoutedPredictor:
+    """Routed inference as one CUDA graph (see `Net.predictor`).  `p(x0, k_cpt=None)` runs n <= batch examples and
+    returns Ns(cls, prob, exit, ops) of device tensors with the dtypes and meaning of `Net.predict`.  They are views
+    [:n] of the predictor's own output buffers: the next call overwrites them (clone what you keep).
+
+    A call copies x0 into the walk's input buffer, writes n and the per-example router feature with device copies,
+    and replays the graph on the current stream: with device inputs it does not synchronise the host.  The graph
+    starts with the weight packing and the BatchNorm constants of the running moments (what `predict` runs before its
+    walk), so every call sees the current parameters."""
+
+    def __init__(self, ev):
+        self.ev, eng = ev, ev.eng
+        self.B = ev.B
+        dev = eng.dev
+        B, nc = ev.B, ev.n_cls
+        self.n_dev = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.cls = torch.zeros(B, dtype=torch.int32, device=dev)
+        self.prob = torch.zeros((B, nc), dtype=torch.float32, device=dev)
+        self.exit = torch.zeros(B, dtype=torch.int32, device=dev)
+        self.ops = torch.zeros(B, dtype=torch.float64, device=dev)
+        self._out = Ns(prob=self.prob.data_ptr(), cls=self.cls.data_ptr(), exit=self.exit.data_ptr(),
+                       ops=self.ops.data_ptr())
+        self._side = {}
+        self.graph = None
+        self.graph_launches = 0
+
+    def _fork(self, key):
+        if key not in self._side:
+            self._side[key] = torch.cuda.Stream(self.ev.eng.dev)
+        return self._side[key]
+
+    def _ops(self):
+        self.ev._prepare()
+        self.ev._counted_walk(self.n_dev, self._out, self._fork)
+
+    def _capture(self):
+        import gc
+        eng = self.ev.eng
+        s = torch.cuda.Stream(eng.dev)
+        s.wait_stream(torch.cuda.current_stream(eng.dev))
+        with torch.cuda.stream(s):               # warm-up: lazy module loads and per-kernel attributes stay out of capture
+            self._ops()
+        torch.cuda.current_stream(eng.dev).wait_stream(s)
+        torch.cuda.synchronize(eng.dev)
+        g = torch.cuda.CUDAGraph()
+        before = eng.L.launches
+        # no cyclic garbage collection inside capture (see Engine._capture)
+        gc.collect()
+        gc_was_on = gc.isenabled()
+        gc.disable()
+        try:
+            with torch.cuda.graph(g):
+                self._ops()
+        finally:
+            if gc_was_on:
+                gc.enable()
+        self.graph_launches = eng.L.launches - before
+        self.graph = g
+
+    def __call__(self, x0, k_cpt=None):
+        ev = self.ev
+        eng = ev.eng
+        n = ev._check_x0(x0)
+        if n > self.B:
+            raise ValueError('batch %d > predictor capacity %d' % (n, self.B))
+        kf = ev._k_feature(k_cpt, n)
+        if n > 0:
+            with torch.cuda.device(eng.dev):
+                if self.graph is None:
+                    self._capture()
+                hy = eng.net.hypers
+                ev.plan.x0[:n].copy_(eng._to_dev(x0, (n,) + tuple(hy.x0_shape), 'x0'), non_blocking=True)
+                if kf is not None:
+                    ev.kfeat[:n].copy_(torch.as_tensor(kf), non_blocking=True)
+                self.n_dev.fill_(n)
+                self.graph.replay()
+        return Ns(cls=self.cls[:n], prob=self.prob[:n], exit=self.exit[:n], ops=self.ops[:n])

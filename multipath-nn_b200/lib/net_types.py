@@ -140,6 +140,19 @@ class Net:
         call between training steps sees the current parameters."""
         return self.compact_evaluator(batch).predict(x0, k_cpt)
 
+    def predictor(self, batch=4096):
+        """Routed inference replayed as one CUDA graph (lib/compact_eval.py, RoutedPredictor), cached per capacity.
+        `p = net.predictor(batch)`; `p(x0, k_cpt=None)` takes n <= batch examples (host or device) and returns the
+        Ns(cls, prob, exit, ops) of `predict` as DEVICE torch tensors -- views [:n] of the predictor's output buffers,
+        overwritten by the next call.  With device inputs a call does not synchronise the host.  The checks, the
+        refused compositions and the use of the current parameters are those of `predict`; n > batch raises
+        ValueError.  The graph is captured on the first call with n > 0."""
+        cache = self.__dict__.setdefault('_predictors', {})
+        if batch not in cache:
+            from lib.compact_eval import RoutedPredictor
+            cache[batch] = RoutedPredictor(self.compact_evaluator(batch))
+        return cache[batch]
+
     def eval_stats(self, feed_dict):
         """Per-example `state_tensors` (train-nets:111-130) for one batch, as a
         dict {(net|layer, name): ndarray}; `mode` defaults to 'ev'."""
