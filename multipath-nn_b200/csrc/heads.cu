@@ -49,25 +49,24 @@ fc_fwd_kernel(const T* __restrict__ X, int F, int Balloc, int B, const float* __
     }
 }
 
-extern "C" int mpnn_fc_fwd(const void* X, int F, int Balloc, int B, const float* W, const float* bias,
-                           const float* extra, int n, float* Z, int dtype, void* stream) {
+extern "C" int mpnn_fc_fwd_counted(const void* X, int F, int Balloc, int B, const float* W, const float* bias,
+                                   const float* extra, int n, float* Z, int dtype, const int* count, void* stream) {
     MPNN_REQUIRE(F % 8 == 0 && n >= 1 && n <= FC_NMAX, "fc_fwd: F=%d n=%d (n<=%d)", F, n, FC_NMAX);
     MPNN_REQUIRE(B >= 1 && Balloc >= B, "fc_fwd: B=%d Balloc=%d", B, Balloc);
     dim3 block(32, 8), grid(ceil_div(B, 32));
-    MPNN_DISPATCH_DTYPE(dtype, (fc_fwd_kernel<T><<<grid, block, 0, (cudaStream_t)stream>>>(
-        (const T*)X, F, Balloc, B, W, bias, extra, n, Z, nullptr)));
+    if (count) {
+        MPNN_DISPATCH_DTYPE(dtype, (fc_fwd_kernel<T, true><<<grid, block, 0, (cudaStream_t)stream>>>(
+            (const T*)X, F, Balloc, B, W, bias, extra, n, Z, count)));
+    } else {
+        MPNN_DISPATCH_DTYPE(dtype, (fc_fwd_kernel<T, false><<<grid, block, 0, (cudaStream_t)stream>>>(
+            (const T*)X, F, Balloc, B, W, bias, extra, n, Z, nullptr)));
+    }
     return mpnn_check_launch("fc_fwd");
 }
 
-extern "C" int mpnn_fc_fwd_counted(const void* X, int F, int Balloc, int B, const float* W, const float* bias,
-                                   const float* extra, int n, float* Z, int dtype, const int* count, void* stream) {
-    if (!count) return mpnn_fc_fwd(X, F, Balloc, B, W, bias, extra, n, Z, dtype, stream);
-    MPNN_REQUIRE(F % 8 == 0 && n >= 1 && n <= FC_NMAX, "fc_fwd: F=%d n=%d (n<=%d)", F, n, FC_NMAX);
-    MPNN_REQUIRE(B >= 1 && Balloc >= B, "fc_fwd: B=%d Balloc=%d", B, Balloc);
-    dim3 block(32, 8), grid(ceil_div(B, 32));
-    MPNN_DISPATCH_DTYPE(dtype, (fc_fwd_kernel<T, true><<<grid, block, 0, (cudaStream_t)stream>>>(
-        (const T*)X, F, Balloc, B, W, bias, extra, n, Z, count)));
-    return mpnn_check_launch("fc_fwd_counted");
+extern "C" int mpnn_fc_fwd(const void* X, int F, int Balloc, int B, const float* W, const float* bias,
+                           const float* extra, int n, float* Z, int dtype, void* stream) {
+    return mpnn_fc_fwd_counted(X, F, Balloc, B, W, bias, extra, n, Z, dtype, nullptr, stream);
 }
 
 // ---------------------------------------------------------- fc backward data

@@ -682,22 +682,18 @@ route_compact_kernel(const float* __restrict__ R, int ldr, int ns, int n_max, co
     if (threadIdx.x < ns) count[threadIdx.x] = base_s[threadIdx.x];
 }
 
-extern "C" int mpnn_route_compact(const float* R, int ldr, int ns, int n, const int* parent_orig, int cap,
-                                  int* dec, int* pos, int* orig, int* count, void* stream) {
-    MPNN_REQUIRE(R && pos && orig && count && ns >= 1 && ns <= 8 && n >= 0 && cap >= n && ldr >= ns,
-                 "route_compact: ns=%d n=%d cap=%d ldr=%d", ns, n, cap, ldr);
-    route_compact_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(R, ldr, ns, n, parent_orig, cap, dec, pos, orig, count,
-                                                               nullptr);
-    return mpnn_check_launch("route_compact");
-}
-
 extern "C" int mpnn_route_compact_counted(const float* R, int ldr, int ns, int n, const int* parent_orig, int cap,
                                           int* dec, int* pos, int* orig, int* count, const int* n_count, void* stream) {
     MPNN_REQUIRE(R && pos && orig && count && ns >= 1 && ns <= 8 && n >= 0 && cap >= n && ldr >= ns,
                  "route_compact: ns=%d n=%d cap=%d ldr=%d", ns, n, cap, ldr);
     route_compact_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(R, ldr, ns, n, parent_orig, cap, dec, pos, orig, count,
                                                                n_count);
-    return mpnn_check_launch("route_compact_counted");
+    return mpnn_check_launch("route_compact");
+}
+
+extern "C" int mpnn_route_compact(const float* R, int ldr, int ns, int n, const int* parent_orig, int cap,
+                                  int* dec, int* pos, int* orig, int* count, void* stream) {
+    return mpnn_route_compact_counted(R, ldr, ns, n, parent_orig, cap, dec, pos, orig, count, nullptr, stream);
 }
 
 // Leaf statistics of the examples routed to one classifier (train-nets:117-130 with p_ev one-hot):

@@ -21,11 +21,15 @@ example's softmax, predicted class, exit leaf and path cost (mpnn_leaf_emit) ins
 Nets with a per-example k_cpt carry the router feature alpha_cpt * k_cpt through the compaction by original
 example id (mpnn_gather_feature), so one batch may mix cost budgets.
 
-The walk above reads every switch's child batch sizes back to the host, because they are launch parameters of the
-kernels below it.  `RoutedPredictor` (behind `Net.predictor`) runs the same tables through the counted entry points
-instead: every node of the tree is launched in a static order at the capacity `batch`, and each kernel reads its live
-batch from the parent switch's device-side count (zero for the subtrees no example takes).  That walk has no host
-round trip, so it is captured once as a CUDA graph and replayed per call.
+One walker serves both ways of running the tree.  Every kernel takes its live batch as a pair (launch batch,
+device count) through the counted entry points, and only the step at a switch differs:
+  * host-synced (`run_batch`, `predict`): a node runs at its batch n with no count (the uncounted launch).  A switch
+    reads its sinks' counts back to the host, because they are the launch batches below it, and walks the non-empty
+    sinks on the same stream.
+  * graph (`RoutedPredictor`, behind `Net.predictor`): every node is launched in a static order at the capacity
+    `batch` and reads its live batch from the parent switch's device-side count (zero for the subtrees no example
+    takes).  Sinks 1.. of a switch fork side streams.  The walk has no host round trip, so it is captured once as a
+    CUDA graph and replayed per call.
 """
 import ctypes
 from types import SimpleNamespace as Ns
@@ -33,13 +37,46 @@ from types import SimpleNamespace as Ns
 import numpy as np
 import torch
 
-from lib.engine import BF16, _RT_FWD, _ru, _vp
+from lib.engine import BF16, _RT_FWD, _gc_off, _vp
 
 __all__ = ['CompactEvaluator', 'RoutedPredictor']
 
 
 def _node_ops(nd):
     return nd.layer.n_ops + (nd.router.n_ops if nd.router is not None else 0)
+
+
+class _LeafStats:
+    """leaf action of `run_batch`: count every node's examples in `visits` and add each classifier's statistics"""
+    def __init__(self, ev):
+        self.ev = ev
+
+    def visit(self, nd, n):
+        self.ev.visits[nd.idx] += n
+
+    def __call__(self, nd, n, orig, pos, sink_cnt, S):
+        ev = self.ev
+        r = ev.plan.reg[nd.idx]
+        ev.L.leaf_stats(_vp(r.Zbuf), r.ldz, ev.n_cls, _vp(ev.plan.y), _vp(pos), _vp(orig), _vp(sink_cnt), n,
+                        _vp(ev.acc[nd.err]), S)
+
+
+class _LeafEmit:
+    """leaf action of prediction: write the results of the examples that exit at each classifier to four device
+    arrays, given by the addresses of their first rows"""
+    def __init__(self, ev, prob, cls, exit, ops):
+        self.ev = ev
+        self.out = [ctypes.c_void_p(p) for p in (prob, cls, exit, ops)]
+
+    def visit(self, nd, n):
+        pass
+
+    def __call__(self, nd, n, orig, pos, sink_cnt, S):
+        ev = self.ev
+        r = ev.plan.reg[nd.idx]
+        no = ev.leaf_no[nd.idx]
+        ev.L.leaf_emit(_vp(r.Zbuf), r.ldz, ev.n_cls, _vp(pos), _vp(orig), _vp(sink_cnt), n, no, ev.path_ops[no],
+                       *self.out, S)
 
 
 class CompactEvaluator:
@@ -62,7 +99,7 @@ class CompactEvaluator:
         B = self.B
         dev = eng.dev
         self.dyn_k = eng.dynamic and bool(eng.net.hypers.dyn_k_cpt)
-        # alpha_cpt * k_cpt of the chunk's examples by original id (the dense path's plan.kextra)
+        # alpha_cpt * k_cpt of the chunk's examples by original id (the dense path's router feature)
         self.kfeat = torch.zeros(B, dtype=torch.float32, device=dev) if self.dyn_k else None
         # per classifier: its index in `net.leaves` and the ops of the nodes on its root-to-leaf path, summed in node
         # order like the dense `moc` (Engine.eval_stats) with a one-hot p_ev
@@ -77,7 +114,6 @@ class CompactEvaluator:
             for i in sorted(on_path):
                 tot += float(_node_ops(eng.nodes[i]))
             self.path_ops.append(tot)
-        self._emit = None                     # None: the leaves add statistics; else the output arrays of predict
         zi = lambda *shape: torch.zeros(shape, dtype=torch.int32, device=dev)
         self.sw = {}
         for nd in eng.nodes:
@@ -99,8 +135,8 @@ class CompactEvaluator:
             if nd.kind == 'rcm' and len(eng.nodes[nd.parent].kids) > 1:
                 st = plan.node[nd.idx]
                 self.cin[nd.idx] = [plan.planes(s.C, s.geo) for s in st.pin]
-        # the counted walk runs sibling subtrees concurrently: each router of the CUDA-core heads gets its own k_cpt
-        # feature vector instead of the plan's shared `kextra`
+        # each router of the CUDA-core heads gets its own k_cpt feature vector: in the graph, sibling subtrees run
+        # concurrently
         self._kext = {i: torch.zeros(B, dtype=torch.float32, device=dev) for i in plan.rtr} \
             if self.dyn_k and not plan.umma_heads else {}
         n_leaf = len(eng.regs)
@@ -155,22 +191,30 @@ class CompactEvaluator:
             raise ValueError('k_cpt: %d values for %d examples' % (kc.size, n))
         return kc * np.float32(hy.α_cpt)
 
-    def _walk(self, x0, n, kf):
-        """run the chunk x0 (n <= batch examples, host or device) down the tree; kf: its router features or None"""
-        eng, plan, L = self.eng, self.plan, self.L
-        hy = eng.net.hypers
-        plan.x0[:n].copy_(eng._to_dev(x0, (n,) + tuple(hy.x0_shape), 'x0'), non_blocking=True)
+    def _load(self, x0, n, kf):
+        """copy the chunk x0 (n <= batch examples, host or device) and its router features kf (or None) into the
+        walk's input buffers"""
+        eng = self.eng
+        self.plan.x0[:n].copy_(eng._to_dev(x0, (n,) + tuple(eng.net.hypers.x0_shape), 'x0'), non_blocking=True)
         if kf is not None:
             self.kfeat[:n].copy_(torch.as_tensor(kf), non_blocking=True)
+
+    def _walk(self, live, leaf, split):
+        """run the loaded chunk down the tree on the current stream.  live: its (launch batch, device count), (n, None)
+        or (B, count of the chunk); leaf: the leaf action; split: the switch step"""
+        eng, plan = self.eng, self.plan
+        H0, W0, C0 = eng.net.hypers.x0_shape
+        stream = torch.cuda.current_stream(eng.dev)
+        S = ctypes.c_void_p(stream.cuda_stream)
+        for i, slot in enumerate(plan.node[0].out):
+            self.L.pack_input_counted(_vp(plan.x0), live[0], H0, W0, C0, 2 ** i, _vp(slot.t),
+                                      min(slot.C, (C0 + 7) // 8 * 8), slot.geo.G, slot.geo.P, eng.dtype, _vp(live[1]), S)
         root = eng.nodes[0]
-        st = plan.node[0]
-        H0, W0, C0 = hy.x0_shape
-        for i, slot in enumerate(st.out):
-            L.pack_input(_vp(plan.x0), n, H0, W0, C0, 2 ** i, _vp(slot.t), min(slot.C, (C0 + 7) // 8 * 8), slot.geo.G, slot.geo.P,
-                         eng.dtype, self._S())
-        self.visits[0] += n
+        leaf.visit(root, live[0])
+        if live[0] == 0:                            # run_batch of no examples
+            return
         for k in root.kids:
-            self._node(eng.nodes[k], n, None, None, None)
+            self._node(eng.nodes[k], live, live, None, None, live[1], stream, leaf, split)
 
     def run_batch(self, x0, y, k_cpt=None):
         """accumulate the statistics of one batch (n <= batch examples; host or device arrays).  k_cpt (nets with a
@@ -188,7 +232,8 @@ class CompactEvaluator:
             y = eng._to_dev(y, (n,) + tuple(eng.net.hypers.y_shape), 'y')
             plan.y[:n].copy_(y, non_blocking=True)
             self.n_seen += n
-            self._walk(x0, n, kf)
+            self._load(x0, n, kf)
+            self._walk((n, None), _LeafStats(self), self._host_split)
 
     def _check_x0(self, x0):
         hy = self.eng.net.hypers
@@ -215,159 +260,69 @@ class CompactEvaluator:
                 self._prepare()                      # every call: the current parameters and running moments
                 buf = torch.empty(nbytes, dtype=torch.uint8, device=eng.dev)
                 kfd = torch.as_tensor(kf).to(eng.dev, non_blocking=True) if kf is not None else None
-                base_ptr = buf.data_ptr()
-                visits = self.visits.copy()          # node visits belong to the statistics of the data set
-                try:
-                    for b0 in range(0, n, self.B):
-                        m = min(self.B, n - b0)
-                        self._emit = Ns(prob=base_ptr + o_prob + 4 * nc * b0, cls=base_ptr + o_cls + 4 * b0,
-                                        exit=base_ptr + o_exit + 4 * b0, ops=base_ptr + 8 * b0)
-                        self._walk(x0[b0:b0 + m], m, kfd[b0:b0 + m] if kfd is not None else None)
-                finally:
-                    self._emit = None
-                    self.visits[:] = visits
+                p = buf.data_ptr()
+                for b0 in range(0, n, self.B):
+                    m = min(self.B, n - b0)
+                    self._load(x0[b0:b0 + m], m, kfd[b0:b0 + m] if kfd is not None else None)
+                    emit = _LeafEmit(self, p + o_prob + 4 * nc * b0, p + o_cls + 4 * b0, p + o_exit + 4 * b0, p + 8 * b0)
+                    self._walk((m, None), emit, self._host_split)
                 host = buf.cpu().numpy()
         return Ns(cls=host[o_cls:o_exit].view(np.int32), prob=host[o_prob:o_cls].view(np.float32).reshape(n, nc),
                   exit=host[o_exit:nbytes].view(np.int32), ops=host[:o_prob].view(np.float64))
 
+    def _host_split(self, nd, sw, stream):
+        """switch step of the host-synced walk: the sinks' counts are the launch batches below them, so they are read
+        back; the non-empty sinks run one after another on the switch's stream"""
+        sw['host'].copy_(sw['count'], non_blocking=True)
+        stream.synchronize()
+        for s, c in enumerate(sw['host'].tolist()):
+            if c:
+                yield s, (c, None), stream
+
     # ------------------------------------------------------------------ #
-    def _node(self, nd, n, orig, pos, count_dev):
-        """evaluate node `nd` on the n examples routed to it.  orig: device list of their original ids
-        (None = identity); pos / count_dev: their rows in the parent's compact batch (None = all of them)."""
+    def _node(self, nd, live, par, orig, pos, sink_cnt, stream, leaf, split):
+        """Run node `nd` and its subtree on `stream`.  live / par: the (launch batch, device count or None) of this
+        node's examples and of its parent's compact batch; orig / pos: the examples' original ids and rows in the
+        parent's compact batch (None = identity, no switch above); sink_cnt: the device count of the switch sink (or
+        of the chunk) the examples come from, which the gathers and the leaf action read; leaf: the leaf action;
+        split(nd, sw, stream): the switch step, yields (sink, its live pair, its stream) for the sinks to run."""
         eng, plan, L = self.eng, self.plan, self.L
-        if n == 0:
-            return
-        self.visits[nd.idx] += n
+        dt = eng.dtype
+        n, cnt = live
+        S = ctypes.c_void_p(stream.cuda_stream)
+        leaf.visit(nd, n)
         if nd.kind == 'reg':
-            par = eng.nodes[nd.parent]
-            r = plan.reg[nd.idx]
             if not plan.umma_heads:
-                pst = plan.node[par.idx]
+                pst = plan.node[nd.parent]
+                r = plan.reg[nd.idx]
                 # logits of the parent's compact batch (rows of the examples that exit here are read through pos)
-                L.fc_fwd(_vp(pst.feat), pst.F, plan.Balloc, self._n_parent, eng.tptr(r.fc.params.w),
-                         eng.tptr(r.fc.params.b), None, self.n_cls, _vp(r.Zbuf), eng.dtype, self._S())
-            o = self._emit
-            if o is None:
-                L.leaf_stats(_vp(r.Zbuf), r.ldz, self.n_cls, _vp(plan.y), _vp(pos), _vp(orig), _vp(count_dev), n,
-                             _vp(self.acc[nd.err]), self._S())
-            else:
-                V = ctypes.c_void_p
-                L.leaf_emit(_vp(r.Zbuf), r.ldz, self.n_cls, _vp(pos), _vp(orig), _vp(count_dev), n,
-                            self.leaf_no[nd.idx], self.path_ops[self.leaf_no[nd.idx]],
-                            V(o.prob), V(o.cls), V(o.exit), V(o.ops), self._S())
+                L.fc_fwd_counted(_vp(pst.feat), pst.F, plan.Balloc, par[0], eng.tptr(r.fc.params.w),
+                                 eng.tptr(r.fc.params.b), None, self.n_cls, _vp(r.Zbuf), dt, _vp(par[1]), S)
+            leaf(nd, n, orig, pos, sink_cnt, S)
             return
         st = plan.node[nd.idx]
-        dt, impl = eng.dtype, eng.impl
         ins = [s.t for s in st.pin]
         if pos is not None:                         # below a switch: gather the inputs of the examples that continue
-            for k, (slot, dst) in enumerate(zip(st.pin, self.cin[nd.idx])):
+            for slot, dst in zip(st.pin, self.cin[nd.idx]):
                 g = slot.geo
-                L.gather_images(_vp(slot.t), self._n_parent, g.P, _vp(pos), _vp(count_dev), _vp(dst), n, g.P,
-                                slot.C, g.H, g.W, g.G, dt, self._S())
+                L.gather_images(_vp(slot.t), par[0], g.P, _vp(pos), _vp(sink_cnt), _vp(dst), n, g.P, slot.C, g.H, g.W,
+                                g.G, dt, S)
             ins = self.cin[nd.idx]
         rt = plan.rtr.get(nd.idx)
         if self.dyn_k and rt is not None:           # the router's k_cpt feature, in this node's compact order
             if plan.umma_heads:                      # channel 0 of the extra planes of the head GEMM's input
-                L.gather_feature(_vp(self.kfeat), _vp(orig), _vp(count_dev), n, None, _vp(st.feat[st.F // 8, :, 0]), 8,
-                                 dt, self._S())
+                L.gather_feature(_vp(self.kfeat), _vp(orig), _vp(sink_cnt), n, None, _vp(st.feat[st.F // 8, :, 0]), 8,
+                                 dt, S)
             else:
-                L.gather_feature(_vp(self.kfeat), _vp(orig), _vp(count_dev), n, _vp(plan.kextra), None, 0, 0, self._S())
-        for k, sc in enumerate(st.sc):
-            g = sc.geo
-            prev = st.sc[k - 1] if k > 0 else None
-            L.stencil_gemm(_vp(ins[k]), sc.K0, _vp(prev.pooled) if prev is not None else None, sc.K1, _vp(sc.Wf), 9,
-                           eng.tptr(sc.bk), _vp(sc.lin), sc.N, 0, None, 0, 0, n, g.H, g.W, g.G, g.P,
-                           None, 0, None, dt, dt, impl, self._S())
-            if sc.live or sc.pooled is not None:
-                L.bn_relu_pool_fwd(_vp(sc.lin), sc.N, n, g.H, g.W, g.G, g.P, _vp(sc.ss) if sc.live else None,
-                                   _vp(sc.act), _vp(sc.pooled), sc.geo_p.P if sc.pooled is not None else 0,
-                                   _vp(sc.feat), plan.Balloc, dt, self._S())
-        if not nd.kids:
-            return
-        if plan.umma_heads and nd.idx in plan.heads:
-            hd = plan.heads[nd.idx]
-            outs = ([(hd.Z16, 16)] if hd.leaf_off is not None else []) + ([(rt.Z1, 16)] if rt is not None else [])
-            outs.append((None, 0))
-            (o0, n0), (o1, n1) = outs[0], outs[1]
-            L.stencil_gemm(_vp(st.feat), st.Fext, None, 0, _vp(hd.Wfc), 1, _vp(hd.bias), _vp(o0), n0, 0, _vp(o1), n1, 0,
-                           n, 0, 0, 0, plan.Balloc, None, 0, None, BF16, 2, 1, self._S())
-        elif rt is not None:
-            L.fc_fwd(_vp(st.feat), st.F, plan.Balloc, n, eng.tptr(rt.fc1.params.w), eng.tptr(rt.fc1.params.b),
-                     _vp(plan.kextra) if self.dyn_k else None, 16, _vp(rt.Z1), dt, self._S())
-        if len(nd.kids) == 1:                       # no switch: the only sink sees every example of this node
-            self._n_parent = n
-            self._node(eng.nodes[nd.kids[0]], n, orig, None, None)
-            return
-        sw = self.sw[nd.idx]
-        ns = len(nd.kids)
-        L.router_tail_fwd_batched(_vp(sw['tab']), 1, n, 16, float(rt.bn1.hypers.d), float(rt.bn1.hypers.ε), 0, self._S())
-        L.route_compact(_vp(rt.R), ns, ns, n, _vp(orig), self.B, None, _vp(sw['pos']), _vp(sw['orig']),
-                        _vp(sw['count']), self._S())
-        sw['host'].copy_(sw['count'], non_blocking=True)
-        torch.cuda.current_stream(eng.dev).synchronize()            # the child batches are launch parameters
-        counts = [int(c) for c in sw['host']]
-        for s, kid in enumerate(nd.kids):
-            self._n_parent = n
-            self._node(eng.nodes[kid], counts[s], sw['orig'][s], sw['pos'][s], sw['count'][s:s + 1])
-
-    # ------------------------------------------------------------------ #
-    def _counted_walk(self, n_dev, out, fork):
-        """The whole tree at capacity B with the live batch sizes on the device: n_dev (int32 [1]) is the chunk's count,
-        every switch writes its sinks' counts, and every kernel takes its batch from one of them.  No host read.
-        out: Ns of the output pointers (leaf_emit).  fork(key) -> a side stream for the subtree of one sink."""
-        eng, plan, L, B = self.eng, self.plan, self.L, self.B
-        hy = eng.net.hypers
-        H0, W0, C0 = hy.x0_shape
-        main = torch.cuda.current_stream(eng.dev)
-        S = ctypes.c_void_p(main.cuda_stream)
-        for i, slot in enumerate(plan.node[0].out):
-            L.pack_input_counted(_vp(plan.x0), B, H0, W0, C0, 2 ** i, _vp(slot.t), min(slot.C, (C0 + 7) // 8 * 8),
-                                 slot.geo.G, slot.geo.P, eng.dtype, _vp(n_dev), S)
-        joins = []
-        for k in eng.nodes[0].kids:
-            self._cnode(eng.nodes[k], n_dev, None, None, None, main, out, fork, joins)
-        for st in joins:                             # every side stream rejoins the origin (required under capture)
-            main.wait_stream(st)
-
-    def _cnode(self, nd, cnt, orig, pos, pcnt, stream, out, fork, joins):
-        """node `nd` on `stream` with its live count at cnt (device int32 [1]); orig / pos: the examples' original ids
-        and rows in the parent's compact batch (None = identity, no switch above); pcnt: the parent's count"""
-        eng, plan, L, B = self.eng, self.plan, self.L, self.B
-        dt = eng.dtype
-        S = ctypes.c_void_p(stream.cuda_stream)
-        if nd.kind == 'reg':
-            par = eng.nodes[nd.parent]
-            r = plan.reg[nd.idx]
-            if not plan.umma_heads:
-                pst = plan.node[par.idx]
-                L.fc_fwd_counted(_vp(pst.feat), pst.F, plan.Balloc, B, eng.tptr(r.fc.params.w), eng.tptr(r.fc.params.b),
-                                 None, self.n_cls, _vp(r.Zbuf), dt, _vp(pcnt if pcnt is not None else cnt), S)
-            no = self.leaf_no[nd.idx]
-            L.leaf_emit(_vp(r.Zbuf), r.ldz, self.n_cls, _vp(pos), _vp(orig), _vp(cnt), B, no, self.path_ops[no],
-                        ctypes.c_void_p(out.prob), ctypes.c_void_p(out.cls), ctypes.c_void_p(out.exit),
-                        ctypes.c_void_p(out.ops), S)
-            return
-        st = plan.node[nd.idx]
-        ins = [s.t for s in st.pin]
-        if pos is not None:
-            for slot, dst in zip(st.pin, self.cin[nd.idx]):
-                g = slot.geo
-                L.gather_images(_vp(slot.t), B, g.P, _vp(pos), _vp(cnt), _vp(dst), B, g.P, slot.C, g.H, g.W, g.G, dt, S)
-            ins = self.cin[nd.idx]
-        rt = plan.rtr.get(nd.idx)
-        if self.dyn_k and rt is not None:
-            if plan.umma_heads:
-                L.gather_feature(_vp(self.kfeat), _vp(orig), _vp(cnt), B, None, _vp(st.feat[st.F // 8, :, 0]), 8, dt, S)
-            else:                                    # a vector per router: sibling subtrees run concurrently
-                L.gather_feature(_vp(self.kfeat), _vp(orig), _vp(cnt), B, _vp(self._kext[nd.idx]), None, 0, 0, S)
+                L.gather_feature(_vp(self.kfeat), _vp(orig), _vp(sink_cnt), n, _vp(self._kext[nd.idx]), None, 0, 0, S)
         for k, sc in enumerate(st.sc):
             g = sc.geo
             prev = st.sc[k - 1] if k > 0 else None
             L.stencil_gemm_counted(_vp(ins[k]), sc.K0, _vp(prev.pooled) if prev is not None else None, sc.K1, _vp(sc.Wf),
-                                   9, eng.tptr(sc.bk), _vp(sc.lin), sc.N, 0, None, 0, 0, B, g.H, g.W, g.G, g.P,
+                                   9, eng.tptr(sc.bk), _vp(sc.lin), sc.N, 0, None, 0, 0, n, g.H, g.W, g.G, g.P,
                                    None, 0, None, dt, dt, eng.impl, _vp(cnt), S)
             if sc.live or sc.pooled is not None:
-                L.bn_relu_pool_fwd_counted(_vp(sc.lin), sc.N, B, g.H, g.W, g.G, g.P, _vp(sc.ss) if sc.live else None,
+                L.bn_relu_pool_fwd_counted(_vp(sc.lin), sc.N, n, g.H, g.W, g.G, g.P, _vp(sc.ss) if sc.live else None,
                                            _vp(sc.act), _vp(sc.pooled), sc.geo_p.P if sc.pooled is not None else 0,
                                            _vp(sc.feat), plan.Balloc, dt, _vp(cnt), S)
         if not nd.kids:
@@ -378,29 +333,22 @@ class CompactEvaluator:
             outs.append((None, 0))
             (o0, n0), (o1, n1) = outs[0], outs[1]
             L.stencil_gemm_counted(_vp(st.feat), st.Fext, None, 0, _vp(hd.Wfc), 1, _vp(hd.bias), _vp(o0), n0, 0,
-                                   _vp(o1), n1, 0, B, 0, 0, 0, plan.Balloc, None, 0, None, BF16, 2, 1, _vp(cnt), S)
+                                   _vp(o1), n1, 0, n, 0, 0, 0, plan.Balloc, None, 0, None, BF16, 2, 1, _vp(cnt), S)
         elif rt is not None:
-            L.fc_fwd_counted(_vp(st.feat), st.F, plan.Balloc, B, eng.tptr(rt.fc1.params.w), eng.tptr(rt.fc1.params.b),
+            L.fc_fwd_counted(_vp(st.feat), st.F, plan.Balloc, n, eng.tptr(rt.fc1.params.w), eng.tptr(rt.fc1.params.b),
                              _vp(self._kext[nd.idx]) if self.dyn_k else None, 16, _vp(rt.Z1), dt, _vp(cnt), S)
-        if len(nd.kids) == 1:
-            self._cnode(eng.nodes[nd.kids[0]], cnt, orig, None, cnt, stream, out, fork, joins)
+        if len(nd.kids) == 1:                       # no switch: the only sink sees every example of this node
+            self._node(eng.nodes[nd.kids[0]], live, live, orig, None, cnt, stream, leaf, split)
             return
         sw = self.sw[nd.idx]
         ns = len(nd.kids)
-        L.router_tail_fwd_batched_counted(_vp(sw['tab']), 1, B, 16, float(rt.bn1.hypers.d), float(rt.bn1.hypers.ε), 0,
+        L.router_tail_fwd_batched_counted(_vp(sw['tab']), 1, n, 16, float(rt.bn1.hypers.d), float(rt.bn1.hypers.ε), 0,
                                           _vp(cnt), S)
-        L.route_compact_counted(_vp(rt.R), ns, ns, B, _vp(orig), B, None, _vp(sw['pos']), _vp(sw['orig']),
+        L.route_compact_counted(_vp(rt.R), ns, ns, n, _vp(orig), self.B, None, _vp(sw['pos']), _vp(sw['orig']),
                                 _vp(sw['count']), _vp(cnt), S)
-        # sink 0 continues on this stream, the others fork: the graph's critical path is one root-to-leaf chain
-        ev = torch.cuda.Event()
-        ev.record(stream)
-        for s, kid in enumerate(nd.kids):
-            st2 = stream
-            if s > 0:
-                st2 = fork((nd.idx, s))
-                st2.wait_event(ev)
-                joins.append(st2)
-            self._cnode(eng.nodes[kid], sw['count'][s:s + 1], sw['orig'][s], sw['pos'][s], cnt, st2, out, fork, joins)
+        for s, sink, sink_stream in split(nd, sw, stream):
+            self._node(eng.nodes[nd.kids[s]], sink, live, sw['orig'][s], sw['pos'][s], sw['count'][s:s + 1],
+                       sink_stream, leaf, split)
 
     # ------------------------------------------------------------------ #
     def result(self):
@@ -421,8 +369,7 @@ class CompactEvaluator:
             acc += float(row[0])
         moc = 0.0
         for nd in eng.nodes:
-            ops = nd.layer.n_ops + (nd.router.n_ops if nd.router is not None else 0)
-            moc += self.visits[nd.idx] * float(ops)
+            moc += self.visits[nd.idx] * float(_node_ops(nd))
         out[(eng.net, 'acc')] = acc
         out[(eng.net, 'moc')] = moc / n
         return out
@@ -448,23 +395,37 @@ class RoutedPredictor:
         self.prob = torch.zeros((B, nc), dtype=torch.float32, device=dev)
         self.exit = torch.zeros(B, dtype=torch.int32, device=dev)
         self.ops = torch.zeros(B, dtype=torch.float64, device=dev)
-        self._out = Ns(prob=self.prob.data_ptr(), cls=self.cls.data_ptr(), exit=self.exit.data_ptr(),
-                       ops=self.ops.data_ptr())
+        self._out = _LeafEmit(ev, self.prob.data_ptr(), self.cls.data_ptr(), self.exit.data_ptr(), self.ops.data_ptr())
         self._side = {}
+        self._joins = []
         self.graph = None
         self.graph_launches = 0
 
-    def _fork(self, key):
-        if key not in self._side:
-            self._side[key] = torch.cuda.Stream(self.ev.eng.dev)
-        return self._side[key]
+    def _split(self, nd, sw, stream):
+        """switch step of the graph: every sink runs at the capacity with its device count.  Sink 0 continues on the
+        switch's stream and the others fork side streams, so the graph's critical path is one root-to-leaf chain."""
+        ev = torch.cuda.Event()
+        ev.record(stream)
+        for s in range(len(nd.kids)):
+            st = stream
+            if s > 0:
+                if (nd.idx, s) not in self._side:
+                    self._side[(nd.idx, s)] = torch.cuda.Stream(self.ev.eng.dev)
+                st = self._side[(nd.idx, s)]
+                st.wait_event(ev)
+                self._joins.append(st)
+            yield s, (self.B, sw['count'][s:s + 1]), st
 
     def _ops(self):
-        self.ev._prepare()
-        self.ev._counted_walk(self.n_dev, self._out, self._fork)
+        ev = self.ev
+        main = torch.cuda.current_stream(ev.eng.dev)
+        ev._prepare()
+        self._joins = []
+        ev._walk((self.B, self.n_dev), self._out, self._split)
+        for st in self._joins:                   # every side stream rejoins the origin (required under capture)
+            main.wait_stream(st)
 
     def _capture(self):
-        import gc
         eng = self.ev.eng
         s = torch.cuda.Stream(eng.dev)
         s.wait_stream(torch.cuda.current_stream(eng.dev))
@@ -474,34 +435,23 @@ class RoutedPredictor:
         torch.cuda.synchronize(eng.dev)
         g = torch.cuda.CUDAGraph()
         before = eng.L.launches
-        # no cyclic garbage collection inside capture (see Engine._capture)
-        gc.collect()
-        gc_was_on = gc.isenabled()
-        gc.disable()
-        try:
+        with _gc_off():
             with torch.cuda.graph(g):
                 self._ops()
-        finally:
-            if gc_was_on:
-                gc.enable()
         self.graph_launches = eng.L.launches - before
         self.graph = g
 
     def __call__(self, x0, k_cpt=None):
         ev = self.ev
-        eng = ev.eng
         n = ev._check_x0(x0)
         if n > self.B:
             raise ValueError('batch %d > predictor capacity %d' % (n, self.B))
         kf = ev._k_feature(k_cpt, n)
         if n > 0:
-            with torch.cuda.device(eng.dev):
+            with torch.cuda.device(ev.eng.dev):
                 if self.graph is None:
                     self._capture()
-                hy = eng.net.hypers
-                ev.plan.x0[:n].copy_(eng._to_dev(x0, (n,) + tuple(hy.x0_shape), 'x0'), non_blocking=True)
-                if kf is not None:
-                    ev.kfeat[:n].copy_(torch.as_tensor(kf), non_blocking=True)
+                ev._load(x0, n, kf)
                 self.n_dev.fill_(n)
                 self.graph.replay()
         return Ns(cls=self.cls[:n], prob=self.prob[:n], exit=self.exit[:n], ops=self.ops[:n])

@@ -10,7 +10,9 @@ reverse preorder, one fused optimiser kernel over the flat parameter buffer.
 Every node is evaluated densely on the whole batch, exactly like the
 reference (SURVEY F2).
 """
+import contextlib
 import ctypes
+import gc
 import os
 from types import SimpleNamespace as Ns
 
@@ -76,6 +78,22 @@ def _ru(a, b):
 def _vp(t):
     """device pointer of a tensor (or None) as c_void_p"""
     return None if t is None else ctypes.c_void_p(t.data_ptr())
+
+
+@contextlib.contextmanager
+def _gc_off():
+    """Around a CUDA graph capture.  The cyclic garbage collector must not run inside capture: freeing a tensor of an
+    engine that was dropped earlier (plans and their launch closures are reference cycles) makes the allocator record
+    an event on a capturing stream, which invalidates the capture.  Collect now, keep the collector off until capture
+    ends."""
+    gc.collect()
+    was_on = gc.isenabled()
+    gc.disable()
+    try:
+        yield
+    finally:
+        if was_on:
+            gc.enable()
 
 
 def _comps(layer):
@@ -800,14 +818,7 @@ class Engine:
             with torch.cuda.stream(s):           # the communicator's first collective (channel setup) stays out of capture
                 self._allreduce()
             torch.cuda.synchronize(self.dev)
-        # The cyclic garbage collector must not run inside capture: freeing a tensor of an engine that was dropped
-        # earlier (plans and their launch closures are reference cycles) makes the allocator record an event on a
-        # capturing stream, which invalidates the capture.  Collect now, keep the collector off until capture ends.
-        import gc
-        gc.collect()
-        gc_was_on = gc.isenabled()
-        gc.disable()
-        try:
+        with _gc_off():
             if one_graph:
                 # the whole step is ONE graph: with our own communicator the NCCL launch is captured like any kernel
                 with torch.cuda.graph(g1):
@@ -821,9 +832,6 @@ class Engine:
                     self._compute_ops(plan)
                 with torch.cuda.graph(g2):
                     self._run(plan.opt_ops)
-        finally:
-            if gc_was_on:
-                gc.enable()
         plan.graph_launches = self.L.launches - before
         self._graphs[id(plan)] = (g1, g2)
         return self._graphs[id(plan)]
