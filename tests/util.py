@@ -130,6 +130,27 @@ def dropout_mask(seed, draw, shape, keep):
     return (u.astype(np.uint64) < np.uint64(int(keep * 4294967296.0))).reshape(shape).astype(np.float32)
 
 
+def _mul32(x, c):
+    """x * c mod 2^32 for int64 tensors holding uint32 values, without int64 overflow"""
+    return (x * (c & 0xFFFF) + (((x * (c >> 16)) & 0xFFFF) << 16)) & 0xFFFFFFFF
+
+
+def _mix32(x):
+    x = x ^ (x >> 16); x = _mul32(x, 0x7feb352d); x = x ^ (x >> 15); x = _mul32(x, 0x846ca68b)
+    return x ^ (x >> 16)
+
+
+def dropout_mask_t(seed, draw, shape, keep, device):
+    """torch restatement of dropout_mask on any device (bool tensor of `shape`, NHWC element order)"""
+    import torch
+    n = 1
+    for s in shape:
+        n *= int(s)
+    i = torch.arange(n, dtype=torch.int64, device=device)
+    u = _mix32(_mix32((_mul32(i, 0x9E3779B9) + seed) & 0xFFFFFFFF) ^ ((draw * 0x85EBCA6B) & 0xFFFFFFFF))
+    return (u < int(keep * 4294967296.0)).view(*shape)
+
+
 def randomize_routers(net, seed=1, scale=0.5):
     """The reference zero-initialises the last router layer (all decisions tie
     to sink 0); give it weights so parity tests see non-trivial routing."""
@@ -203,6 +224,44 @@ def from_planes(t, geo, C):
             + (np.arange(W)[None, None, :] + 1)).reshape(-1)
     out = np.concatenate([t[kg, rows] for kg in range(t.shape[0])], 1)
     return out.reshape(B, H, W, -1)[..., :C]
+
+
+def _planes_view(t, geo):
+    """[KG][P][8] -> view [KG][B][H+1][W+1][8] of the image blocks (row G + n*S + r*Wp + c is [n][r][c]);
+    the valid pixel (h, w) is [h+1][w+1], row 0 and column 0 of a block are its zero pads."""
+    return t[:, geo.G:geo.G + geo.rows].view(t.shape[0], geo.B, geo.H + 1, geo.W + 1, 8)
+
+
+def to_planes_t(x, geo, Cpad=None):
+    """torch version of to_planes on x's device and dtype: NHWC -> [Cpad/8][P][8] with zero pads / guards"""
+    B, H, W, C = x.shape
+    Cpad = C if Cpad is None else Cpad
+    t = x.new_zeros((Cpad // 8, geo.P, 8))
+    v = _planes_view(t, geo)[:, :, 1:, 1:, :]
+    for kg in range(Cpad // 8):          # one plane at a time: no NHWC-sized temporary
+        c = min(8, max(C - kg * 8, 0))
+        if c:
+            v[kg, ..., :c] = x[..., kg * 8:kg * 8 + c]
+    return t
+
+
+def from_planes_t(t, geo, C):
+    """torch version of from_planes: [KG][P][8] -> NHWC (first C channels), a new tensor"""
+    v = _planes_view(t, geo)[:, :, 1:, 1:, :]
+    return v.permute(1, 2, 3, 0, 4).reshape(geo.B, geo.H, geo.W, -1)[..., :C].contiguous()
+
+
+def to_feat_t(x, Balloc):
+    """(B, F) -> the flattened-feature layout [F/8][Balloc][8] of the heads, rows >= B zero"""
+    B, F = x.shape
+    t = x.new_zeros((F // 8, Balloc, 8))
+    t[:, :B] = x.view(B, F // 8, 8).permute(1, 0, 2)
+    return t
+
+
+def from_feat_t(t, B):
+    """[F/8][Balloc][8] -> (B, F)"""
+    return t[:, :B].permute(1, 0, 2).reshape(B, -1)
 
 
 def stencil_offsets(Wp):
