@@ -7,9 +7,11 @@
 #include "../../include/mpnn.h"
 
 #define FC_NMAX 16
+#define FC_NWIDE 64          // widest FC head: the first layer of a 64-wide router, in FC_NMAX-column slices
 
 // ---------------------------------------------------------------- fc forward
-// CNT: only the rows b < min(*count, B) are stored (B: the capacity the grid was sized for)
+// CNT: only the rows b < min(*count, B) are stored (B: the capacity the grid was sized for).  blockIdx.y selects the
+// FC_NMAX-column slice j0 = 16 * blockIdx.y of the n outputs (one slice for n <= 16).
 template <typename T, bool CNT = false>
 __global__ void __launch_bounds__(256)
 fc_fwd_kernel(const T* __restrict__ X, int F, int Balloc, int B, const float* __restrict__ W,
@@ -20,6 +22,7 @@ fc_fwd_kernel(const T* __restrict__ X, int F, int Balloc, int B, const float* __
     const int bl = b < B ? b : B - 1;
     const int Bn = CNT ? min(max(*count, 0), B) : B;
     if (CNT && (int)blockIdx.x * 32 >= Bn) return;
+    const int j0 = blockIdx.y * FC_NMAX, nj = min(FC_NMAX, n - j0);
     float acc[FC_NMAX];
 #pragma unroll
     for (int j = 0; j < FC_NMAX; ++j) acc[j] = 0.f;
@@ -28,10 +31,10 @@ fc_fwd_kernel(const T* __restrict__ X, int F, int Balloc, int B, const float* __
         Row8<T>::load(plane_row(X, fg, Balloc, bl), x);
 #pragma unroll
         for (int c = 0; c < 8; ++c) {
-            const float* wr = W + (size_t)(fg * 8 + c) * n;
+            const float* wr = W + (size_t)(fg * 8 + c) * n + j0;
 #pragma unroll
             for (int j = 0; j < FC_NMAX; ++j)
-                if (j < n) acc[j] = fmaf(x[c], __ldg(wr + j), acc[j]);
+                if (j < nj) acc[j] = fmaf(x[c], __ldg(wr + j), acc[j]);
         }
     }
     __shared__ float red[8][32][FC_NMAX + 1];
@@ -39,21 +42,21 @@ fc_fwd_kernel(const T* __restrict__ X, int F, int Balloc, int B, const float* __
     for (int j = 0; j < FC_NMAX; ++j) red[ky][lane][j] = acc[j];
     __syncthreads();
     // thread (lane, ky) finalises outputs j = ky, ky+8
-    for (int j = ky; j < n; j += 8) {
+    for (int j = ky; j < nj; j += 8) {
         float t = 0.f;
 #pragma unroll
         for (int s = 0; s < 8; ++s) t += red[s][lane][j];
-        if (extra) t = fmaf(extra[bl], __ldg(W + (size_t)F * n + j), t);
-        t += bias ? bias[j] : 0.f;
-        if (b < Bn) Z[(size_t)b * n + j] = t;
+        if (extra) t = fmaf(extra[bl], __ldg(W + (size_t)F * n + j0 + j), t);
+        t += bias ? bias[j0 + j] : 0.f;
+        if (b < Bn) Z[(size_t)b * n + j0 + j] = t;
     }
 }
 
 extern "C" int mpnn_fc_fwd_counted(const void* X, int F, int Balloc, int B, const float* W, const float* bias,
                                    const float* extra, int n, float* Z, int dtype, const int* count, void* stream) {
-    MPNN_REQUIRE(F % 8 == 0 && n >= 1 && n <= FC_NMAX, "fc_fwd: F=%d n=%d (n<=%d)", F, n, FC_NMAX);
+    MPNN_REQUIRE(F % 8 == 0 && n >= 1 && n <= FC_NWIDE, "fc_fwd: F=%d n=%d (n<=%d)", F, n, FC_NWIDE);
     MPNN_REQUIRE(B >= 1 && Balloc >= B, "fc_fwd: B=%d Balloc=%d", B, Balloc);
-    dim3 block(32, 8), grid(ceil_div(B, 32));
+    dim3 block(32, 8), grid(ceil_div(B, 32), ceil_div(n, FC_NMAX));
     if (count) {
         MPNN_DISPATCH_DTYPE(dtype, (fc_fwd_kernel<T, true><<<grid, block, 0, (cudaStream_t)stream>>>(
             (const T*)X, F, Balloc, B, W, bias, extra, n, Z, count)));
@@ -70,7 +73,8 @@ extern "C" int mpnn_fc_fwd(const void* X, int F, int Balloc, int B, const float*
 }
 
 // ---------------------------------------------------------- fc backward data
-template <typename T>
+// N1MAX: register row of the second operand (FC_NMAX, or FC_NWIDE for the first layer of a wide router)
+template <typename T, int N1MAX = FC_NMAX>
 __global__ void __launch_bounds__(256)
 fc_bwd_data_kernel(const float* __restrict__ dZ0, const float* __restrict__ W0, int n0,
                    const float* __restrict__ dZ1, const float* __restrict__ W1, int n1,
@@ -78,12 +82,11 @@ fc_bwd_data_kernel(const float* __restrict__ dZ0, const float* __restrict__ W0, 
     const int lane = threadIdx.x, ky = threadIdx.y;
     const int b = blockIdx.x * 32 + lane;
     if (b >= B) return;
-    float d0[FC_NMAX], d1[FC_NMAX];
+    float d0[FC_NMAX], d1[N1MAX];
 #pragma unroll
-    for (int j = 0; j < FC_NMAX; ++j) {
-        d0[j] = j < n0 ? dZ0[(size_t)b * n0 + j] : 0.f;
-        d1[j] = (dZ1 && j < n1) ? dZ1[(size_t)b * n1 + j] : 0.f;
-    }
+    for (int j = 0; j < FC_NMAX; ++j) d0[j] = j < n0 ? dZ0[(size_t)b * n0 + j] : 0.f;
+#pragma unroll
+    for (int j = 0; j < N1MAX; ++j) d1[j] = (dZ1 && j < n1) ? dZ1[(size_t)b * n1 + j] : 0.f;
     for (int fg = blockIdx.y * 8 + ky; fg < F / 8; fg += 8 * gridDim.y) {
         float v[8];
 #pragma unroll
@@ -95,7 +98,7 @@ fc_bwd_data_kernel(const float* __restrict__ dZ0, const float* __restrict__ W0, 
                 if (j < n0) t = fmaf(d0[j], __ldg(W0 + (size_t)f * n0 + j), t);
             if (dZ1) {
 #pragma unroll
-                for (int j = 0; j < FC_NMAX; ++j)
+                for (int j = 0; j < N1MAX; ++j)
                     if (j < n1) t = fmaf(d1[j], __ldg(W1 + (size_t)f * n1 + j), t);
             }
             v[c] = t;
@@ -107,12 +110,22 @@ fc_bwd_data_kernel(const float* __restrict__ dZ0, const float* __restrict__ W0, 
 extern "C" int mpnn_fc_bwd_data(const float* dZ0, const float* W0, int n0,
                                 const float* dZ1, const float* W1, int n1,
                                 int F, int Balloc, int B, void* dX, int dtype, void* stream) {
-    MPNN_REQUIRE(F % 8 == 0 && n0 >= 1 && n0 <= FC_NMAX && n1 <= FC_NMAX, "fc_bwd_data: n0=%d n1=%d", n0, n1);
+    MPNN_REQUIRE(F % 8 == 0 && n0 >= 1 && n0 <= FC_NWIDE && n1 <= FC_NWIDE && (n0 <= FC_NMAX || n1 == 0),
+                 "fc_bwd_data: n0=%d n1=%d (n0 <= %d beside a second operand, each <= %d)", n0, n1, FC_NMAX, FC_NWIDE);
+    if (n0 > FC_NMAX) {          // a wide operand alone takes the wide slot (same summation order)
+        dZ1 = dZ0; W1 = W0; n1 = n0;
+        dZ0 = nullptr; W0 = nullptr; n0 = 0;
+    }
     int gy = ceil_div(F / 8, 8 * 4);
     if (gy < 1) gy = 1;
     dim3 block(32, 8), grid(ceil_div(B, 32), gy);
-    MPNN_DISPATCH_DTYPE(dtype, (fc_bwd_data_kernel<T><<<grid, block, 0, (cudaStream_t)stream>>>(
-        dZ0, W0, n0, dZ1, W1, n1, F, Balloc, B, (T*)dX)));
+    if (n1 <= FC_NMAX) {
+        MPNN_DISPATCH_DTYPE(dtype, (fc_bwd_data_kernel<T><<<grid, block, 0, (cudaStream_t)stream>>>(
+            dZ0, W0, n0, dZ1, W1, n1, F, Balloc, B, (T*)dX)));
+    } else {
+        MPNN_DISPATCH_DTYPE(dtype, (fc_bwd_data_kernel<T, FC_NWIDE><<<grid, block, 0, (cudaStream_t)stream>>>(
+            dZ0, W0, n0, dZ1, W1, n1, F, Balloc, B, (T*)dX)));
+    }
     return mpnn_check_launch("fc_bwd_data");
 }
 
@@ -149,7 +162,7 @@ __global__ void fc_bwd_weight_kernel(const T* __restrict__ X, int F, int Balloc,
 
 extern "C" int mpnn_fc_bwd_weight(const void* X, int F, int Balloc, int B, const float* extra,
                                   const float* dZ, int n, float* dW, float* db, int dtype, void* stream) {
-    MPNN_REQUIRE(F % 8 == 0 && n >= 1 && n <= FC_NMAX, "fc_bwd_weight: F=%d n=%d", F, n);
+    MPNN_REQUIRE(F % 8 == 0 && n >= 1 && n <= FC_NWIDE, "fc_bwd_weight: F=%d n=%d (n<=%d)", F, n, FC_NWIDE);
     int bchunk = 512;
     dim3 block(n, 8), grid(F / 8 + 1, ceil_div(B, bchunk));
     MPNN_DISPATCH_DTYPE(dtype, (fc_bwd_weight_kernel<T><<<grid, block, 0, (cudaStream_t)stream>>>(
@@ -490,7 +503,7 @@ extern "C" int mpnn_router_tail_fwd(const float* Z1, int B, int C,
                                     const float* W3, const float* bias3, int ns,
                                     float d, float eps, int train,
                                     float* Z2, float* R, float* save, void* stream) {
-    MPNN_REQUIRE(C == RT_C, "router_tail_fwd: C=%d (only %d supported)", C, RT_C);
+    MPNN_REQUIRE(C == RT_C, "router_tail_fwd: C=%d (only %d; wider routers run in mpnn_router_tail_fwd_batched)", C, RT_C);
     MPNN_REQUIRE(ns >= 2 && ns <= RT_NSMAX, "router_tail_fwd: ns=%d", ns);
     router_tail_fwd_kernel<<<1, RT_THREADS, 0, (cudaStream_t)stream>>>(
         Z1, B, g1, b1, m1, v1, W2, bias2, g2, b2, m2, v2, W3, bias3, ns, d, eps, train, Z2, R, save);
@@ -691,7 +704,7 @@ extern "C" int mpnn_router_tail_bwd(const float* Z1, const float* Z2, const floa
                                     float* dg1, float* dbt1, float* dW2, float* dbias2,
                                     float* dg2, float* dbt2, float* dW3, float* dbias3,
                                     float* dZ1, float* scratch, void* stream) {
-    MPNN_REQUIRE(C == RT_C, "router_tail_bwd: C=%d", C);
+    MPNN_REQUIRE(C == RT_C, "router_tail_bwd: C=%d (only %d; wider routers run in mpnn_router_tail_bwd_batched)", C, RT_C);
     MPNN_REQUIRE(ns >= 2 && ns <= RT_NSMAX, "router_tail_bwd: ns=%d", ns);
     router_tail_bwd_kernel<<<1, RT_THREADS, 0, (cudaStream_t)stream>>>(
         Z1, Z2, dR, B, ns, g1, b1, W2, g2, b2, W3, save, dg1, dbt1, dW2, dbias2, dg2, dbt2, dW3, dbias3,

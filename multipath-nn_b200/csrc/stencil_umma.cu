@@ -619,20 +619,24 @@ int mpnn_stencil_gemm_umma(const void* A0, int K0, const void* A1, int K1, const
     const size_t kMax = 227 * 1024 - 1024;
     const size_t red_bytes = bwd ? (size_t)12 * N0 : 0;        // staged scale / shift / mean of the BN behind out0
     int split = 0, nstage = 0, NB = 0;
-    for (int s = 1; s <= 8; s *= 2) {
-        if (N % (16 * s)) break;
+    auto try_split = [&](int s) {            // N in s slices of NB columns, if the resident weights fit
         NB = N / s;
-        if (NB > 256) continue;
+        if (NB > 256) return false;
         size_t w = ((size_t)ntaps * KG * NB * 16 + 127) & ~(size_t)127;
         size_t fixed = w + 256 + (size_t)9 * NB * 4 + red_bytes;
-        if (fixed + 2 * stage <= kMax) {
-            split = s;
-            nstage = (int)((kMax - fixed) / stage);
-            if (nstage > 4) nstage = 4;
-            if (tune_nstage && nstage > tune_nstage) nstage = tune_nstage;
-            break;
-        }
-    }
+        if (fixed + 2 * stage > kMax) return false;
+        split = s;
+        nstage = (int)((kMax - fixed) / stage);
+        if (nstage > 4) nstage = 4;
+        if (tune_nstage && nstage > tune_nstage) nstage = tune_nstage;
+        return true;
+    };
+    for (int s = 1; s <= 8; s *= 2)
+        if (N % (16 * s) || try_split(s)) break;
+    // N = 48 or 80 (a head GEMM [W_leaf | W_r1] with a 32- or 64-wide router) has no power-of-two split into 16-wide
+    // slices: when the whole N does not fit, fall back to the smallest other divisor (3 or 5 slices of 16 at F = 2048)
+    for (int s = 3; split == 0 && s <= 16; ++s)
+        if (N % (16 * s) == 0) try_split(s);
     MPNN_REQUIRE(split > 0, "stencil_gemm(tcgen05): K=%d N=%d does not fit shared memory", K0 + K1, N);
     // fully-connected data gradients at small batches (one or two row tiles, N = 256 .. 2048 outputs): the slice
     // width above leaves a handful of CTAs, each walking up to 16 accumulator chunks through the generic epilogue

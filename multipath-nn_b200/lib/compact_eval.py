@@ -329,21 +329,23 @@ class CompactEvaluator:
             return
         if plan.umma_heads and nd.idx in plan.heads:
             hd = plan.heads[nd.idx]
-            outs = ([(hd.Z16, 16)] if hd.leaf_off is not None else []) + ([(rt.Z1, 16)] if rt is not None else [])
+            outs = ([(hd.Z16, 16)] if hd.leaf_off is not None else []) + \
+                ([(rt.Z1, eng.router_width)] if rt is not None else [])
             outs.append((None, 0))
             (o0, n0), (o1, n1) = outs[0], outs[1]
             L.stencil_gemm_counted(_vp(st.feat), st.Fext, None, 0, _vp(hd.Wfc), 1, _vp(hd.bias), _vp(o0), n0, 0,
                                    _vp(o1), n1, 0, n, 0, 0, 0, plan.Balloc, None, 0, None, BF16, 2, 1, _vp(cnt), S)
         elif rt is not None:
             L.fc_fwd_counted(_vp(st.feat), st.F, plan.Balloc, n, eng.tptr(rt.fc1.params.w), eng.tptr(rt.fc1.params.b),
-                             _vp(self._kext[nd.idx]) if self.dyn_k else None, 16, _vp(rt.Z1), dt, _vp(cnt), S)
+                             _vp(self._kext[nd.idx]) if self.dyn_k else None, eng.router_width, _vp(rt.Z1), dt,
+                             _vp(cnt), S)
         if len(nd.kids) == 1:                       # no switch: the only sink sees every example of this node
             self._node(eng.nodes[nd.kids[0]], live, live, orig, None, cnt, stream, leaf, split)
             return
         sw = self.sw[nd.idx]
         ns = len(nd.kids)
-        L.router_tail_fwd_batched_counted(_vp(sw['tab']), 1, n, 16, float(rt.bn1.hypers.d), float(rt.bn1.hypers.ε), 0,
-                                          _vp(cnt), S)
+        L.router_tail_fwd_batched_counted(_vp(sw['tab']), 1, n, eng.router_width, float(rt.bn1.hypers.d),
+                                          float(rt.bn1.hypers.ε), 0, _vp(cnt), S)
         L.route_compact_counted(_vp(rt.R), ns, ns, n, _vp(orig), self.B, None, _vp(sw['pos']), _vp(sw['orig']),
                                 _vp(sw['count']), _vp(cnt), S)
         for s, sink, sink_stream in split(nd, sw, stream):

@@ -55,6 +55,29 @@ _P2P = np.dtype([('base', '<u8', (_P2P_MAX,)), ('world', '<i4'), ('rank', '<i4')
 assert _P2P.itemsize == 168
 
 
+ROUTER_WIDTHS = (16, 32, 64)
+
+
+def _router_width(nodes):
+    """Hidden width W of the net's routers, Chain([Select(-1), LinTrans(W), BatchNorm, Rect, LinTrans(W), BatchNorm,
+    Rect, LinTrans(n_sinks)]) (arch_and_hypers.router_n_chan).  Both hidden layers and every router of a net have the
+    same W, because the tails of all routers run as one launch of one width; 16 when the net has no router."""
+    widths = {}
+    for nd in nodes:
+        if nd.router is None:
+            continue
+        c = nd.router.comps
+        w = (c[1].hypers.n_chan, c[4].hypers.n_chan)
+        if w[0] != w[1] or w[0] not in ROUTER_WIDTHS:
+            raise NotImplementedError('engine: router %r has hidden widths %d and %d; both must be one of %s'
+                                      % (nd.layer.name, w[0], w[1], ROUTER_WIDTHS))
+        widths[w[0]] = nd.layer.name
+    if len(widths) > 1:
+        raise NotImplementedError('engine: routers of different widths in one net (%s); all must share one of %s'
+                                  % (', '.join('%s: %d' % (n, w) for w, n in sorted(widths.items())), ROUTER_WIDTHS))
+    return next(iter(widths), 16)
+
+
 class _DevMem:
     """device memory that is not torch's (the cudaMalloc'ed exchange buffer of the fused data-parallel tail) as
     a zero-copy torch tensor, through __cuda_array_interface__"""
@@ -381,6 +404,7 @@ class Engine:
         self.regs = [nd for nd in self.nodes if nd.kind == 'reg']
         if not self.dynamic and self.switches:
             raise NotImplementedError('engine: SRNet with switches')
+        self.router_width = _router_width(self.nodes)
 
     # ------------------------------------------------------------------ #
     # parameters: flat trainable buffer + flat state buffer (BN EMAs)
@@ -1047,6 +1071,8 @@ class _Plan:
             nd.router is not None or any(eng.nodes[k].kind == 'reg' for k in nd.kids))]
         # the head GEMM keeps [W_leaf | W_r1] resident in shared memory: F/8 x 32 x 16 bytes must fit (F = 2048 at the
         # reference architecture; a Conv chain at full resolution has F = H*W*C and takes the CUDA-core heads)
+        # a wider head (N = 16 + W = 48 or 80) is split over blockIdx.y into slices of 16 columns (stencil_umma.cu), so
+        # the same bound holds for every router width
         fits = all((head_features(nd) + 16) // 8 * 32 * 16 <= 150 * 1024 for nd in with_heads)
         self.umma_heads = eng.impl == 1 and all(nd.fc.hypers.n_chan <= 16 for nd in eng.regs) and not eng.split and fits
         Balloc = _ru(B, 128) if self.umma_heads else _ru(B, 8)
@@ -1154,7 +1180,7 @@ class _Plan:
             tab = self._desc_table(_RT_FWD, self.rt_fwd)
             self.keep.append(tab)
             tails = lambda: L.router_tail_fwd_batched(
-                _vp(tab), len(self.rt_fwd), B, 16, float(bn0.hypers.d), float(bn0.hypers.ε),
+                _vp(tab), len(self.rt_fwd), B, eng.router_width, float(bn0.hypers.d), float(bn0.hypers.ε),
                 1 if self.bn_train else 0, S())
             # the tails need the head GEMMs that write a router's first layer -- not the classifiers' losses, and not the
             # head of a stage without a router (the last stage: its GEMM and loss then run beside the tails and the
@@ -1189,7 +1215,7 @@ class _Plan:
                 rows = [self._router_bwd_desc(nd) for nd in eng.switches]
                 tabb = self._desc_table(_RT_BWD, rows)
                 self.keep.append(tabb)
-                self.bwd_ops.append(lambda: L.router_tail_bwd_batched(_vp(tabb), len(rows), B, 16, S()))
+                self.bwd_ops.append(lambda: L.router_tail_bwd_batched(_vp(tabb), len(rows), B, eng.router_width, S()))
         main_ops = [op for op in self.bwd_ops if getattr(op, 'lane', 0) == 0]
         self.bwd_head_dep = main_ops[-1] if main_ops else None             # routing gradients are complete
         # data parallel: the gradients of the DEEP stages are complete long before the backward pass ends (it
@@ -1318,8 +1344,9 @@ class _Plan:
         if len(leaves) > 1:
             raise NotImplementedError('engine: more than one LogReg under one node')
         rt = self.rtr.get(nd.idx)
+        W = eng.router_width
         hd = Ns(leaf_off=0 if leaves else None, r_off=(16 if leaves else 0) if rt is not None else None)
-        hd.N = 16 * (bool(leaves) + (rt is not None))
+        hd.N = 16 * bool(leaves) + (W if rt is not None else 0)
         # heads only feed the losses / the routers: off the conv lanes, and spread over a few lanes of their own so
         # that a head never queues behind the head of another stage
         hd.lane = 1 if eng.head_lanes == 1 else 21 + len(self.heads) % eng.head_lanes
@@ -1335,11 +1362,11 @@ class _Plan:
             self._pack(fc.params.b, hd.bias, 1, fc.hypers.n_chan, 2, 0, 8, hd.leaf_off, hd.N, ntaps=1)
         if rt is not None:
             rows = F + (1 if dyn_k else 0)
-            self._pack(rt.fc1.params.w, hd.Wfc, rows, 16, 0, 0, Fext, hd.r_off, hd.N, ntaps=1)
-            self._pack(rt.fc1.params.b, hd.bias, 1, 16, 2, 0, 8, hd.r_off, hd.N, ntaps=1)
+            self._pack(rt.fc1.params.w, hd.Wfc, rows, W, 0, 0, Fext, hd.r_off, hd.N, ntaps=1)
+            self._pack(rt.fc1.params.b, hd.bias, 1, W, 2, 0, 8, hd.r_off, hd.N, ntaps=1)
         outs = [(hd.Z16, 16)] if leaves else []
         if rt is not None:
-            outs.append((rt.Z1, 16))
+            outs.append((rt.Z1, W))
         outs.append((None, 0))
         (o0, n0), (o1, n1) = outs[0], outs[1]
         self.heads[nd.idx] = hd
@@ -1375,12 +1402,13 @@ class _Plan:
         leaf = getattr(hd, 'fc_leaf', None)
         # weight gradients of both heads in one launch
         a = (eng.gptr(leaf.params.w), F, leaf.hypers.n_chan) if leaf is not None else (None, 0, 0)
-        b = (eng.gptr(rt.fc1.params.w), F + (1 if dyn_k else 0), 16) if rt is not None else (None, 0, 0)
+        b = (eng.gptr(rt.fc1.params.w), F + (1 if dyn_k else 0), eng.router_width) if rt is not None else (None, 0, 0)
         if leaf is None:
             a, b = b, (None, 0, 0)
+        nsplit = 16 if leaf is not None else hd.N           # columns of dZ that belong to the first head
 
         def wgrad():
-            L.fc_wgrad(_vp(st.feat), Fext, Balloc, B, _vp(hd.dZ), hd.N, 16, a[0], a[1], a[2], b[0], b[1], b[2], S())
+            L.fc_wgrad(_vp(st.feat), Fext, Balloc, B, _vp(hd.dZ), hd.N, nsplit, a[0], a[1], a[2], b[0], b[1], b[2], S())
         self._tag(wgrad, 'fc_wgrad', desc='F%d N%d' % (Fext, hd.N), flops=2.0 * B * F * hd.N, nbytes=B * F * 2)
         wgrad.lane = 9                               # off the heads lane: the data gradient below is what the chain waits for
         wgrad.early = rt is None
@@ -1391,7 +1419,7 @@ class _Plan:
         if leaf is not None:
             self._pack(leaf.params.w, hd.Wfd, F, leaf.hypers.n_chan, 1, hd.leaf_off, hd.N, 0, F, ntaps=1)
         if rt is not None:
-            self._pack(rt.fc1.params.w, hd.Wfd, F, 16, 1, hd.r_off, hd.N, 0, F, ntaps=1)
+            self._pack(rt.fc1.params.w, hd.Wfd, F, eng.router_width, 1, hd.r_off, hd.N, 0, F, ntaps=1)
         st.dfeat = self.zeros((F // 8, Balloc, 8), eng.tdtype)
 
         def dgrad():
@@ -1744,7 +1772,7 @@ class _Plan:
                 pairs.append((r.dZ, r.fc.params.w, r.dZ.shape[1]))
             if nd.router is not None:
                 rt = self.rtr[nd.idx]
-                pairs.append((rt.dZ1, rt.fc1.params.w, 16))
+                pairs.append((rt.dZ1, rt.fc1.params.w, eng.router_width))
             p0 = pairs[0]
             p1 = pairs[1] if len(pairs) > 1 else (None, None, 0)
             fbd = lambda p0=p0, p1=p1: L.fc_bwd_data(
@@ -1983,18 +2011,19 @@ class _Plan:
         if c[0].hypers.i != -1:
             raise NotImplementedError('engine: router must select the coarsest scale')
         ns = len(nd.kids)
-        if fc1.hypers.n_chan != 16 or fc2.hypers.n_chan != 16 or fc3.hypers.n_chan != ns:
-            raise NotImplementedError('engine: router widths')
+        if fc3.hypers.n_chan != ns:
+            raise NotImplementedError('engine: router output width %d for %d sinks' % (fc3.hypers.n_chan, ns))
+        W = eng.router_width                    # hidden width, checked for the whole net by _router_width
         bwd = self.need_bwd
         rt = Ns(fc1=fc1, bn1=bn1, fc2=fc2, bn2=bn2, fc3=fc3, ns=ns,
-                Z1=self.f32(B, 16), Z2=self.f32(B, 16), R=self.f32(B, ns), save=self.f32(64),
-                dR=self.f32(B, ns) if bwd else None, dZ1=self.f32(B, 16) if bwd else None,
-                scratch=self.f32(2 * B * 16) if bwd else None)
+                Z1=self.f32(B, W), Z2=self.f32(B, W), R=self.f32(B, ns), save=self.f32(4 * W),
+                dR=self.f32(B, ns) if bwd else None, dZ1=self.f32(B, W) if bwd else None,
+                scratch=self.f32(2 * B * W) if bwd else None)
         self.rtr[nd.idx] = rt
         if emit_fc:
             fcr = lambda: L.fc_fwd(
                 _vp(st.feat), st.F, Balloc, B, eng.tptr(fc1.params.w), eng.tptr(fc1.params.b),
-                _vp(self.kextra) if dyn_k else None, 16, _vp(rt.Z1), dt, S())
+                _vp(self.kextra) if dyn_k else None, W, _vp(rt.Z1), dt, S())
             self.fwd_ops.append(self._after(fcr, getattr(st, 'feat_op', None)))
         P = lambda lay, k: eng.tptr(getattr(lay.params, k))
         # the tails of all routers run as ONE launch after the conv pipeline (see _build)
@@ -2012,7 +2041,7 @@ class _Plan:
         Gp = lambda lay, k: eng.gptr(getattr(lay.params, k))
         # (the tail itself ran in the batched launch right after route_bwd)
         self.bwd_ops.append(lambda: L.fc_bwd_weight(
-            _vp(st.feat), st.F, Balloc, B, _vp(self.kextra) if dyn_k else None, _vp(rt.dZ1), 16,
+            _vp(st.feat), st.F, Balloc, B, _vp(self.kextra) if dyn_k else None, _vp(rt.dZ1), eng.router_width,
             Gp(rt.fc1, 'w'), Gp(rt.fc1, 'b'), dt, S()))
 
     # -- routing ----------------------------------------------------------- #
