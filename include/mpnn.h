@@ -518,6 +518,13 @@ int mpnn_router_tail_fwd_batched_counted(const mpnn_router_fwd_desc* descs, int 
                                          float d, float eps, int train, const int* count, void* stream);
 int mpnn_route_compact_counted(const float* R, int ldr, int ns, int n, const int* parent_orig, int cap,
                                int* dec, int* pos, int* orig, int* count, const int* n_count, void* stream);
+/* mpnn_split_planes3 on the live images of a padded-planes tensor of geometry (B, H, W, G, P) and C channels: rows
+ * [0, G + m*(H+1)*(W+1)) of each of the C/8 planes, m = min(*count, B), with the same bits as the whole-tensor call;
+ * the rest of dst is not written, and m = 0 writes nothing.  Rows past the live images may keep a larger earlier
+ * batch's values: the row after the last live image is a pad row, zero in src and dst, so no 3x3 conv of a live
+ * image reads them.  Unlike the entry points above it takes the geometry (the uncounted call takes only P). */
+int mpnn_split_planes3_counted(const float* src, int C, int B, int H, int W, int G, int P, void* dst,
+                               const int* count, void* stream);
 
 /* ---- tcgen05 bring-up probe (tests only) -------------------------------- */
 /* D[128][N] = A[128][K] * B[N][K]^T through one CTA of tcgen05.mma; all

@@ -235,22 +235,41 @@ split_planes_kernel(const float* __restrict__ src, long long rows, __nv_bfloat16
 
 // three-way split (hi | mid | lo), x = hi + mid + lo up to 2^-25 |x|: operand format of the "bf16x6" mode, where a
 // product is a_hi*b_hi + a_mid*b_hi + a_lo*b_hi + a_hi*b_mid + a_mid*b_mid + a_hi*b_lo (every term above 2^-24).
+// Row r of the C/8 * P source rows; `rows` = C/8 * P is the distance between the three parts of dst.  Shared by the
+// whole-tensor and the counted launch, so both write the same bits.
+__device__ __forceinline__ void split3_row(const float* __restrict__ src, long long rows, long long r,
+                                           __nv_bfloat16* __restrict__ dst) {
+    float v[8], hi[8], mid[8], lo[8];
+    Row8<float>::load(src + r * 8, v);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+        hi[j] = __bfloat162float(__float2bfloat16_rn(v[j]));
+        const float r1 = v[j] - hi[j];
+        mid[j] = __bfloat162float(__float2bfloat16_rn(r1));
+        lo[j] = r1 - mid[j];
+    }
+    Row8<__nv_bfloat16>::store(dst + r * 8, hi);
+    Row8<__nv_bfloat16>::store(dst + (rows + r) * 8, mid);
+    Row8<__nv_bfloat16>::store(dst + (2 * rows + r) * 8, lo);
+}
+
 __global__ void __launch_bounds__(256)
 split_planes3_kernel(const float* __restrict__ src, long long rows, __nv_bfloat16* __restrict__ dst) {
-    for (long long r = blockIdx.x * (long long)blockDim.x + threadIdx.x; r < rows; r += (long long)gridDim.x * blockDim.x) {
-        float v[8], hi[8], mid[8], lo[8];
-        Row8<float>::load(src + r * 8, v);
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            hi[j] = __bfloat162float(__float2bfloat16_rn(v[j]));
-            const float r1 = v[j] - hi[j];
-            mid[j] = __bfloat162float(__float2bfloat16_rn(r1));
-            lo[j] = r1 - mid[j];
-        }
-        Row8<__nv_bfloat16>::store(dst + r * 8, hi);
-        Row8<__nv_bfloat16>::store(dst + (rows + r) * 8, mid);
-        Row8<__nv_bfloat16>::store(dst + (2 * rows + r) * 8, lo);
-    }
+    for (long long r = blockIdx.x * (long long)blockDim.x + threadIdx.x; r < rows; r += (long long)gridDim.x * blockDim.x)
+        split3_row(src, rows, r, dst);
+}
+
+// counted: rows [0, G + m*S) of every plane (blockIdx.y), m = min(*count, g.B); m = 0 writes nothing
+__global__ void __launch_bounds__(256)
+split_planes3_counted_kernel(const float* __restrict__ src, Geom g, __nv_bfloat16* __restrict__ dst,
+                             const int* __restrict__ count) {
+    const int m = count ? min(max(*count, 0), g.B) : g.B;
+    if (m == 0) return;
+    const long long live = (long long)g.G + (long long)m * g.S;
+    const long long rows = (long long)gridDim.y * g.P;
+    const long long base = (long long)blockIdx.y * g.P;
+    for (long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x; p < live; p += (long long)gridDim.x * blockDim.x)
+        split3_row(src, rows, base + p, dst);
 }
 
 extern "C" int mpnn_split_planes3(const float* src, int C, int P, void* dst, void* stream) {
@@ -260,6 +279,23 @@ extern "C" int mpnn_split_planes3(const float* src, int C, int P, void* dst, voi
     if (g > 148 * 16) g = 148 * 16;
     split_planes3_kernel<<<(int)g, 256, 0, (cudaStream_t)stream>>>(src, rows, (__nv_bfloat16*)dst);
     return mpnn_check_launch("split_planes3");
+}
+
+extern "C" int mpnn_split_planes3_counted(const float* src, int C, int B, int H, int W, int G, int P, void* dst,
+                                          const int* count, void* stream) {
+    MPNN_REQUIRE(src && dst && C % 8 == 0 && C > 0 && B >= 0 && H > 0 && W > 0,
+                 "split_planes3_counted: C=%d B=%d H=%d W=%d", C, B, H, W);
+    MPNN_REQUIRE(C / 8 <= 65535, "split_planes3_counted: C=%d", C);
+    Geom g = make_geom(B, H, W, G, P);
+    MPNN_REQUIRE(G + g.rows <= P, "split_planes3_counted: P=%d < G + B*(H+1)*(W+1)", P);
+    if (B == 0) return MPNN_OK;
+    const int planes = C / 8;
+    long long gx = ((long long)G + g.rows + 255) / 256;              // sized for the capacity
+    const long long cap = (148 * 16 + planes - 1) / planes;
+    if (gx > cap) gx = cap;
+    split_planes3_counted_kernel<<<dim3((unsigned)gx, planes), 256, 0, (cudaStream_t)stream>>>(
+        src, g, (__nv_bfloat16*)dst, count);
+    return mpnn_check_launch("split_planes3_counted");
 }
 
 extern "C" int mpnn_split_planes(const float* src, int C, int P, void* dst, void* stream) {

@@ -21,6 +21,12 @@ example's softmax, predicted class, exit leaf and path cost (mpnn_leaf_emit) ins
 Nets with a per-example k_cpt carry the router feature alpha_cpt * k_cpt through the compaction by original
 example id (mpnn_gather_feature), so one batch may mix cost budgets.
 
+In bf16x6 precision the convs read only the (hi | mid | lo) bf16 splits of their fp32 inputs: the root splits every
+pyramid scale after packing it, the gathers below a switch move the parent's split planes, and every scale launches the
+dense eval plan's list of passes (`sc.passes`, Plan._build_conv_fwd_split) into fp32 planes, then BN / ReLU / pool in
+fp32 and the counted splits (mpnn_split_planes3_counted) of what the next convs read.  The heads are the CUDA-core
+fp32 ones, as in the dense plan.
+
 One walker serves both ways of running the tree.  Every kernel takes its live batch as a pair (launch batch,
 device count) through the counted entry points, and only the step at a switch differs:
   * host-synced (`run_batch`, `predict`): a node runs at its batch n with no count (the uncounted launch).  A switch
@@ -37,7 +43,7 @@ from types import SimpleNamespace as Ns
 import numpy as np
 import torch
 
-from lib.engine import BF16, _RT_FWD, _gc_off, _vp
+from lib.engine import BF16, F32, _RT_FWD, _gc_off, _vp
 
 __all__ = ['CompactEvaluator', 'RoutedPredictor']
 
@@ -81,8 +87,8 @@ class _LeafEmit:
 
 class CompactEvaluator:
     def __init__(self, eng, batch=4096):
-        if eng.split:
-            raise NotImplementedError('compacted evaluation runs in fp32 or bf16 precision (not the split modes bf16x3 / bf16x6)')
+        if eng.split == 2:
+            raise NotImplementedError('compacted evaluation runs in fp32, bf16 or bf16x6 precision (not bf16x3)')
         if any(getattr(nd, 'maxpool', False) or getattr(nd, 'gmp', False) for nd in eng.nodes):
             raise NotImplementedError('compacted evaluation does not cover MaxPool / GlobalMaxPool blocks')
         if any(nd.loss != 'ce' for nd in eng.regs):
@@ -129,12 +135,14 @@ class CompactEvaluator:
                 host = torch.zeros(ns, dtype=torch.int32)
                 self.sw[nd.idx] = dict(tab=tab, pos=zi(ns, B), orig=zi(ns, B), count=zi(ns),
                                        host=host if eng.dry else host.pin_memory())
-        # compacted inputs of every conv stage below a switch: one planes tensor per scale it consumes
+        # compacted inputs of every conv stage below a switch: one planes tensor per scale it consumes (bf16x6: the
+        # (hi | mid | lo) split planes, the only form of the input its convs read)
         self.cin = {}
         for nd in eng.nodes:
             if nd.kind == 'rcm' and len(eng.nodes[nd.parent].kids) > 1:
                 st = plan.node[nd.idx]
-                self.cin[nd.idx] = [plan.planes(s.C, s.geo) for s in st.pin]
+                self.cin[nd.idx] = [plan.zeros((3 * s.C // 8, s.geo.P, 8), torch.bfloat16) if eng.split
+                                    else plan.planes(s.C, s.geo) for s in st.pin]
         # each router of the CUDA-core heads gets its own k_cpt feature vector: in the graph, sibling subtrees run
         # concurrently
         self._kext = {i: torch.zeros(B, dtype=torch.float32, device=dev) for i in plan.rtr} \
@@ -207,8 +215,12 @@ class CompactEvaluator:
         stream = torch.cuda.current_stream(eng.dev)
         S = ctypes.c_void_p(stream.cuda_stream)
         for i, slot in enumerate(plan.node[0].out):
+            g = slot.geo
             self.L.pack_input_counted(_vp(plan.x0), live[0], H0, W0, C0, 2 ** i, _vp(slot.t),
-                                      min(slot.C, (C0 + 7) // 8 * 8), slot.geo.G, slot.geo.P, eng.dtype, _vp(live[1]), S)
+                                      min(slot.C, (C0 + 7) // 8 * 8), g.G, g.P, eng.dtype, _vp(live[1]), S)
+            if eng.split:
+                self.L.split_planes3_counted(_vp(slot.t), slot.C, live[0], g.H, g.W, g.G, g.P, _vp(slot.split),
+                                             _vp(live[1]), S)
         root = eng.nodes[0]
         leaf.visit(root, live[0])
         if live[0] == 0:                            # run_batch of no examples
@@ -301,12 +313,13 @@ class CompactEvaluator:
             leaf(nd, n, orig, pos, sink_cnt, S)
             return
         st = plan.node[nd.idx]
-        ins = [s.t for s in st.pin]
+        x6 = bool(eng.split)                        # bf16x6: the convs read the split planes only
+        ins = [s.split if x6 else s.t for s in st.pin]
         if pos is not None:                         # below a switch: gather the inputs of the examples that continue
-            for slot, dst in zip(st.pin, self.cin[nd.idx]):
+            for slot, src, dst in zip(st.pin, ins, self.cin[nd.idx]):
                 g = slot.geo
-                L.gather_images(_vp(slot.t), par[0], g.P, _vp(pos), _vp(sink_cnt), _vp(dst), n, g.P, slot.C, g.H, g.W,
-                                g.G, dt, S)
+                L.gather_images(_vp(src), par[0], g.P, _vp(pos), _vp(sink_cnt), _vp(dst), n, g.P,
+                                3 * slot.C if x6 else slot.C, g.H, g.W, g.G, BF16 if x6 else dt, S)
             ins = self.cin[nd.idx]
         rt = plan.rtr.get(nd.idx)
         if self.dyn_k and rt is not None:           # the router's k_cpt feature, in this node's compact order
@@ -318,13 +331,28 @@ class CompactEvaluator:
         for k, sc in enumerate(st.sc):
             g = sc.geo
             prev = st.sc[k - 1] if k > 0 else None
-            L.stencil_gemm_counted(_vp(ins[k]), sc.K0, _vp(prev.pooled) if prev is not None else None, sc.K1, _vp(sc.Wf),
-                                   9, eng.tptr(sc.bk), _vp(sc.lin), sc.N, 0, None, 0, 0, n, g.H, g.W, g.G, g.P,
-                                   None, 0, None, dt, dt, eng.impl, _vp(cnt), S)
+            if x6:                                  # the dense plan's launches (Plan._build_conv_fwd_split), fp32 out
+                for ps in sc.passes:
+                    src = ins[k] if ps.src == 'h' else prev.pooled_split
+                    L.stencil_gemm_counted(_vp(src), ps.na0 * ps.K, _vp(src) if ps.na1 else None, ps.na1 * ps.K,
+                                           _vp(ps.W), 9, eng.tptr(sc.bk) if ps.first else None, _vp(sc.lin), sc.N,
+                                           0 if ps.first else 1, None, 0, 0, n, g.H, g.W, g.G, g.P, None, 0, None,
+                                           BF16, F32, 1, _vp(cnt), S)
+            else:
+                L.stencil_gemm_counted(_vp(ins[k]), sc.K0, _vp(prev.pooled) if prev is not None else None, sc.K1,
+                                       _vp(sc.Wf), 9, eng.tptr(sc.bk), _vp(sc.lin), sc.N, 0, None, 0, 0, n, g.H, g.W,
+                                       g.G, g.P, None, 0, None, dt, dt, eng.impl, _vp(cnt), S)
             if sc.live or sc.pooled is not None:
                 L.bn_relu_pool_fwd_counted(_vp(sc.lin), sc.N, n, g.H, g.W, g.G, g.P, _vp(sc.ss) if sc.live else None,
                                            _vp(sc.act), _vp(sc.pooled), sc.geo_p.P if sc.pooled is not None else 0,
                                            _vp(sc.feat), plan.Balloc, dt, _vp(cnt), S)
+                if x6:                              # the split operands of the convs that read act / pooled
+                    if sc.act_split is not None:
+                        L.split_planes3_counted(_vp(sc.act), sc.N, n, g.H, g.W, g.G, g.P, _vp(sc.act_split), _vp(cnt), S)
+                    if sc.pooled_split is not None:
+                        q = sc.geo_p
+                        L.split_planes3_counted(_vp(sc.pooled), sc.N, n, q.H, q.W, q.G, q.P, _vp(sc.pooled_split),
+                                                _vp(cnt), S)
         if not nd.kids:
             return
         if plan.umma_heads and nd.idx in plan.heads:

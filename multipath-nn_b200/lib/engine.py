@@ -1686,21 +1686,23 @@ class _Plan:
                                   ss=_vp(sc.ss), mr=_vp(sc.mr), count=float(B * geo.H * geo.W),
                                   d=float(bn.hypers.d), eps=float(bn.hypers.ε), defer=1 if eng.defer_bn else 0)
             bnp = ctypes.c_void_p(sc.bnf.ctypes.data)
-        two = prev is not None
-        todo = [(sc.src.split, K0, sc.K0real, W, sc.src.split_op, 'h') for W in sc.W3h]
-        if two:
-            todo += [(prev.pooled_split, K1, K1, W, prev.post_op, 'v') for W in sc.W3v]
-        for i, (src, K, Kreal, W, dep, which) in enumerate(todo):
-            na0, na1, _ = passes[i % len(passes)]
-            first, last = i == 0, i == len(todo) - 1
+        # the scale's launches in order -- source ('h': the split input, 'v': the split pooled predecessor), its K,
+        # parts of it in A0 / A1, packed weights, first (bias, no accumulation) / last (BN moments) -- read by the ops
+        # below and by the compacted walk (lib/compact_eval.py), which launches the same list on its own batch
+        sc.passes = [Ns(src='h', K=K0, Kreal=sc.K0real, na0=na0, na1=na1, W=W) for (na0, na1, _), W in zip(passes, sc.W3h)]
+        if prev is not None:
+            sc.passes += [Ns(src='v', K=K1, Kreal=K1, na0=na0, na1=na1, W=W) for (na0, na1, _), W in zip(passes, sc.W3v)]
+        for i, ps in enumerate(sc.passes):
+            ps.first, ps.last = i == 0, i == len(sc.passes) - 1
+            src, dep = (sc.src.split, sc.src.split_op) if ps.src == 'h' else (prev.pooled_split, prev.post_op)
 
-            def conv(src=src, K=K, W=W, na0=na0, na1=na1, first=first, last=last):
-                L.conv_acc_bn_stats(_vp(src), na0 * K, _vp(src) if na1 else None, na1 * K, _vp(W),
-                                    eng.tptr(sc.bk) if first else None, _vp(sc.lin), N, 0 if first else 1, *geo.args(),
-                                    bnp if last else None, BF16, F32, 1, S())
-            self._tag(conv, 'conv_fwd', desc='H%d K3x%d N%d%s' % (geo.H, K, N, '' if first else ' +acc'),
-                      flops=3 * 2.0 * B * geo.H * geo.W * 9 * Kreal * N,
-                      nbytes=B * geo.H * geo.W * (3 * K * 2 + (1 if first else 2) * N * 4))
+            def conv(src=src, ps=ps):
+                L.conv_acc_bn_stats(_vp(src), ps.na0 * ps.K, _vp(src) if ps.na1 else None, ps.na1 * ps.K, _vp(ps.W),
+                                    eng.tptr(sc.bk) if ps.first else None, _vp(sc.lin), N, 0 if ps.first else 1,
+                                    *geo.args(), bnp if ps.last else None, BF16, F32, 1, S())
+            self._tag(conv, 'conv_fwd', desc='H%d K3x%d N%d%s' % (geo.H, ps.K, N, '' if ps.first else ' +acc'),
+                      flops=3 * 2.0 * B * geo.H * geo.W * 9 * ps.Kreal * N,
+                      nbytes=B * geo.H * geo.W * (3 * ps.K * 2 + (1 if ps.first else 2) * N * 4))
             conv.lane = sc.lane
             self._after(conv, dep)
             self.fwd_ops.append(conv)

@@ -1,6 +1,6 @@
 """Routed inference (`net.predict`, and `net.predictor`, the same walk replayed as one CUDA graph) against the dense
-'ev' forward (`Engine.forward` on an eval plan) on cifar10-ac at the real architecture in bf16, for three router
-settings and B in {128, 4096, 16384}:
+'ev' forward (`Engine.forward` on an eval plan) on cifar10-ac at the real architecture in bf16 (or --precision fp32 /
+bf16x6), for three router settings and B in {128, 4096, 16384}:
 
   (a) fresh net: the zero-initialised last router layer ties, every example exits at stage 0;
   (b) every switch biased to continue: every example runs the whole chain (worst case for the compaction);
@@ -11,6 +11,7 @@ rewritten before every timed call so that no path reads its inputs or weights fr
 ms per call (median of the repeats), images/s, mean ops as a fraction of the whole tree, the exit histogram,
 the host synchronisations of one predict call (one per switch visited per chunk, plus the final read-back) and
 those of one predictor call with device inputs (counted by torch's sync debug mode)."""
+import argparse
 import os
 import subprocess
 import sys
@@ -35,7 +36,7 @@ def card():
     return q.stdout.strip().splitlines()[torch.cuda.current_device()] if q.returncode == 0 else 'nvidia-smi failed'
 
 
-def make_net(setting):
+def make_net(setting, precision):
     layer_types.seed(0)
     net = ah.ac_chain(k_cpt=4e-9)((32, 32, 3), (10,))
     if setting == 'continue':
@@ -48,7 +49,7 @@ def make_net(setting):
                 last.params.b.assign(b)
     elif setting == 'random':
         randomize_routers(net)
-    return net.configure(precision='bf16')
+    return net.configure(precision=precision)
 
 
 def switches_visited(eng, exit_, B):
@@ -80,6 +81,9 @@ def predictor_syncs(call):
 
 
 def main():
+    ap = argparse.ArgumentParser(description=__doc__.split('\n')[0])
+    ap.add_argument('--precision', default='bf16', choices=['bf16', 'fp32', 'bf16x6'])
+    args = ap.parse_args()
     torch.cuda.init()
     print('card (name, power limit, max SM clock): %s' % card())
     rng = np.random.default_rng(0)
@@ -89,7 +93,7 @@ def main():
         'routers', 'B', 'dense ms', 'predict', 'predictor', 'dense im/s', 'predict', 'predictor', 'x pred', 'x dense',
         'ops frac', 'syncs', 'graph', 'exits'))
     for setting in ('fresh', 'continue', 'random'):
-        net = make_net(setting)
+        net = make_net(setting, args.precision)
         eng = net._get_engine()
         ops_tree = float(sum(l.n_ops + (l.router.n_ops if l.router is not None else 0) for l in net.layers))
         for B in BATCHES:
