@@ -21,11 +21,12 @@ example's softmax, predicted class, exit leaf and path cost (mpnn_leaf_emit) ins
 Nets with a per-example k_cpt carry the router feature alpha_cpt * k_cpt through the compaction by original
 example id (mpnn_gather_feature), so one batch may mix cost budgets.
 
-In bf16x6 precision the convs read only the (hi | mid | lo) bf16 splits of their fp32 inputs: the root splits every
-pyramid scale after packing it, the gathers below a switch move the parent's split planes, and every scale launches the
-dense eval plan's list of passes (`sc.passes`, Plan._build_conv_fwd_split) into fp32 planes, then BN / ReLU / pool in
-fp32 and the counted splits (mpnn_split_planes3_counted) of what the next convs read.  The heads are the CUDA-core
-fp32 ones, as in the dense plan.
+Every scale launches the dense eval plan's list of conv passes (`sc.passes`, _Plan._conv_passes) on the node's
+inputs: one launch in fp32 and bf16.  In bf16x6 precision the convs read only the (hi | mid | lo) bf16 splits of their
+fp32 inputs: the root splits every pyramid scale after packing it, the gathers below a switch move the parent's split
+planes, and the passes write fp32 planes, followed by BN / ReLU / pool in fp32 and the counted splits
+(mpnn_split_planes3_counted) of what the next convs read.  The heads are the CUDA-core fp32 ones, as in the dense
+plan.
 
 One walker serves both ways of running the tree.  Every kernel takes its live batch as a pair (launch batch,
 device count) through the counted entry points, and only the step at a switch differs:
@@ -43,13 +44,9 @@ from types import SimpleNamespace as Ns
 import numpy as np
 import torch
 
-from lib.engine import BF16, F32, _RT_FWD, _gc_off, _vp
+from lib.engine import BF16, _RT_FWD, _gc_off, _vp, node_ops
 
 __all__ = ['CompactEvaluator', 'RoutedPredictor']
-
-
-def _node_ops(nd):
-    return nd.layer.n_ops + (nd.router.n_ops if nd.router is not None else 0)
 
 
 class _LeafStats:
@@ -118,20 +115,14 @@ class CompactEvaluator:
                 i = eng.nodes[i].parent
             tot = 0.0
             for i in sorted(on_path):
-                tot += float(_node_ops(eng.nodes[i]))
+                tot += float(node_ops(eng.nodes[i]))
             self.path_ops.append(tot)
         zi = lambda *shape: torch.zeros(shape, dtype=torch.int32, device=dev)
         self.sw = {}
         for nd in eng.nodes:
             if len(nd.kids) > 1:
                 ns = len(nd.kids)
-                rt = plan.rtr[nd.idx]
-                P = lambda lay, k: eng.tptr(getattr(lay.params, k))
-                tab = plan._desc_table(_RT_FWD, [dict(
-                    Z1=rt.Z1, g1=P(rt.bn1, 'γ'), b1=P(rt.bn1, 'β'), m1=P(rt.bn1, 'm_avg'), v1=P(rt.bn1, 'v_avg'),
-                    W2=P(rt.fc2, 'w'), bias2=P(rt.fc2, 'b'), g2=P(rt.bn2, 'γ'), b2=P(rt.bn2, 'β'),
-                    m2=P(rt.bn2, 'm_avg'), v2=P(rt.bn2, 'v_avg'), W3=P(rt.fc3, 'w'), bias3=P(rt.fc3, 'b'),
-                    Z2=rt.Z2, R=rt.R, save=rt.save, ns=ns)])
+                tab = plan._desc_table(_RT_FWD, [plan.rtr[nd.idx].fwd_desc])
                 host = torch.zeros(ns, dtype=torch.int32)
                 self.sw[nd.idx] = dict(tab=tab, pos=zi(ns, B), orig=zi(ns, B), count=zi(ns),
                                        host=host if eng.dry else host.pin_memory())
@@ -331,17 +322,11 @@ class CompactEvaluator:
         for k, sc in enumerate(st.sc):
             g = sc.geo
             prev = st.sc[k - 1] if k > 0 else None
-            if x6:                                  # the dense plan's launches (Plan._build_conv_fwd_split), fp32 out
-                for ps in sc.passes:
-                    src = ins[k] if ps.src == 'h' else prev.pooled_split
-                    L.stencil_gemm_counted(_vp(src), ps.na0 * ps.K, _vp(src) if ps.na1 else None, ps.na1 * ps.K,
-                                           _vp(ps.W), 9, eng.tptr(sc.bk) if ps.first else None, _vp(sc.lin), sc.N,
-                                           0 if ps.first else 1, None, 0, 0, n, g.H, g.W, g.G, g.P, None, 0, None,
-                                           BF16, F32, 1, _vp(cnt), S)
-            else:
-                L.stencil_gemm_counted(_vp(ins[k]), sc.K0, _vp(prev.pooled) if prev is not None else None, sc.K1,
-                                       _vp(sc.Wf), 9, eng.tptr(sc.bk), _vp(sc.lin), sc.N, 0, None, 0, 0, n, g.H, g.W,
-                                       g.G, g.P, None, 0, None, dt, dt, eng.impl, _vp(cnt), S)
+            for ps in sc.passes:                    # the dense plan's conv launches (Plan._conv_passes)
+                A0, K0, A1, K1 = plan.pass_operands(sc, prev, ps, h=ins[k])
+                L.stencil_gemm_counted(_vp(A0), K0, _vp(A1), K1, _vp(ps.W), 9, eng.tptr(sc.bk) if ps.first else None,
+                                       _vp(sc.lin), sc.N, 0 if ps.first else 1, None, 0, 0, n, g.H, g.W, g.G, g.P,
+                                       None, 0, None, *plan.conv_dtypes, _vp(cnt), S)
             if sc.live or sc.pooled is not None:
                 L.bn_relu_pool_fwd_counted(_vp(sc.lin), sc.N, n, g.H, g.W, g.G, g.P, _vp(sc.ss) if sc.live else None,
                                            _vp(sc.act), _vp(sc.pooled), sc.geo_p.P if sc.pooled is not None else 0,
@@ -357,10 +342,7 @@ class CompactEvaluator:
             return
         if plan.umma_heads and nd.idx in plan.heads:
             hd = plan.heads[nd.idx]
-            outs = ([(hd.Z16, 16)] if hd.leaf_off is not None else []) + \
-                ([(rt.Z1, eng.router_width)] if rt is not None else [])
-            outs.append((None, 0))
-            (o0, n0), (o1, n1) = outs[0], outs[1]
+            o0, n0, o1, n1 = hd.outs
             L.stencil_gemm_counted(_vp(st.feat), st.Fext, None, 0, _vp(hd.Wfc), 1, _vp(hd.bias), _vp(o0), n0, 0,
                                    _vp(o1), n1, 0, n, 0, 0, 0, plan.Balloc, None, 0, None, BF16, 2, 1, _vp(cnt), S)
         elif rt is not None:
@@ -399,7 +381,7 @@ class CompactEvaluator:
             acc += float(row[0])
         moc = 0.0
         for nd in eng.nodes:
-            moc += self.visits[nd.idx] * float(_node_ops(nd))
+            moc += self.visits[nd.idx] * float(node_ops(nd))
         out[(eng.net, 'acc')] = acc
         out[(eng.net, 'moc')] = moc / n
         return out

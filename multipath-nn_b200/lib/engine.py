@@ -212,6 +212,19 @@ class Geo:
         return (self.B, self.H, self.W, self.G, self.P)
 
 
+def node_ops(nd):
+    """operations of a node of the tree: its layer and its router (the cost the routing weighs)"""
+    return nd.layer.n_ops + (nd.router.n_ops if nd.router is not None else 0)
+
+
+def _slot(t, C, Creal, geo, sc=None, split=None, split_op=None, **kw):
+    """an output of a node that conv stages read: its planes tensor, channels (padded and real), geometry, the scale
+    that wrote it, its bf16 parts in the split modes and the launch that fills them, and the gradient written into it
+    (dact, by `writers` launches)"""
+    return Ns(t=t, C=C, Creal=Creal, geo=geo, dact=None, writers=0, sc=sc, consumers=0, fused_red=False, split=split,
+              split_op=split_op, **kw)
+
+
 class Engine:
     def __init__(self, net, precision='fp32', device=None, graphs=False, dist=False, impl=None,
                  dry_run=False):
@@ -889,8 +902,7 @@ class Engine:
         acc = np.zeros(B)
         moc = np.zeros(B)
         for nd in self.nodes:
-            ops = nd.layer.n_ops + (nd.router.n_ops if nd.router is not None else 0)
-            moc += p_ev[nd.idx] * ops
+            moc += p_ev[nd.idx] * node_ops(nd)
         for nd in self.regs:
             l = nd.layer
             d_cor = plan.reg[nd.idx].d_cor.cpu().numpy().astype(np.float64)
@@ -1020,8 +1032,7 @@ class _Plan:
             cpad = _ru(C0, 16 if (eng.dtype == BF16 or eng.split) else 8)
             geo = Geo(B, H0, W0)
             t = self.planes(cpad, geo)
-            slot = Ns(t=t, C=cpad, Creal=C0, geo=geo, dact=None, writers=0, sc=None, consumers=0, fused_red=False,
-                      split=None, split_op=None)
+            slot = _slot(t, cpad, C0, geo)
             # (planes beyond the image's channels stay at their one-time zero fill: only the live ones are written)
             pk = lambda: L.pack_input(_vp(self.x0), B, H0, W0, C0, 1, _vp(t), min(cpad, _ru(C0, 8)), geo.G, geo.P, eng.dtype, eng.stream)
             pk.lane = 3
@@ -1076,6 +1087,9 @@ class _Plan:
         fits = all((head_features(nd) + 16) // 8 * 32 * 16 <= 150 * 1024 for nd in with_heads)
         self.umma_heads = eng.impl == 1 and all(nd.fc.hypers.n_chan <= 16 for nd in eng.regs) and not eng.split and fits
         Balloc = _ru(B, 128) if self.umma_heads else _ru(B, 8)
+        # (operand, output, implementation) types of the conv launches: the split modes read bf16 parts, write fp32
+        self.conv_dtypes = (BF16, F32, 1) if eng.split else (dt, dt, impl)
+        self.conv_esz = (2, 4) if eng.split else (2, 2) if dt == BF16 else (4, 4)     # their bytes per element
         self.Balloc = Balloc
         self.node = {}
         self.reg, self.rtr, self.heads = {}, {}, {}
@@ -1098,8 +1112,7 @@ class _Plan:
                 for i in range(n_sc):
                     geo = Geo(B, H0 // 2 ** i, W0 // 2 ** i)
                     t = self.planes(cpad, geo)
-                    st.out.append(Ns(t=t, C=cpad, Creal=C0, geo=geo, dact=None, writers=0, sc=None, consumers=0, fused_red=False,
-                                     split=None, split_op=None))
+                    st.out.append(_slot(t, cpad, C0, geo))
                     if getattr(nd, 'lln', None) is not None:
                         # MultiscaleLLN behind ToPyramid: normalise the scale in fp32 NHWC, then pack that
                         tmp = self.f32(B, geo.H, geo.W, C0)
@@ -1247,12 +1260,10 @@ class _Plan:
             if nd.kind == 'reg':
                 r = self.reg[nd.idx]
                 par = self.node[nd.parent]
-                coef = (lambda nd=nd: ctypes.c_void_p(self.p_tr.data_ptr() + 4 * nd.idx * B)) if eng.dynamic \
-                    else (lambda: None)
                 if self.umma_heads:
                     hd = self.heads[nd.parent]
                     dzp = ctypes.c_void_p(hd.dZ.data_ptr() + (hd.leaf_off // 8) * Balloc * 16)
-                    ceb = lambda r=r, coef=coef, dzp=dzp: self._loss_bwd(r, coef(), None, dzp, eng.gptr(r.fc.params.b))
+                    ceb = lambda r=r, nd=nd, dzp=dzp: self._loss_bwd(r, self._coef(nd), None, dzp, eng.gptr(r.fc.params.b))
                     ceb.lane = hd.lane
                     # a stage without a router only needs p_tr (forward): its head gradients are issued
                     # ahead of the routing backward so the deepest conv chain starts under it
@@ -1260,7 +1271,7 @@ class _Plan:
                     hd.ceb_op = ceb
                     self.bwd_ops.append(ceb if ceb.early else self._after(ceb, self.bwd_head_dep))
                 else:
-                    self.bwd_ops.append(lambda r=r, coef=coef: self._loss_bwd(r, coef(), _vp(r.dZ), None, None))
+                    self.bwd_ops.append(lambda r=r, nd=nd: self._loss_bwd(r, self._coef(nd), _vp(r.dZ), None, None))
                     self.bwd_ops.append(lambda r=r, par=par: L.fc_bwd_weight(
                         _vp(par.feat), par.F, Balloc, B, None, _vp(r.dZ), r.n,
                         eng.gptr(r.fc.params.w), eng.gptr(r.fc.params.b), dt, S()))
@@ -1368,10 +1379,11 @@ class _Plan:
         if rt is not None:
             outs.append((rt.Z1, W))
         outs.append((None, 0))
-        (o0, n0), (o1, n1) = outs[0], outs[1]
+        hd.outs = outs[0] + outs[1]                  # (out0, N0, out1, N1) of the GEMM
         self.heads[nd.idx] = hd
 
         def gemm():
+            o0, n0, o1, n1 = hd.outs
             L.stencil_gemm(_vp(st.feat), Fext, None, 0, _vp(hd.Wfc), 1, _vp(hd.bias), _vp(o0), n0, 0, _vp(o1), n1, 0,
                            B, 0, 0, 0, Balloc, None, 0, None, BF16, 2, 1, S())
         self._tag(gemm, 'fc_fwd', desc='F%d N%d' % (Fext, hd.N), flops=2.0 * B * F * hd.N, nbytes=B * F * 2)
@@ -1381,6 +1393,10 @@ class _Plan:
         self.last_head_op = gemm
         self.head_ops.append(gemm)
         self.fwd_ops.append(gemm)
+
+    def _coef(self, nd):
+        """per-example weight of a node's costs in the backward pass: its row of p_tr when routed, else none"""
+        return ctypes.c_void_p(self.p_tr.data_ptr() + 4 * nd.idx * self.B) if self.eng.dynamic else None
 
     def _loss_bwd(self, r, coef, dZ, dZp, dbias):
         """gradient of a leaf's error layer wrt the LinTrans output (fp32 rows and / or the bf16 planes operand)"""
@@ -1456,6 +1472,7 @@ class _Plan:
     def _build_rcm_fwd(self, nd, st, Balloc):
         eng, L, B = self.eng, self.eng.L, self.B
         dt, impl = eng.dtype, eng.impl
+        ein, eout = self.conv_esz
         S = lambda: eng.stream
         lay = nd.layer
         cm, mbn = nd.cm, nd.mbn
@@ -1515,7 +1532,6 @@ class _Plan:
                     self.kplanes.append(sc.feat[st.F // 8, :, 0])
                 if pooled_out or gmp:
                     sc.feat = None                  # written by the pooling kernel (st.feat), not by BN / ReLU
-            sc.Wf = None if eng.split else self.zeros((9, (K0 + K1) // 8, N, 8), eng.tdtype)
             sc.ss = self.f32(2, N)
             sc.mr = self.f32(2, N)
             sc.bn = mbn.comps[k]
@@ -1525,48 +1541,56 @@ class _Plan:
             sc.wh, sc.wv, sc.bk = wh, wv, bk
             if tuple(wh.shape[:2]) != (3, 3):
                 raise NotImplementedError('engine: conv window %s' % (wh.shape[:2],))
-            if not eng.split:
-                self._pack(wh, sc.Wf, sc.K0real, sc.N, 0, 0, sc.K0 + sc.K1, 0, sc.N)
-                if wv is not None:
-                    self._pack(wv, sc.Wf, sc.K1, sc.N, 0, sc.K0, sc.K0 + sc.K1, 0, sc.N)
             prev = st.sc[k - 1] if k > 0 else None
             use_stats = sc.live and train
-            if eng.split:
-                self._build_conv_fwd_split(sc, prev, use_stats, B, Balloc, st)
-                st.sc.append(sc)
-                st.out.append(Ns(t=sc.act, C=N, Creal=N, geo=geo, dact=None, writers=0, sc=sc, consumers=0, fused_red=False,
-                                 split=getattr(sc, 'act_split', None), split_op=getattr(sc, 'post_op', None)))
-                continue
+            sc.lane = 3 + int(round(np.log2(eng.net.hypers.x0_shape[0] / geo.H)))
+            sc.act_split = sc.pooled_split = None
 
             # small tensors without a pooled output (the coarsest scale of a stage at the reference's batch): the conv
             # stores `lin` only, and ONE cluster launch takes the statistics and applies BN / ReLU (mpnn_bn_fwd_small)
-            small_f = (use_stats and not eng.defer_bn and eng.bn_small and sc.pooled is None
+            small_f = (use_stats and not eng.split and not eng.defer_bn and eng.bn_small and sc.pooled is None
                        and B * geo.H * geo.W <= _BN_SMALL_MAX_PIXELS and (sc.act is not None or sc.feat is not None))
+            bnf = None
             if use_stats and not small_f:
                 # train-mode BN statistics ride on the conv launch (last CTA finalises): no bn_finalize
                 bn = sc.bn
                 sc.acc_f = self._acc_f(2 * N + 1) if eng.defer_bn else self.zeros(2 * N + 1, torch.float64)
-                sc.bnf = _host_struct(_BN_FUSE, acc=_vp(sc.acc_f), gamma=eng.tptr(bn.params.γ), beta=eng.tptr(bn.params.β),
-                                      m_avg=eng.tptr(bn.params.m_avg), v_avg=eng.tptr(bn.params.v_avg),
-                                      ss=_vp(sc.ss), mr=_vp(sc.mr), count=float(B * geo.H * geo.W),
-                                      d=float(bn.hypers.d), eps=float(bn.hypers.ε), defer=1 if eng.defer_bn else 0)
+                sc.bnf = bnf = _host_struct(
+                    _BN_FUSE, acc=_vp(sc.acc_f), gamma=eng.tptr(bn.params.γ), beta=eng.tptr(bn.params.β),
+                    m_avg=eng.tptr(bn.params.m_avg), v_avg=eng.tptr(bn.params.v_avg), ss=_vp(sc.ss), mr=_vp(sc.mr),
+                    count=float(B * geo.H * geo.W), d=float(bn.hypers.d), eps=float(bn.hypers.ε),
+                    defer=1 if eng.defer_bn else 0)
+            sc.passes = self._conv_passes(sc)
+            for ps in sc.passes:
+                A0, K0p, A1, K1p = self.pass_operands(sc, prev, ps)
 
-                def conv(sc=sc, prev=prev):
-                    L.conv_bn_stats(_vp(sc.src.t), sc.K0, _vp(prev.pooled) if prev is not None else None, sc.K1,
-                                    _vp(sc.Wf), eng.tptr(sc.bk), _vp(sc.lin), sc.N, *sc.geo.args(),
-                                    ctypes.c_void_p(sc.bnf.ctypes.data), dt, impl, S())
-            else:
-                def conv(sc=sc, prev=prev):
-                    L.stencil_gemm(_vp(sc.src.t), sc.K0, _vp(prev.pooled) if prev is not None else None, sc.K1,
-                                   _vp(sc.Wf), 9, eng.tptr(sc.bk), _vp(sc.lin), sc.N, 0, None, 0, 0,
-                                   *sc.geo.args(), None, 0, None, dt, dt, impl, S())
-            self._tag(conv, 'conv_fwd', desc='H%d K%d+%d N%d' % (sc.geo.H, sc.K0, sc.K1, sc.N), flops=2.0 * B * sc.geo.H * sc.geo.W * 9 * (sc.K0real + sc.K1) * sc.N,
-                      nbytes=B * sc.geo.H * sc.geo.W * (sc.K0 + sc.K1 + sc.N) * (2 if dt == BF16 else 4))
-            sc.lane = 3 + int(round(np.log2(eng.net.hypers.x0_shape[0] / geo.H)))
-            conv.lane = sc.lane
-            self._after(conv, getattr(prev, 'post_op', None) if prev is not None else None)   # pooled input
-            self._after(conv, getattr(src, 'op', None))        # a MaxPool-ed parent tensor comes from another lane
-            self.fwd_ops.append(conv)
+                def conv(sc=sc, ps=ps, A0=A0, K0p=K0p, A1=A1, K1p=K1p, bnf=bnf):
+                    bias = eng.tptr(sc.bk) if ps.first else None
+                    bnp = ctypes.c_void_p(bnf.ctypes.data) if bnf is not None and ps.last else None
+                    if eng.split:
+                        L.conv_acc_bn_stats(_vp(A0), K0p, _vp(A1), K1p, _vp(ps.W), bias, _vp(sc.lin), sc.N,
+                                            0 if ps.first else 1, *sc.geo.args(), bnp, *self.conv_dtypes, S())
+                    elif bnp is not None:
+                        L.conv_bn_stats(_vp(A0), K0p, _vp(A1), K1p, _vp(ps.W), bias, _vp(sc.lin), sc.N, *sc.geo.args(),
+                                        bnp, dt, impl, S())
+                    else:
+                        L.stencil_gemm(_vp(A0), K0p, _vp(A1), K1p, _vp(ps.W), 9, bias, _vp(sc.lin), sc.N, 0, None, 0, 0,
+                                       *sc.geo.args(), None, 0, None, *self.conv_dtypes, S())
+                used = [a for a in (ps.a0, ps.a1) if a is not None]
+                srcs = {s for s, _ in used}
+                Kreal = sum(n * (sc.K0real if s == 'h' else K1) for s, n in used)
+                if eng.split:                       # one source per pass: its parts along K
+                    desc = 'H%d K%dx%d N%d%s' % (geo.H, sum(n for _, n in used), K0 if 'h' in srcs else K1, N,
+                                                 '' if ps.first else ' +acc')
+                else:
+                    desc = 'H%d K%d+%d N%d' % (geo.H, K0, K1, N)
+                self._tag(conv, 'conv_fwd', desc=desc, flops=2.0 * B * geo.H * geo.W * 9 * Kreal * N,
+                          nbytes=B * geo.H * geo.W * ((K0p + K1p) * ein + (1 if ps.first else 2) * N * eout))
+                conv.lane = sc.lane
+                # the pooled predecessor, and the input (a MaxPool-ed parent tensor comes from another lane)
+                self._after(conv, getattr(prev, 'post_op', None) if 'v' in srcs else None,
+                            (src.split_op if eng.split else getattr(src, 'op', None)) if 'h' in srcs else None)
+                self.fwd_ops.append(conv)
             if sc.live and not use_stats:
                 bn = sc.bn
 
@@ -1601,6 +1625,11 @@ class _Plan:
                 self.fwd_ops.append(post)
                 if sc.feat is not None:
                     st.feat_op = post
+                if eng.split:                       # the bf16 parts of what the next convs read
+                    if sc.act is not None:
+                        sc.act_split, sc.post_op = self._split(sc.act, N, geo, sc.lane)
+                    if sc.pooled is not None:
+                        sc.pooled_split, sc.post_op = self._split(sc.pooled, N, sc.geo_p, sc.lane)
             st.sc.append(sc)
             sc.keep = getattr(nd, 'keep', 1.0)
             if sc.keep != 1.0:
@@ -1647,96 +1676,48 @@ class _Plan:
                 if sc.mp.feat is not None:
                     st.feat_op = pool
                 if pooled_out:
-                    st.out.append(Ns(t=sc.mp.out, C=N, Creal=N, geo=geo_q, dact=None, writers=0, sc=None, consumers=0,
-                                     fused_red=False, split=None, split_op=None, op=pool, dact_ops=[]))
+                    st.out.append(_slot(sc.mp.out, N, N, geo_q, op=pool, dact_ops=[]))
                     continue
-            st.out.append(Ns(t=sc.act, C=N, Creal=N, geo=geo, dact=None, writers=0, sc=sc, consumers=0, fused_red=False,
-                             split=getattr(sc, 'act_split', None), split_op=getattr(sc, 'post_op', None)))
+            st.out.append(_slot(sc.act, N, N, geo, sc=sc, split=sc.act_split, split_op=getattr(sc, 'post_op', None)))
 
-    def _build_conv_fwd_split(self, sc, prev, use_stats, B, Balloc, st):
-        """bf16x3 mode: the conv of one scale as up to two tcgen05 launches over (hi | lo) operands --
-        horizontal input, then the pooled predecessor accumulated on top -- with fp32 planes out; the BN moments
-        ride on the last launch.  Followed by the fp32 BN / ReLU / pool kernel and the splits of what it wrote."""
-        eng, L = self.eng, self.eng.L
-        S = lambda: eng.stream
-        geo, N, K0, K1 = sc.geo, sc.N, sc.K0, sc.K1
-        sc.lane = 3 + int(round(np.log2(eng.net.hypers.x0_shape[0] / geo.H)))
+    def _conv_passes(self, sc):
+        """The conv launches of one scale, in order.  A pass names its operands A0 and A1 as (source, number of parts)
+        -- 'h' the scale's input, 'v' the pooled predecessor -- and carries its packed weights and its first (bias, no
+        accumulation) and last (BN moments) flags.  The plain modes have one pass over both sources; the split modes
+        launch each source's _SPLIT_PASSES over its bf16 parts, accumulated into the same fp32 planes.  The compacted
+        walk (lib/compact_eval.py) launches the same list on its own batch."""
+        eng, N = self.eng, sc.N
+        srcs = [('h', sc.wh, sc.K0, sc.K0real)] + ([('v', sc.wv, sc.K1, sc.K1)] if sc.wv is not None else [])
+        if eng.split:
+            # weight parts along K as (weight, K, real K, pack mode): 0 = bf16(w), 4 = first residual, 8 = second
+            specs = [((s, na0), (s, na1) if na1 else None, [(w, K, Kr, mode) for mode in wparts])
+                     for s, w, K, Kr in srcs for na0, na1, wparts in _SPLIT_PASSES[eng.split]]
+        else:
+            specs = [(('h', 1), ('v', 1) if sc.wv is not None else None, [(w, K, Kr, 0) for _, w, K, Kr in srcs])]
+        passes = []
+        for a0, a1, parts in specs:
+            Ktot = sum(K for _, K, _, _ in parts)
+            W = self.zeros((9, Ktot // 8, N, 8), torch.bfloat16 if eng.split else eng.tdtype)
+            k_off = 0
+            for w, K, Kr, mode in parts:
+                self._pack(w, W, Kr, N, mode, k_off, Ktot, 0, N)
+                k_off += K
+            passes.append(Ns(a0=a0, a1=a1, W=W, first=not passes, last=False))
+        passes[-1].last = True
+        return passes
 
-        # launches of one source tensor as (parts of A0, parts of A1, weight parts along K): x3 = one launch
-        # [hi | lo | hi] x [hi; hi; lo]; x6 = two launches [hi | mid | lo] x [hi; hi; hi] and
-        # [hi | mid | hi] x [mid; mid; lo] (pack modes: 0 = hi, 4 = first residual, 8 = second residual)
-        passes = _SPLIT_PASSES[eng.split]
-
-        def packs(w, K, Kreal):
-            out = []
-            for _, _, wparts in passes:
-                W3 = self.zeros((9, 3 * K // 8, N, 8), torch.bfloat16)
-                for j, mode in enumerate(wparts):
-                    self._pack(w, W3, Kreal, N, mode, j * K, 3 * K, 0, N)
-                out.append(W3)
-            return out
-        sc.W3h = packs(sc.wh, K0, sc.K0real)
-        sc.W3v = packs(sc.wv, K1, K1) if sc.wv is not None else None
-        bnp = None
-        if use_stats:
-            bn = sc.bn
-            sc.acc_f = self._acc_f(2 * N + 1) if eng.defer_bn else self.zeros(2 * N + 1, torch.float64)
-            sc.bnf = _host_struct(_BN_FUSE, acc=_vp(sc.acc_f), gamma=eng.tptr(bn.params.γ), beta=eng.tptr(bn.params.β),
-                                  m_avg=eng.tptr(bn.params.m_avg), v_avg=eng.tptr(bn.params.v_avg),
-                                  ss=_vp(sc.ss), mr=_vp(sc.mr), count=float(B * geo.H * geo.W),
-                                  d=float(bn.hypers.d), eps=float(bn.hypers.ε), defer=1 if eng.defer_bn else 0)
-            bnp = ctypes.c_void_p(sc.bnf.ctypes.data)
-        # the scale's launches in order -- source ('h': the split input, 'v': the split pooled predecessor), its K,
-        # parts of it in A0 / A1, packed weights, first (bias, no accumulation) / last (BN moments) -- read by the ops
-        # below and by the compacted walk (lib/compact_eval.py), which launches the same list on its own batch
-        sc.passes = [Ns(src='h', K=K0, Kreal=sc.K0real, na0=na0, na1=na1, W=W) for (na0, na1, _), W in zip(passes, sc.W3h)]
-        if prev is not None:
-            sc.passes += [Ns(src='v', K=K1, Kreal=K1, na0=na0, na1=na1, W=W) for (na0, na1, _), W in zip(passes, sc.W3v)]
-        for i, ps in enumerate(sc.passes):
-            ps.first, ps.last = i == 0, i == len(sc.passes) - 1
-            src, dep = (sc.src.split, sc.src.split_op) if ps.src == 'h' else (prev.pooled_split, prev.post_op)
-
-            def conv(src=src, ps=ps):
-                L.conv_acc_bn_stats(_vp(src), ps.na0 * ps.K, _vp(src) if ps.na1 else None, ps.na1 * ps.K, _vp(ps.W),
-                                    eng.tptr(sc.bk) if ps.first else None, _vp(sc.lin), N, 0 if ps.first else 1,
-                                    *geo.args(), bnp if ps.last else None, BF16, F32, 1, S())
-            self._tag(conv, 'conv_fwd', desc='H%d K3x%d N%d%s' % (geo.H, ps.K, N, '' if ps.first else ' +acc'),
-                      flops=3 * 2.0 * B * geo.H * geo.W * 9 * ps.Kreal * N,
-                      nbytes=B * geo.H * geo.W * (3 * ps.K * 2 + (1 if ps.first else 2) * N * 4))
-            conv.lane = sc.lane
-            self._after(conv, dep)
-            self.fwd_ops.append(conv)
-        if sc.live and not use_stats:
-            bn = sc.bn
-
-            def fin(sc=sc, bn=bn):             # inference: scale/shift from the running moments
-                L.bn_finalize(None, 0, N, float(B * geo.H * geo.W), eng.tptr(bn.params.γ), eng.tptr(bn.params.β),
-                              eng.tptr(bn.params.m_avg), eng.tptr(bn.params.v_avg),
-                              float(bn.hypers.d), float(bn.hypers.ε), 0, _vp(sc.ss), _vp(sc.mr), S())
-            self._tag(fin, 'bn_finalize')
-            fin.lane = sc.lane
-            self.fwd_ops.append(fin)
-        sc.act_split = sc.pooled_split = None
-        if sc.live or sc.pooled is not None:
-            if use_stats and eng.defer_bn:
-                def post(sc=sc):
-                    L.bn_relu_pool_fwd_acc(_vp(sc.lin), N, *geo.args(), bnp, _vp(sc.act), _vp(sc.pooled),
-                                           sc.geo_p.P if sc.pooled is not None else 0, _vp(sc.feat), Balloc, F32, S())
+    def pass_operands(self, sc, prev, ps, h=None):
+        """[A0, K of A0, A1, K of A1] of a conv pass: 'h' is the scale's input (or `h`, the compacted walk's copy of
+        it), 'v' the pooled predecessor -- in the split modes their bf16 parts"""
+        out = []
+        for a in (ps.a0, ps.a1):
+            if a is None:
+                out += [None, 0]
+            elif a[0] == 'h':
+                out += [h if h is not None else sc.src.split if self.eng.split else sc.src.t, a[1] * sc.K0]
             else:
-                def post(sc=sc):
-                    L.bn_relu_pool_fwd(_vp(sc.lin), N, *geo.args(), _vp(sc.ss) if sc.live else None,
-                                       _vp(sc.act), _vp(sc.pooled), sc.geo_p.P if sc.pooled is not None else 0,
-                                       _vp(sc.feat), Balloc, F32, S())
-            self._tag(post, 'bn_fwd', desc='H%d C%d' % (geo.H, N), nbytes=B * geo.H * geo.W * N * 4 * (1 + (sc.act is not None) + 0.25 * (sc.pooled is not None) + (sc.feat is not None)))
-            post.lane = sc.lane
-            self.fwd_ops.append(post)
-            sc.post_op = post
-            if sc.feat is not None:
-                st.feat_op = post
-            if sc.act is not None:
-                sc.act_split, sc.post_op = self._split(sc.act, N, geo, sc.lane)
-            if sc.pooled is not None:
-                sc.pooled_split, sc.post_op = self._split(sc.pooled, N, sc.geo_p, sc.lane)
+                out += [prev.pooled_split if self.eng.split else prev.pooled, a[1] * sc.K1]
+        return out
 
     def _bn_bwd_bufs(self, sc):
         """sums / fp64 accumulator / finalisation struct of a scale's BatchNorm backward (shared by the
@@ -1753,6 +1734,7 @@ class _Plan:
     def _build_rcm_bwd(self, nd, Balloc):
         eng, L, B = self.eng, self.eng.L, self.B
         dt, impl = eng.dtype, eng.impl
+        ein, eout = self.conv_esz
         S = lambda: eng.stream
         st = self.node[nd.idx]
         lay = nd.layer
@@ -1821,11 +1803,10 @@ class _Plan:
                 acc = 1 if dact is not None else 0
                 if dact is None:
                     dact = self.planes(sc.N, geo)
-                coef = (lambda nd=nd: ctypes.c_void_p(self.p_tr.data_ptr() + 4 * nd.idx * B)) if eng.dynamic \
-                    else (lambda: None)
 
-                def agrad(sc=sc, dact=dact, acc=acc, coef=coef):
-                    L.activity_bwd(_vp(sc.act), sc.N, *sc.geo.args(), coef(), 2.0 * sc.act_alpha / B, _vp(dact), acc, dt, S())
+                def agrad(sc=sc, dact=dact, acc=acc, nd=nd):
+                    L.activity_bwd(_vp(sc.act), sc.N, *sc.geo.args(), self._coef(nd), 2.0 * sc.act_alpha / B, _vp(dact),
+                                   acc, dt, S())
                 agrad.lane = sc.lane
                 if getattr(sc, 'mp', None) is None:
                     self._after(agrad, *getattr(st.out[k], 'dact_ops', []))
@@ -1870,30 +1851,34 @@ class _Plan:
             self._after(elt, getattr(sc, 'dpooled_op', None))      # written by scale k+1's data gradient
             self.bwd_ops.append(elt)
             prev = st.sc[k - 1] if k > 0 else None
+            # the gradient operand of both convolutions: dLin, or its bf16 parts in the split modes
+            g, g_op = sc.dlin, elt
             if eng.split:
-                self._build_conv_bwd_split(sc, prev, elt, par_grad, B)
-                continue
-
-            def wgrad(sc=sc, prev=prev):
-                L.stencil_wgrad(_vp(sc.src.t), sc.K0, sc.K0real, eng.gptr(sc.wh),
-                                _vp(prev.pooled) if prev is not None else None, sc.K1, sc.K1,
-                                eng.gptr(sc.wv) if sc.wv is not None else None,
-                                _vp(sc.dlin), sc.N, sc.N, None, 9, *sc.geo.args(), dt,   # db: see bn_relu_pool_bwd
-                                eng.impl_w if (sc.K0 + sc.K1 <= 128 and sc.N <= 256) else 0, S())
-            self._tag(wgrad, 'conv_wgrad', desc='H%d K%d+%d N%d' % (sc.geo.H, sc.K0, sc.K1, sc.N), flops=2.0 * B * sc.geo.H * sc.geo.W * 9 * (sc.K0real + sc.K1) * sc.N,
-                      nbytes=B * sc.geo.H * sc.geo.W * (sc.K0 + sc.K1 + sc.N) * (2 if dt == BF16 else 4))
-            wgrad.lane = 10 + (sc.lane - 3)          # weight gradients are mutually independent: one lane per scale
-            self.bwd_ops.append(self._after(wgrad, elt))
+                g, g_op = self._split(sc.dlin, sc.N, geo, sc.lane, ops=self.bwd_ops)
+                self._after(g_op, elt)
+            act0 = sc.src.split if eng.split else sc.src.t
+            act1 = None if prev is None else prev.pooled_split if eng.split else prev.pooled
+            part = lambda t, C, j: None if t is None else ctypes.c_void_p(t.data_ptr() + j * (C // 8) * geo.P * 8 * t.element_size())
+            # weight gradient: one launch per (activation part, gradient part) product kept -- all pairs with
+            # i + j < number of parts, reduced into the same fp32 gradient tensors
+            pairs = [(i, j) for j in range(eng.split) for i in range(eng.split - j)] if eng.split else [(0, 0)]
+            wdt, wimpl = (BF16, 1) if eng.split else (dt, eng.impl_w)
+            for n_, (i, j) in enumerate(pairs):
+                def wgrad(sc=sc, a0=part(act0, sc.K0, i), a1=part(act1, sc.K1, i), gj=part(g, sc.N, j)):
+                    L.stencil_wgrad(a0, sc.K0, sc.K0real, eng.gptr(sc.wh), a1, sc.K1, sc.K1,
+                                    eng.gptr(sc.wv) if sc.wv is not None else None,
+                                    gj, sc.N, sc.N, None, 9, *sc.geo.args(), wdt,   # db: see bn_relu_pool_bwd
+                                    wimpl if (sc.K0 + sc.K1 <= 128 and sc.N <= 256) else 0, S())
+                self._tag(wgrad, 'conv_wgrad', desc='H%d K%d+%d N%d%s' % (geo.H, sc.K0, sc.K1, sc.N, ' x%d[%d]' % (len(pairs), n_) if eng.split else ''),
+                          flops=2.0 * B * geo.H * geo.W * 9 * (sc.K0real + sc.K1) * sc.N,
+                          nbytes=B * geo.H * geo.W * (sc.K0 + sc.K1 + sc.N) * (2 if wdt == BF16 else 4))
+                wgrad.lane = 10 + (sc.lane - 3)          # weight gradients are mutually independent: one lane per scale
+                self.bwd_ops.append(self._after(wgrad, g_op))
             # data gradient: towards the parent's activation (N0) and the pooled predecessor (N1)
             N0 = sc.K0 if par_grad else 0
             N1 = sc.K1
             if N0 + N1 == 0:
                 continue
-            sc.Wd = self.zeros((9, sc.N // 8, N0 + N1, 8), eng.tdtype)
-            if N0:
-                self._pack(sc.wh, sc.Wd, sc.K0real, sc.N, 1, 0, sc.N, 0, N0 + N1)
-            if N1:
-                self._pack(sc.wv, sc.Wd, sc.K1, sc.N, 1, 0, sc.N, N0, N0 + N1)
             acc0 = 0
             out0 = None
             if N0:
@@ -1905,14 +1890,28 @@ class _Plan:
                 out0 = slot.dact
             if N1:
                 prev.dpooled = self.planes(sc.K1, geo)
+            # its launches: parts of the gradient operand in A0 / A1 as in the forward (_SPLIT_PASSES), the weights
+            # transposed with flipped taps and their parts along K (= output channels); later passes accumulate
+            specs = _SPLIT_PASSES[eng.split] if eng.split else [(1, 0, (0,))]
+            sc.dpasses = []
+            for na0, na1, wparts in specs:
+                Ktot = len(wparts) * sc.N
+                Wd = self.zeros((9, Ktot // 8, N0 + N1, 8), torch.bfloat16 if eng.split else eng.tdtype)
+                for j, mode in enumerate(wparts):
+                    if N0:
+                        self._pack(sc.wh, Wd, sc.K0real, sc.N, mode | 1, j * sc.N, Ktot, 0, N0 + N1)
+                    if N1:
+                        self._pack(sc.wv, Wd, sc.K1, sc.N, mode | 1, j * sc.N, Ktot, N0, N0 + N1)
+                first = not sc.dpasses
+                sc.dpasses.append(Ns(na0=na0, na1=na1, W=Wd, acc0=acc0 if first else 1, acc1=0 if first else 1))
             # BatchNorm-backward sums of the layer below ride on this data gradient when it is the only
             # producer of that layer's dAct (one consumer, no head gradient at that scale): removes the
             # bn_bwd_reduce pass over (lin, dAct)
             psc = sc.src.sc if N0 else None
             # (measured: a win where the 16- / 32-wide fast epilogue applies and the tensor is large; on
             #  small tensors and in the generic epilogue the stand-alone reduction is as fast or faster)
-            fuse = (psc is not None and eng.fuse_bn_red and impl == 1 and self.bn_train and sc.src.consumers == 1
-                    and psc.live and psc.feat is None and psc.N == N0 and (N0 + N1) in (16, 32)
+            fuse = (psc is not None and not eng.split and eng.fuse_bn_red and impl == 1 and self.bn_train
+                    and sc.src.consumers == 1 and psc.live and psc.feat is None and psc.N == N0 and (N0 + N1) in (16, 32)
                     and not getattr(psc, 'act_alpha', 0.0) and getattr(psc, 'keep', 1.0) == 1.0
                     and B * sc.geo.H * sc.geo.W >= eng.fuse_bn_red_min_rows)
             if fuse:
@@ -1921,86 +1920,30 @@ class _Plan:
                 sc.epi = _host_struct(_BN_BWD_EPI, lin=_vp(psc.lin), ss=_vp(psc.ss), mr=_vp(psc.mr), acc=_vp(psc.acc),
                                       sums=_vp(psc.sums), dgamma=eng.gptr(psc.bn.params.γ),
                                       dbeta=eng.gptr(psc.bn.params.β))
-
-                def dgrad(sc=sc, out0=out0, N0=N0, N1=N1, prev=prev):
-                    L.conv_dgrad_bn_reduce(_vp(sc.dlin), sc.N, _vp(sc.Wd), _vp(out0), N0,
-                                           _vp(prev.dpooled) if N1 else None, N1, *sc.geo.args(),
-                                           ctypes.c_void_p(sc.epi.ctypes.data), dt, impl, S())
-            else:
-                def dgrad(sc=sc, out0=out0, N0=N0, N1=N1, acc0=acc0, prev=prev):
-                    L.stencil_gemm(_vp(sc.dlin), sc.N, None, 0, _vp(sc.Wd), 9, None,
-                                   _vp(out0), N0, acc0, _vp(prev.dpooled) if N1 else None, N1, 0,
-                                   *sc.geo.args(), None, 0, None, dt, dt, impl, S())
-            self._tag(dgrad, 'conv_dgrad', desc='H%d K%d N%d+%d%s' % (sc.geo.H, sc.N, N0, N1, ' +bnred' if fuse else ''),
-                      flops=2.0 * B * sc.geo.H * sc.geo.W * 9 * sc.N * (N0 + N1),
-                      nbytes=B * sc.geo.H * sc.geo.W * (sc.N + N0 + N1 + (N0 if fuse else 0)) * (2 if dt == BF16 else 4))
-            dgrad.lane = sc.lane
-            if N1:
-                prev.dpooled_op = dgrad
-            if N0 and hasattr(sc.src, 'dact_ops'):
-                sc.src.dact_ops.append(dgrad)
-            self.bwd_ops.append(dgrad)
-
-    def _build_conv_bwd_split(self, sc, prev, elt, par_grad, B):
-        """bf16x3 mode: dLin (fp32) is split into (hi | lo); the weight gradient is three tcgen05 launches
-        (A_hi x G_hi, A_lo x G_hi, A_hi x G_lo, all reduced into the same fp32 gradient tensors), the data
-        gradient one launch over [G_hi | G_lo | G_hi] x [W_hi; W_hi; W_lo] with fp32 planes out."""
-        eng, L = self.eng, self.eng.L
-        S = lambda: eng.stream
-        geo, N, K0, K1 = sc.geo, sc.N, sc.K0, sc.K1
-        sc.dlin_split, sp = self._split(sc.dlin, N, geo, sc.lane, ops=self.bwd_ops)
-        self._after(sp, elt)
-        part = lambda t, C, j: ctypes.c_void_p(t.data_ptr() + j * (C // 8) * geo.P * 16) if t is not None else None
-        psp = prev.pooled_split if prev is not None else None
-        dWv = eng.gptr(sc.wv) if sc.wv is not None else None
-        # (activation part, gradient part) of every product kept: all pairs with i + j < number of parts
-        pairs = [(i, j) for j in range(eng.split) for i in range(eng.split - j)]
-        for n_, (i, j) in enumerate(pairs):
-            a0, a1, g = part(sc.src.split, K0, i), part(psp, K1, i), part(sc.dlin_split, N, j)
-
-            def wgrad(a0=a0, a1=a1, g=g):
-                L.stencil_wgrad(a0, K0, sc.K0real, eng.gptr(sc.wh), a1, K1, K1, dWv, g, N, N, None, 9,
-                                *geo.args(), BF16, 1 if (K0 + K1 <= 128 and N <= 256) else 0, S())
-            self._tag(wgrad, 'conv_wgrad', desc='H%d K%d+%d N%d x%d[%d]' % (geo.H, K0, K1, N, len(pairs), n_),
-                      flops=2.0 * B * geo.H * geo.W * 9 * (sc.K0real + K1) * N, nbytes=B * geo.H * geo.W * (K0 + K1 + N) * 2)
-            wgrad.lane = 10 + (sc.lane - 3)
-            self.bwd_ops.append(self._after(wgrad, sp))
-        N0 = K0 if par_grad else 0
-        N1 = K1
-        if N0 + N1 == 0:
-            return
-        passes = _SPLIT_PASSES[eng.split]
-        sc.Wd3 = []
-        for _, _, wparts in passes:
-            Wd = self.zeros((9, 3 * N // 8, N0 + N1, 8), torch.bfloat16)
-            for j, mode in enumerate(wparts):                                  # parts along K (= output channels)
-                if N0:
-                    self._pack(sc.wh, Wd, sc.K0real, N, mode | 1, j * N, 3 * N, 0, N0 + N1)
+            for i, ps in enumerate(sc.dpasses):
+                if fuse:
+                    def dgrad(sc=sc, ps=ps, out0=out0, N0=N0, N1=N1, prev=prev):
+                        L.conv_dgrad_bn_reduce(_vp(sc.dlin), sc.N, _vp(ps.W), _vp(out0), N0,
+                                               _vp(prev.dpooled) if N1 else None, N1, *sc.geo.args(),
+                                               ctypes.c_void_p(sc.epi.ctypes.data), dt, impl, S())
+                else:
+                    def dgrad(sc=sc, ps=ps, g=g, out0=out0, N0=N0, N1=N1, prev=prev):
+                        L.stencil_gemm(_vp(g), ps.na0 * sc.N, _vp(g) if ps.na1 else None, ps.na1 * sc.N, _vp(ps.W), 9,
+                                       None, _vp(out0), N0, ps.acc0, _vp(prev.dpooled) if N1 else None, N1, ps.acc1,
+                                       *sc.geo.args(), None, 0, None, *self.conv_dtypes, S())
+                parts = ps.na0 + ps.na1
+                self._tag(dgrad, 'conv_dgrad',
+                          desc='H%d K%s N%d+%d%s' % (geo.H, '%dx%d' % (parts, sc.N) if eng.split else sc.N, N0, N1,
+                                                     ' +bnred' if fuse else ' +acc' if i else ''),
+                          flops=2.0 * B * geo.H * geo.W * 9 * parts * sc.N * (N0 + N1),
+                          nbytes=B * geo.H * geo.W * (parts * sc.N * ein + (N0 + N1) * eout * (2 if i else 1)
+                                                      + (N0 * ein if fuse else 0)))
+                dgrad.lane = sc.lane
                 if N1:
-                    self._pack(sc.wv, Wd, K1, N, mode | 1, j * N, 3 * N, N0, N0 + N1)
-            sc.Wd3.append(Wd)
-        acc0, out0 = 0, None
-        if N0:
-            slot = sc.src
-            if slot.dact is None:
-                slot.dact = self.planes(slot.C, geo)
-            acc0 = 1 if slot.writers > 0 else 0
-            slot.writers += 1
-            out0 = slot.dact
-        if N1:
-            prev.dpooled = self.planes(K1, geo)
-        for i, ((na0, na1, _), Wd) in enumerate(zip(passes, sc.Wd3)):
-            def dgrad(out0=out0, acc0=acc0 if i == 0 else 1, acc1=0 if i == 0 else 1, na0=na0, na1=na1, Wd=Wd):
-                L.stencil_gemm(_vp(sc.dlin_split), na0 * N, _vp(sc.dlin_split) if na1 else None, na1 * N, _vp(Wd), 9, None,
-                               _vp(out0), N0, acc0, _vp(prev.dpooled) if N1 else None, N1, acc1,
-                               *geo.args(), None, 0, None, BF16, F32, 1, S())
-            self._tag(dgrad, 'conv_dgrad', desc='H%d K3x%d N%d+%d%s' % (geo.H, N, N0, N1, ' +acc' if i else ''),
-                      flops=3 * 2.0 * B * geo.H * geo.W * 9 * N * (N0 + N1),
-                      nbytes=B * geo.H * geo.W * (3 * N * 2 + (N0 + N1) * 4 * (2 if i else 1)))
-            dgrad.lane = sc.lane
-            if N1:
-                prev.dpooled_op = dgrad
-            self.bwd_ops.append(dgrad)
+                    prev.dpooled_op = dgrad
+                if N0 and hasattr(sc.src, 'dact_ops'):
+                    sc.src.dact_ops.append(dgrad)
+                self.bwd_ops.append(dgrad)
 
     # -- router ------------------------------------------------------------ #
     def _build_router_fwd(self, nd, Balloc, dyn_k, emit_fc=True):
@@ -2028,11 +1971,13 @@ class _Plan:
                 _vp(self.kextra) if dyn_k else None, W, _vp(rt.Z1), dt, S())
             self.fwd_ops.append(self._after(fcr, getattr(st, 'feat_op', None)))
         P = lambda lay, k: eng.tptr(getattr(lay.params, k))
-        # the tails of all routers run as ONE launch after the conv pipeline (see _build)
-        self.rt_fwd.append(dict(
+        # the tails of all routers run as ONE launch after the conv pipeline (see _build); the compacted walk launches
+        # each router's row on its own
+        rt.fwd_desc = dict(
             Z1=rt.Z1, g1=P(bn1, 'γ'), b1=P(bn1, 'β'), m1=P(bn1, 'm_avg'), v1=P(bn1, 'v_avg'),
             W2=P(fc2, 'w'), bias2=P(fc2, 'b'), g2=P(bn2, 'γ'), b2=P(bn2, 'β'), m2=P(bn2, 'm_avg'),
-            v2=P(bn2, 'v_avg'), W3=P(fc3, 'w'), bias3=P(fc3, 'b'), Z2=rt.Z2, R=rt.R, save=rt.save, ns=ns))
+            v2=P(bn2, 'v_avg'), W3=P(fc3, 'w'), bias3=P(fc3, 'b'), Z2=rt.Z2, R=rt.R, save=rt.save, ns=ns)
+        self.rt_fwd.append(rt.fwd_desc)
 
     def _build_router_bwd(self, nd, Balloc, dyn_k):
         eng, L, B = self.eng, self.eng.L, self.B
@@ -2065,7 +2010,7 @@ class _Plan:
         self.t_child = ti(child)
         self.t_floor = tf([n_leaves(nd.layer) / root_leaves for nd in nodes])
         self.t_sw = ti([getattr(nd, 'sw', -1) if len(nd.kids) > 1 else -1 for nd in nodes])
-        self.t_ops = tf([float(nd.layer.n_ops + (nd.router.n_ops if nd.router is not None else 0)) for nd in nodes])
+        self.t_ops = tf([float(node_ops(nd)) for nd in nodes])
         self.t_err = ti([nd.err if nd.kind == 'reg' else -1 for nd in nodes])
         self.p_tr = self.f32(nn, B)
         self.p_ev = self.f32(nn, B)
