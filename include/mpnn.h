@@ -526,6 +526,32 @@ int mpnn_route_compact_counted(const float* R, int ldr, int ns, int n, const int
 int mpnn_split_planes3_counted(const float* src, int C, int B, int H, int W, int G, int P, void* dst,
                                const int* count, void* stream);
 
+/* ---- dense ev-mode statistics on the device (train-nets:111-130, scripts/lib/desc.py:10-22) ----------------
+ * Adds the per-example statistics of one chunk of a dense 'ev' forward to a running fp64 total, restating in fp64
+ * what the host reduction of the same fp32 buffers computes.  descs: a DEVICE table of n_leaf leaf rows (ns == 0)
+ * followed by n_sw switch rows (ns = the switch's sinks); per example b < n:
+ *   leaf l (pe = p_ev[b], 1 when p_ev is NULL; dc = d_cor[b]), at total[l * (4 + 2*n_cls) + k]:
+ *     k = 0: pe*dc   1: pe*(1-dc)   2: c_err[b]   3: p_tr[b] (0 when p_tr is NULL)
+ *     4 + c: pe*dc*y[b][c]   4 + n_cls + c: pe*(1-dc)*y[b][c]                                   (c < n_cls)
+ *   switch s, at total[n_leaf * (4 + 2*n_cls) + s]: x_rte = (|R[b][0]| + ... + |R[b][ns-1]|) / ns   (R row-major)
+ *   then acc = sum over the leaves in table order of pe*dc, and moc = sum over the n_nodes nodes in order of
+ *   node_p_ev[i][b] * ops[i] (node_p_ev [n_nodes][B], NULL: 1; ops: DEVICE doubles).
+ * M = n_leaf * (4 + 2*n_cls) + n_sw + 2 totals.  Counted like the entry points of the section below: B is the
+ * capacity the grid is sized for, count (NULL: B) a DEVICE int holding the live n; rows at or past n are never read
+ * and n = 0 adds nothing.  Fixed-order reduction, no floating-point atomics: CTA c takes rows
+ * [c * MPNN_STATS_ROWS, (c + 1) * MPNN_STATS_ROWS) and each of its threads sums whole columns over them in row
+ * order into work[c][M] (work: >= ceil(B / MPNN_STATS_ROWS) * M doubles, scratch); a second kernel adds, per column,
+ * the CTAs' partials in CTA order to total.  The same inputs give the same bits, and chunks enter in call order. */
+#define MPNN_STATS_ROWS 32
+typedef struct {
+    const float* p_ev; const float* p_tr; const float* d_cor; const float* c_err;   /* leaf rows */
+    const float* R;                                                                 /* switch rows */
+    int ns; int reserved;
+} mpnn_stats_desc;
+int mpnn_stats_accumulate(const mpnn_stats_desc* descs, int n_leaf, int n_sw, const float* y, int n_cls,
+                          const float* node_p_ev, const double* ops, int n_nodes, int B,
+                          double* work, double* total, const int* count, void* stream);
+
 /* ---- tcgen05 bring-up probe (tests only) -------------------------------- */
 /* D[128][N] = A[128][K] * B[N][K]^T through one CTA of tcgen05.mma; all
  * operands in the interleaved (no-swizzle) core-matrix layout. */

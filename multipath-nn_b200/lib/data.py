@@ -73,6 +73,14 @@ class Dataset:
                      torch.from_numpy(np.ascontiguousarray(self.y_tr, dtype=np.float32)).to(device))
         return self
 
+    def test_to_device(self, device='cuda'):
+        """keep the test set resident in HBM for `test_set(device=True)`, so a statistics pass over it does not upload
+        the data set again"""
+        import torch
+        self._dev_ts = (torch.from_numpy(np.ascontiguousarray(self.x0_ts, dtype=np.float32)).to(device),
+                        torch.from_numpy(np.ascontiguousarray(self.y_ts, dtype=np.float32)).to(device))
+        return self
+
     def augmented_training_batch_gpu(self, n=128, r_shift=4, shard=None):
         """`augmented_training_batch` with the per-example work on the GPU (csrc/augment.cu).  The
         random numbers are drawn on the host in the same order, so a seeded sampler produces the same
@@ -125,8 +133,20 @@ class Dataset:
         for i in range(0, len(x0), n):
             yield x0[i:i + n], y[i:i + n]
 
-    def training_set(self, n=128):
-        yield from self._full_set(self.x0_tr, self.y_tr, n)
+    def training_set(self, n=128, device=False):
+        """the training set in slices of n; device=True: slices (views) of the fp32 copy resident in HBM"""
+        if device:
+            if getattr(self, '_dev', None) is None:
+                self.to_device()
+            yield from self._full_set(*self._dev, n)
+        else:
+            yield from self._full_set(self.x0_tr, self.y_tr, n)
 
-    def test_set(self, n=128):
-        yield from self._full_set(self.x0_ts, self.y_ts, n)
+    def test_set(self, n=128, device=False):
+        """the test set in slices of n; device=True: slices (views) of the fp32 copy resident in HBM"""
+        if device:
+            if getattr(self, '_dev_ts', None) is None:
+                self.test_to_device()
+            yield from self._full_set(*self._dev_ts, n)
+        else:
+            yield from self._full_set(self.x0_ts, self.y_ts, n)

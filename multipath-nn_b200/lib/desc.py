@@ -14,7 +14,8 @@ examples in float64 on the host, divided by the example count -- is unchanged.
 """
 import numpy as np
 
-__all__ = ['state_tensors', 'mean_net_state', 'mean_net_state_compact', 'net_desc', 'render_net_desc']
+__all__ = ['state_tensors', 'mean_net_state', 'mean_net_state_compact', 'mean_net_state_device', 'net_desc',
+           'render_net_desc']
 
 _SPLITS = ('stats_tr', 'stats_ts')
 _RULE = '─' * 59
@@ -100,11 +101,49 @@ def mean_net_state_compact(net, data, hypers, batch=4096):
     return ev.result()
 
 
-def net_desc(net, dataset, hypers={}, state={}, compact=False):
+def mean_net_state_device(net, data, hypers, batch=4096):
+    """`mean_net_state` for every key of `state_tensors(net)` through the device evaluator (lib/dense_stats.py): one
+    graph-replayed dense forward and accumulate launch per chunk, one device-to-host read per data set.  The slices
+    `data` yields (numpy or torch, host or device) are regrouped into chunks of `batch`.  Count-valued statistics have
+    the host path's bits; c_err, p_tr and x_rte differ from it in the last bits (another summation order)."""
+    import torch
+    ev = net.stats_evaluator(batch)
+    ev.reset()
+    xs, ys, n = [], [], 0
+
+    def cat(parts):
+        if len(parts) == 1:
+            return parts[0]
+        if all(isinstance(p, torch.Tensor) for p in parts):
+            return torch.cat(parts)
+        return np.concatenate([p.cpu().numpy() if isinstance(p, torch.Tensor) else np.asarray(p, np.float32)
+                               for p in parts])
+
+    def flush():
+        nonlocal xs, ys, n
+        if n:
+            ev.run_batch(cat(xs), cat(ys), hypers)
+        xs, ys, n = [], [], 0
+    for x0, y in data:
+        if n + len(x0) > batch:
+            flush()
+        xs.append(x0); ys.append(y); n += len(x0)
+    flush()
+    return ev.result()
+
+
+def net_desc(net, dataset, hypers={}, state={}, compact=False, device=False, batch=4096):
     """compact=True (dynamically-routed nets): statistics from the compacted evaluator -- exact for acc, moc,
     p_cor, p_inc and the per-class entries; c_err / p_tr / x_rte, which the reference defines on examples
-    that never reach the node, are omitted (no plotting script reads them)"""
-    if compact and net.dynamic:
+    that never reach the node, are omitted (no plotting script reads them).
+    device=True: the statistics of `state` from the device evaluator, over both splits kept resident in HBM
+    (`Dataset.training_set(device=True)` / `test_set(device=True)`), in chunks of `batch` examples."""
+    if compact and device:
+        raise ValueError('net_desc: compact and device statistics are two different passes; choose one')
+    if device:
+        per_split = [{k: v for k, v in mean_net_state_device(net, batches, hypers, batch).items() if k in state}
+                     for batches in (dataset.training_set(batch, device=True), dataset.test_set(batch, device=True))]
+    elif compact and net.dynamic:
         per_split = [mean_net_state_compact(net, batches, hypers)
                      for batches in (dataset.training_set(), dataset.test_set())]
     else:

@@ -603,6 +603,14 @@ class Engine:
         B = plan.B
         self._upload(plan, self._to_dev(x0, (B,) + tuple(hy.x0_shape), 'x0'),
                      self._to_dev(y, (B,) + tuple(hy.y_shape), 'y'))
+        self._feed_hyp(plan, feed, B)
+
+    def _feed_hyp(self, plan, feed, n):
+        """the per-evaluation scalars (hyp: rates, tau, eps, k_cpt, the Dropout draw) and the per-example k_cpt
+        vectors of the first n <= plan.B examples (rows past n are zero)"""
+        net = self.net
+        hy = net.hypers
+        B = plan.B
         i = self._hyp_i = (self._hyp_i + 1) % len(self._hyp_ring)
         if self._hyp_ev[i] is not None:
             self._hyp_ev[i].synchronize()
@@ -618,9 +626,11 @@ class Engine:
             if hy.dyn_k_cpt:
                 kc = np.asarray(feed[net.k_cpt], dtype=np.float32).reshape(-1)
                 if kc.size == 1:
-                    kc = np.full(B, kc[0], np.float32)      # train-adaptive-nets:102-105
-                if kc.size != B:
-                    raise ValueError('feed k_cpt: %d values for batch %d' % (kc.size, B))
+                    kc = np.full(n, kc[0], np.float32)      # train-adaptive-nets:102-105
+                if kc.size != n:
+                    raise ValueError('feed k_cpt: %d values for batch %d' % (kc.size, n))
+                if n < B:
+                    kc = np.concatenate([kc, np.zeros(B - n, np.float32)])
                 plan.kcpt.copy_(torch.from_numpy(kc), non_blocking=True)
                 plan.kextra.copy_(torch.from_numpy(kc * np.float32(hy.α_cpt)), non_blocking=True)
                 for col in plan.kplanes:          # tcgen05 heads: the feature is one more input column

@@ -127,6 +127,17 @@ class Net:
             cache[batch] = CompactEvaluator(self._get_engine(), batch)
         return cache[batch]
 
+    def stats_evaluator(self, batch=4096):
+        """dense 'ev'-mode statistics on the device (lib/dense_stats.py), cached per batch capacity: `reset()`,
+        `run_batch(x0, y, hypers)` for n <= batch examples, `result()` = `mean_net_state` for every key of
+        `state_tensors(net)`.  Each chunk replays one CUDA graph (weight packing, the dense forward with the current
+        BatchNorm moments, one accumulate launch); nets with Dropout(λ < 1) raise NotImplementedError."""
+        cache = self.__dict__.setdefault('_stats_eval', {})
+        if batch not in cache:
+            from lib.dense_stats import DenseStatsEvaluator
+            cache[batch] = DenseStatsEvaluator(self._get_engine(), batch)
+        return cache[batch]
+
     def predict(self, x0, k_cpt=None, batch=4096):
         """Routed inference: run every example of x0 (numpy or torch, host or device, any n) only along its own
         path in 'ev' mode, in chunks of `batch` on the cached `compact_evaluator(batch)`.  No labels.  Returns
