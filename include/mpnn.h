@@ -50,6 +50,10 @@ int mpnn_pack_input(const float* x0, int B, int H0, int W0, int C0, int step,
  * standard deviation sigma and half-width ceil(2 sigma).  Followed by mpnn_pack_input(out, ..., step = 1). */
 int mpnn_lln(const float* x0, int B, int H0, int W0, int C0, int step, float sigma, float eps,
              float* out, void* stream);
+/* mpnn_lln on the live images of a counted launch: the grid is sized for the capacity B, the images
+ * n < min(*count, B) are written with the same bits and nothing else (count 0: nothing).  count NULL: mpnn_lln. */
+int mpnn_lln_counted(const float* x0, int B, int H0, int W0, int C0, int step, float sigma, float eps,
+                     float* out, const int* count, void* stream);
 
 /* HWIO fp32 conv weights (lib/layer_types.py:158-173) or (n_in,n_chan) FC
  * weights -> packed operand  Wp[tap][Ktot/8][Ntot][8].
@@ -290,6 +294,11 @@ int mpnn_global_maxpool_fwd(const void* x, int C, int B, int H, int W, int G, in
                             void* feat, int* arg, int Balloc, int dtype, void* stream);
 int mpnn_global_maxpool_bwd(const void* dfeat, const int* arg, int Balloc, int C, int B, int H, int W,
                             int G, int P, void* dx, int dtype, void* stream);
+/* mpnn_global_maxpool_fwd on the live images of a counted launch (grid sized for the capacity B, images
+ * n < min(*count, B), rows past them untouched, count 0: nothing); arg may be NULL (no argmax is stored).
+ * count NULL: all B images. */
+int mpnn_global_maxpool_fwd_counted(const void* x, int C, int B, int H, int W, int G, int P,
+                                    void* feat, int* arg, int Balloc, int dtype, const int* count, void* stream);
 
 /* ActivityError (lib/layer_types.py:287-293): cost[b] = alpha * sum_{h,w,c} x^2 (a per-example c_mod);
  * backward: dx (+)= scale * coef[b] * x (scale = 2 alpha / B; coef = the node's p_tr row, NULL: 1;
@@ -411,6 +420,12 @@ int mpnn_route_compact(const float* R, int ldr, int ns, int n, const int* parent
  * (p_cor, p_inc, p_cor_by_cls, p_inc_by_cls of train-nets:121-124 summed over the batch; out is double). */
 int mpnn_leaf_stats(const float* Z, int ldz, int n_cls, const float* y, const int* pos, const int* orig,
                     const int* count, int n, double* out, void* stream);
+/* mpnn_leaf_stats with the correctness target apart from the class bins (superclass classifiers):
+ *   cor = [first argmax of softmax(Z[pos[j]]) == first argmax of t[orig[j]]] over the leaf's n_out <= 32 columns
+ *         (t [B][n_out]; the comparison of mpnn_softmax_ce_fwd, so cor is the dense d_cor),
+ * and the bins over the n_cls one-hot labels y[orig[j]] as above.  mpnn_leaf_stats is t = y, n_out = n_cls. */
+int mpnn_leaf_stats_targets(const float* Z, int ldz, int n_out, const float* t, const float* y, int n_cls,
+                            const int* pos, const int* orig, const int* count, int n, double* out, void* stream);
 /* Routed inference: the results of the examples that exit at one classifier.  Rows pos[j] of the logits Z
  * (row stride ldz) of the parent's compact batch, original ids orig[j], j < *count (count NULL -> j < n;
  * pos / orig NULL -> identity; the grid covers n, so *count <= n):
@@ -420,6 +435,11 @@ int mpnn_leaf_stats(const float* Z, int ldz, int n_cls, const float* y, const in
  * n == 0 is a no-op. */
 int mpnn_leaf_emit(const float* Z, int ldz, int n_cls, const int* pos, const int* orig, const int* count, int n,
                    int leaf, double path_ops, float* prob, int* cls, int* exit_id, double* ops, void* stream);
+/* mpnn_leaf_emit into rows of ldp >= n_out floats: prob[orig[j]][c] = softmax(Z[pos[j]])[c] for c < n_out (the
+ * leaf's outputs: its classes or superclasses), 0 for n_out <= c < ldp.  mpnn_leaf_emit is ldp = n_cls. */
+int mpnn_leaf_emit_strided(const float* Z, int ldz, int n_out, const int* pos, const int* orig, const int* count,
+                           int n, int leaf, double path_ops, float* prob, int ldp, int* cls, int* exit_id,
+                           double* ops, void* stream);
 /* The per-example router feature through the compaction: dst[j] = src[orig[j]] for j < *count (count NULL ->
  * j < n; orig NULL -> identity; dst may be NULL), and, when col != NULL, the same value into the strided column
  * col[j * col_stride] of dtype col_dtype (0 fp32, 1 bf16 rounded to nearest even, like torch's copy_). */

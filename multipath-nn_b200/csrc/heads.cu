@@ -235,12 +235,14 @@ extern "C" int mpnn_softmax_ce_fwd(const float* Z, int ldz, const float* y, int 
 // ------------------------------------------------------ routed inference: results at one classifier
 // The softmax and first argmax of softmax_ce_fwd_kernel (same lane groups, same expressions, so prob is the same
 // bits as the dense path's for the same logits) on rows pos[j] of the parent's compact batch, written at the
-// examples' original ids orig[j].  The live count is read on the device; the grid covers the host bound.
+// examples' original ids orig[j] into rows of ldp >= n floats (columns n .. ldp-1 zero).  The live count is read on
+// the device; the grid covers the host bound.
 template <int LPR>
 __global__ void __launch_bounds__(128)
 leaf_emit_kernel(const float* __restrict__ Z, int ldz, int n, const int* __restrict__ pos,
                  const int* __restrict__ orig, const int* __restrict__ count, int n_max, int leaf, double path_ops,
-                 float* __restrict__ prob, int* __restrict__ cls, int* __restrict__ exit_id, double* __restrict__ ops) {
+                 float* __restrict__ prob, int ldp, int* __restrict__ cls, int* __restrict__ exit_id,
+                 double* __restrict__ ops) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     const int b = t / LPR, j = t % LPR;
     const int nb = count ? min(*count, n_max) : n_max;
@@ -252,7 +254,9 @@ leaf_emit_kernel(const float* __restrict__ Z, int ldz, int n, const int* __restr
     const float mx = grp_max<LPR>(z);
     const float e = on ? expf(z - mx) : 0.f;
     const float p = e * (1.f / grp_sum<LPR>(e));
-    if (on) prob[(size_t)o * n + j] = p;
+    if (on) prob[(size_t)o * ldp + j] = p;
+    if (live)
+        for (int c = n + j; c < ldp; c += LPR) prob[(size_t)o * ldp + c] = 0.f;
     const int am = grp_argmax<LPR>(on ? p : -INFINITY, j);
     if (live && j == 0) {
         cls[o] = am;
@@ -261,19 +265,88 @@ leaf_emit_kernel(const float* __restrict__ Z, int ldz, int n, const int* __restr
     }
 }
 
+extern "C" int mpnn_leaf_emit_strided(const float* Z, int ldz, int n_out, const int* pos, const int* orig,
+                                      const int* count, int n, int leaf, double path_ops, float* prob, int ldp,
+                                      int* cls, int* exit_id, double* ops, void* stream) {
+    MPNN_REQUIRE(n >= 0 && n_out >= 1 && n_out <= CE_NMAX && ldz >= n_out && ldp >= n_out,
+                 "leaf_emit: n=%d n_out=%d ldz=%d ldp=%d", n, n_out, ldz, ldp);
+    if (n == 0) return MPNN_OK;
+    MPNN_REQUIRE(Z && prob && cls && exit_id && ops, "leaf_emit: NULL operand");
+    if (n_out <= 16)
+        leaf_emit_kernel<16><<<ceil_div(n, 128 / 16), 128, 0, (cudaStream_t)stream>>>(
+            Z, ldz, n_out, pos, orig, count, n, leaf, path_ops, prob, ldp, cls, exit_id, ops);
+    else
+        leaf_emit_kernel<32><<<ceil_div(n, 128 / 32), 128, 0, (cudaStream_t)stream>>>(
+            Z, ldz, n_out, pos, orig, count, n, leaf, path_ops, prob, ldp, cls, exit_id, ops);
+    return mpnn_check_launch("leaf_emit");
+}
+
 extern "C" int mpnn_leaf_emit(const float* Z, int ldz, int n_cls, const int* pos, const int* orig, const int* count,
                               int n, int leaf, double path_ops, float* prob, int* cls, int* exit_id, double* ops,
                               void* stream) {
-    MPNN_REQUIRE(n >= 0 && n_cls >= 1 && n_cls <= CE_NMAX && ldz >= n_cls, "leaf_emit: n=%d n_cls=%d ldz=%d", n, n_cls, ldz);
-    if (n == 0) return MPNN_OK;
-    MPNN_REQUIRE(Z && prob && cls && exit_id && ops, "leaf_emit: NULL operand");
-    if (n_cls <= 16)
-        leaf_emit_kernel<16><<<ceil_div(n, 128 / 16), 128, 0, (cudaStream_t)stream>>>(
-            Z, ldz, n_cls, pos, orig, count, n, leaf, path_ops, prob, cls, exit_id, ops);
+    return mpnn_leaf_emit_strided(Z, ldz, n_cls, pos, orig, count, n, leaf, path_ops, prob, n_cls, cls, exit_id, ops,
+                                  stream);
+}
+
+// ------------------------------------------------------ compacted statistics at one classifier
+// Statistics of the examples routed to one classifier (train-nets:117-130 with p_ev one-hot), with the correctness
+// target and the class bins apart:
+//   cor = [first argmax of the softmax of Z[pos[j]] == first argmax of t[orig[j]]] over the leaf's n_out columns --
+//         the comparison of softmax_ce_fwd_kernel (same lane groups and expressions), so it is the dense d_cor bit;
+//   out[0] += #cor, out[1] += #(1 - cor), out[2 + c] += sum cor * y[orig][c], out[2 + n_cls + c] += sum (1 - cor) * y[c]
+// over the n_cls one-hot labels y.  t = y for Softmax + CrossEntropyError leaves, y @ w_cls for superclass leaves.
+// Warp-uniform loop over the examples (the lane groups shuffle); the live count is read on the device.
+template <int LPR>
+__global__ void __launch_bounds__(128)
+leaf_stats_kernel(const float* __restrict__ Z, int ldz, int n, const float* __restrict__ t,
+                  const float* __restrict__ y, int n_cls, const int* __restrict__ pos, const int* __restrict__ orig,
+                  const int* __restrict__ count, int n_fixed, double* __restrict__ out) {
+    const int nb = count ? *count : n_fixed;
+    extern __shared__ float sacc[];                       // [2 + 2 * n_cls]
+    const int na = 2 + 2 * n_cls;
+    for (int i = threadIdx.x; i < na; i += blockDim.x) sacc[i] = 0.f;
+    __syncthreads();
+    const int j = threadIdx.x % LPR;
+    for (int b = (blockIdx.x * blockDim.x + threadIdx.x) / LPR; b - (int)(threadIdx.x & 31) / LPR < nb;
+         b += gridDim.x * blockDim.x / LPR) {
+        const bool live = b < nb;
+        const bool on = live && j < n;
+        const int row = !live ? 0 : pos ? pos[b] : b;
+        const int o = !live ? 0 : orig ? orig[b] : b;
+        const float z = on ? Z[(size_t)row * ldz + j] : -INFINITY;
+        const float tt = on ? t[(size_t)o * n + j] : -INFINITY;
+        const float mx = grp_max<LPR>(z);
+        const float e = on ? expf(z - mx) : 0.f;
+        const float p = e * (1.f / grp_sum<LPR>(e));
+        const int am_p = grp_argmax<LPR>(on ? p : -INFINITY, j);
+        const int am_t = grp_argmax<LPR>(tt, j);
+        if (live) {
+            const bool cor = am_p == am_t;
+            if (j == 0) atomicAdd(sacc + (cor ? 0 : 1), 1.f);
+            const float* yy = y + (size_t)o * n_cls;
+            for (int c = j; c < n_cls; c += LPR)
+                if (yy[c] != 0.f) atomicAdd(sacc + 2 + (cor ? 0 : n_cls) + c, yy[c]);
+        }
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < na; i += blockDim.x)
+        if (sacc[i] != 0.f) atomicAdd(out + i, (double)sacc[i]);
+}
+
+extern "C" int mpnn_leaf_stats_targets(const float* Z, int ldz, int n_out, const float* t, const float* y, int n_cls,
+                                       const int* pos, const int* orig, const int* count, int n, double* out,
+                                       void* stream) {
+    MPNN_REQUIRE(Z && t && y && out && n_out >= 1 && n_out <= CE_NMAX && ldz >= n_out && n_cls >= 1 && n_cls <= 1024
+                 && n >= 0, "leaf_stats: n_out=%d ldz=%d n_cls=%d n=%d", n_out, ldz, n_cls, n);
+    const int lpr = n_out <= 16 ? 16 : 32;
+    int grid = ceil_div(n > 0 ? n : 1, 128 / lpr);
+    if (grid > 148) grid = 148;
+    const size_t smem = (2 + 2 * n_cls) * sizeof(float);
+    if (lpr == 16)
+        leaf_stats_kernel<16><<<grid, 128, smem, (cudaStream_t)stream>>>(Z, ldz, n_out, t, y, n_cls, pos, orig, count, n, out);
     else
-        leaf_emit_kernel<32><<<ceil_div(n, 128 / 32), 128, 0, (cudaStream_t)stream>>>(
-            Z, ldz, n_cls, pos, orig, count, n, leaf, path_ops, prob, cls, exit_id, ops);
-    return mpnn_check_launch("leaf_emit");
+        leaf_stats_kernel<32><<<grid, 128, smem, (cudaStream_t)stream>>>(Z, ldz, n_out, t, y, n_cls, pos, orig, count, n, out);
+    return mpnn_check_launch("leaf_stats");
 }
 
 // dZ in fp32 [B][n] and/or as two bf16 planes [2][Balloc][8] (columns >= n zero) for the

@@ -92,12 +92,16 @@ extern "C" int mpnn_pack_input_counted(const float* x0, int B, int H0, int W0, i
 // an image of ones (so borders are normalised by the weight that falls inside); out = x / (lum / density + eps).
 // x0 is the full-resolution NHWC image, the scale is its `step`-strided subsample (ToPyramid, :118-125);
 // out is NHWC fp32 at the scale's size.  One thread per output pixel.
+// CNT: the first min(*count, B) images only (B: the capacity the grid was sized for); a count of 0 writes nothing.
 // --------------------------------------------------------------------------- //
+template <bool CNT = false>
 __global__ void __launch_bounds__(256)
 lln_kernel(const float* __restrict__ x0, int B, int H0, int W0, int step, float sigma, float eps, int s,
-           float* __restrict__ out) {
+           float* __restrict__ out, const int* __restrict__ count) {
     const int H = H0 / step, W = W0 / step;
+    if (CNT) B = min(max(*count, 0), B);
     const int total = B * H * W;
+    if (CNT && (int)(blockIdx.x * blockDim.x) >= total) return;
     const float inv2s2 = 1.f / (2.f * sigma * sigma), norm = 1.f / (2.f * 3.14159265358979323846f * sigma * sigma);
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
         const int w = i % W, h = (i / W) % H, n = i / (W * H);
@@ -121,16 +125,26 @@ lln_kernel(const float* __restrict__ x0, int B, int H0, int W0, int step, float 
     }
 }
 
-extern "C" int mpnn_lln(const float* x0, int B, int H0, int W0, int C0, int step, float sigma, float eps,
-                        float* out, void* stream) {
+extern "C" int mpnn_lln_counted(const float* x0, int B, int H0, int W0, int C0, int step, float sigma, float eps,
+                                float* out, const int* count, void* stream) {
     MPNN_REQUIRE(x0 && out && C0 == 3, "lln: the luminance weights are defined for 3 channels (C0=%d)", C0);
     MPNN_REQUIRE(step >= 1 && H0 % step == 0 && W0 % step == 0 && sigma > 0.f, "lln: step=%d sigma=%g", step, (double)sigma);
+    MPNN_REQUIRE(B >= 0, "lln: B=%d", B);
+    if (count && B == 0) return MPNN_OK;
     const int s = (int)ceilf(2.f * sigma);
     const long long total = (long long)B * (H0 / step) * (W0 / step);
     int grid = (int)((total + 255) / 256);
     if (grid > 148 * 16) grid = 148 * 16;
-    lln_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(x0, B, H0, W0, step, sigma, eps, s, out);
+    if (count)
+        lln_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>(x0, B, H0, W0, step, sigma, eps, s, out, count);
+    else
+        lln_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(x0, B, H0, W0, step, sigma, eps, s, out, nullptr);
     return mpnn_check_launch("lln");
+}
+
+extern "C" int mpnn_lln(const float* x0, int B, int H0, int W0, int C0, int step, float sigma, float eps,
+                        float* out, void* stream) {
+    return mpnn_lln_counted(x0, B, H0, W0, C0, step, sigma, eps, out, nullptr, stream);
 }
 
 // --------------------------------------------------------------------------- //

@@ -101,12 +101,15 @@ extern "C" int mpnn_maxpool2_bwd(const void* x, const void* dout, const void* df
 // GlobalMaxPool: one warp per (image, 8-channel plane); lanes stride over the pixels in row-major order and keep
 // (value, pixel) of their first maximum per channel; the warp reduction prefers the smaller pixel on ties.
 // feat [C/8][Balloc][8] (the layout of a flattened 1x1 image), arg [C/8][Balloc][8] int32 = h * W + w.
-template <typename T>
+// CNT: count and arg may be NULL; a count limits the launch to the first min(*count, g.B) images (g.B: the capacity
+// the grid was sized for).
+template <typename T, bool CNT = false>
 __global__ void __launch_bounds__(256)
 global_maxpool_fwd_kernel(const T* __restrict__ x, int C, Geom g, T* __restrict__ feat, int* __restrict__ arg,
-                          int Balloc) {
+                          int Balloc, const int* __restrict__ count) {
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     const int KG = C / 8;
+    if (CNT && count) g.B = min(max(*count, 0), g.B);
     if (warp >= g.B * KG) return;
     const int n = warp / KG, kg = warp % KG;
     float bv[8];
@@ -131,9 +134,11 @@ global_maxpool_fwd_kernel(const T* __restrict__ x, int C, Geom g, T* __restrict_
     }
     if (lane == 0) {
         Row8<T>::store(plane_row(feat, kg, Balloc, n), bv);
-        int* a = arg + ((size_t)kg * Balloc + n) * 8;
+        if (!CNT || arg) {
+            int* a = arg + ((size_t)kg * Balloc + n) * 8;
 #pragma unroll
-        for (int j = 0; j < 8; ++j) a[j] = bi[j];
+            for (int j = 0; j < 8; ++j) a[j] = bi[j];
+        }
     }
 }
 
@@ -143,8 +148,24 @@ extern "C" int mpnn_global_maxpool_fwd(const void* x, int C, int B, int H, int W
     Geom g = make_geom(B, H, W, G, P);
     const long long warps = (long long)B * (C / 8);
     MPNN_DISPATCH_DTYPE(dtype, (global_maxpool_fwd_kernel<T><<<(int)((warps * 32 + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
-        (const T*)x, C, g, (T*)feat, arg, Balloc)));
+        (const T*)x, C, g, (T*)feat, arg, Balloc, nullptr)));
     return mpnn_check_launch("global_maxpool_fwd");
+}
+
+// the forward on the live images of a counted launch (grid sized for the capacity B, live images min(*count, B));
+// arg may be NULL (the 'ev' pass needs no argmax).  count NULL: the uncounted launch at B.
+extern "C" int mpnn_global_maxpool_fwd_counted(const void* x, int C, int B, int H, int W, int G, int P,
+                                               void* feat, int* arg, int Balloc, int dtype, const int* count,
+                                               void* stream) {
+    MPNN_REQUIRE(x && feat && C % 8 == 0 && B >= 0 && Balloc >= B,
+                 "global_maxpool_fwd_counted: C=%d B=%d Balloc=%d", C, B, Balloc);
+    if (arg && !count) return mpnn_global_maxpool_fwd(x, C, B, H, W, G, P, feat, arg, Balloc, dtype, stream);
+    if (B == 0) return MPNN_OK;
+    Geom g = make_geom(B, H, W, G, P);
+    const long long warps = (long long)B * (C / 8);
+    MPNN_DISPATCH_DTYPE(dtype, (global_maxpool_fwd_kernel<T, true><<<(int)((warps * 32 + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+        (const T*)x, C, g, (T*)feat, arg, Balloc, count)));
+    return mpnn_check_launch("global_maxpool_fwd_counted");
 }
 
 // dx[n][h][w][c] = dfeat[n][c] where (h, w) is the recorded maximum of channel c, zero elsewhere

@@ -696,44 +696,9 @@ extern "C" int mpnn_route_compact(const float* R, int ldr, int ns, int n, const 
     return mpnn_route_compact_counted(R, ldr, ns, n, parent_orig, cap, dec, pos, orig, count, nullptr, stream);
 }
 
-// Leaf statistics of the examples routed to one classifier (train-nets:117-130 with p_ev one-hot):
-//   out[0] += #correct, out[1] += #incorrect, out[2 + c] += sum cor * y[c], out[2 + n_cls + c] += sum (1 - cor) * y[c]
-// cor = [first argmax Z == first argmax y] (layer_types.py:259-260,271-272; softmax + eps-smoothing are monotone).
-__global__ void __launch_bounds__(256)
-leaf_stats_kernel(const float* __restrict__ Z, int ldz, int n_cls, const float* __restrict__ y,
-                  const int* __restrict__ pos, const int* __restrict__ orig, const int* __restrict__ count, int n_fixed,
-                  double* __restrict__ out) {
-    const int n = count ? *count : n_fixed;
-    extern __shared__ float sacc[];                       // [2 + 2 * n_cls]
-    const int na = 2 + 2 * n_cls;
-    for (int i = threadIdx.x; i < na; i += blockDim.x) sacc[i] = 0.f;
-    __syncthreads();
-    for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < n; j += gridDim.x * blockDim.x) {
-        const int row = pos ? pos[j] : j, o = orig ? orig[j] : j;
-        const float* z = Z + (size_t)row * ldz;
-        const float* yy = y + (size_t)o * n_cls;
-        int az = 0, ay = 0;
-        float bz = z[0], by = yy[0];
-        for (int c = 1; c < n_cls; ++c) {
-            if (z[c] > bz) { bz = z[c]; az = c; }
-            if (yy[c] > by) { by = yy[c]; ay = c; }
-        }
-        const bool cor = az == ay;
-        atomicAdd(sacc + (cor ? 0 : 1), 1.f);
-        for (int c = 0; c < n_cls; ++c)
-            if (yy[c] != 0.f) atomicAdd(sacc + 2 + (cor ? 0 : n_cls) + c, yy[c]);
-    }
-    __syncthreads();
-    for (int i = threadIdx.x; i < na; i += blockDim.x)
-        if (sacc[i] != 0.f) atomicAdd(out + i, (double)sacc[i]);
-}
-
+// Leaf statistics of the examples routed to one Softmax + CrossEntropyError classifier: mpnn_leaf_stats_targets
+// (heads.cu) with the labels as the correctness target.
 extern "C" int mpnn_leaf_stats(const float* Z, int ldz, int n_cls, const float* y, const int* pos, const int* orig,
                                const int* count, int n, double* out, void* stream) {
-    MPNN_REQUIRE(Z && y && out && n_cls >= 1 && n_cls <= 1024 && ldz >= n_cls && n >= 0, "leaf_stats: args");
-    int grid = ceil_div(n > 0 ? n : 1, 256);
-    if (grid > 148) grid = 148;
-    leaf_stats_kernel<<<grid, 256, (2 + 2 * n_cls) * sizeof(float), (cudaStream_t)stream>>>(
-        Z, ldz, n_cls, y, pos, orig, count, n, out);
-    return mpnn_check_launch("leaf_stats");
+    return mpnn_leaf_stats_targets(Z, ldz, n_cls, y, y, n_cls, pos, orig, count, n, out, stream);
 }

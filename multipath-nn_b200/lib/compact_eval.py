@@ -8,8 +8,15 @@ its running moments, so examples are independent and an example only needs the n
 after every switch the batch is compacted (mpnn_route_compact: first-max argmax, ballot + prefix scan into
 per-sink index lists), the activation pyramids of the examples that continue are gathered into the child's
 input buffers (mpnn_gather_images) and the child runs on the smaller batch; classifiers are scored only on
-the examples that exit at them (mpnn_leaf_stats).  All sums stay on the device and are read back once per
-data set.
+the examples that exit at them (mpnn_leaf_stats_targets: correct against the labels, or against y @ w_cls at a
+SuperclassCrossEntropyError classifier, binned by the labels).  All sums stay on the device and are read back once
+per data set.
+
+The root is a ToPyramid (each scale packed from the image, or from mpnn_lln_counted's output behind a
+MultiscaleLLN) or a Conv chain on the image (packed into the dense plan's image slot; the root then runs as an
+ordinary node).  Conv blocks run like one-scale stages; ActivityError costs and
+Dropout(λ = 1) need no launch in 'ev' mode, and a GlobalMaxPool classifier reads the features of
+mpnn_global_maxpool_fwd_counted.  Refused: bf16x3, MaxPool blocks, SquaredError classifiers, Dropout(λ < 1).
 
 Exact for every p_ev-weighted statistic -- acc, moc, and per leaf p_cor, p_inc, p_cor_by_cls, p_inc_by_cls
 (what make-acc-eff-plots / make-nlds / make-routing-hists read).  The three entries of `state_tensors` that
@@ -17,7 +24,8 @@ are NOT p_ev-weighted (per-leaf c_err and p_tr, per-switch x_rte; train-nets:125
 a compacted pass never evaluates: they are absent from its result (use the dense `Engine.eval_stats` for them).
 
 The same walk serves routed inference (`predict`, behind `Net.predict`): at a classifier it writes each
-example's softmax, predicted class, exit leaf and path cost (mpnn_leaf_emit) instead of adding statistics.
+example's softmax, predicted class, exit leaf and path cost (mpnn_leaf_emit_strided: rows of max(n_cls, widest
+leaf) columns, a superclass classifier's superclasses zero-filled to that width) instead of adding statistics.
 Nets with a per-example k_cpt carry the router feature alpha_cpt * k_cpt through the compaction by original
 example id (mpnn_gather_feature), so one batch may mix cost budgets.
 
@@ -60,8 +68,9 @@ class _LeafStats:
     def __call__(self, nd, n, orig, pos, sink_cnt, S):
         ev = self.ev
         r = ev.plan.reg[nd.idx]
-        ev.L.leaf_stats(_vp(r.Zbuf), r.ldz, ev.n_cls, _vp(ev.plan.y), _vp(pos), _vp(orig), _vp(sink_cnt), n,
-                        _vp(ev.acc[nd.err]), S)
+        # correct against r.y (the labels, or a superclass leaf's targets y @ w_cls), binned by the labels
+        ev.L.leaf_stats_targets(_vp(r.Zbuf), r.ldz, r.n, _vp(r.y), _vp(ev.plan.y), ev.n_cls, _vp(pos), _vp(orig),
+                                _vp(sink_cnt), n, _vp(ev.acc[nd.err]), S)
 
 
 class _LeafEmit:
@@ -78,27 +87,30 @@ class _LeafEmit:
         ev = self.ev
         r = ev.plan.reg[nd.idx]
         no = ev.leaf_no[nd.idx]
-        ev.L.leaf_emit(_vp(r.Zbuf), r.ldz, ev.n_cls, _vp(pos), _vp(orig), _vp(sink_cnt), n, no, ev.path_ops[no],
-                       *self.out, S)
+        prob, cls, exit, ops = self.out
+        ev.L.leaf_emit_strided(_vp(r.Zbuf), r.ldz, r.n, _vp(pos), _vp(orig), _vp(sink_cnt), n, no, ev.path_ops[no],
+                               prob, ev.n_prob, cls, exit, ops, S)
 
 
 class CompactEvaluator:
     def __init__(self, eng, batch=4096):
         if eng.split == 2:
             raise NotImplementedError('compacted evaluation runs in fp32, bf16 or bf16x6 precision (not bf16x3)')
-        if any(getattr(nd, 'maxpool', False) or getattr(nd, 'gmp', False) for nd in eng.nodes):
-            raise NotImplementedError('compacted evaluation does not cover MaxPool / GlobalMaxPool blocks')
-        if any(nd.loss != 'ce' for nd in eng.regs):
-            raise NotImplementedError('compacted evaluation scores Softmax + CrossEntropyError classifiers only')
+        if any(getattr(nd, 'maxpool', False) for nd in eng.nodes):
+            raise NotImplementedError('compacted evaluation does not cover MaxPool blocks')
+        if any(nd.loss not in ('ce', 'sce') for nd in eng.regs):
+            # a SquaredError leaf has no softmax: its prob would mean something else
+            raise NotImplementedError('compacted evaluation scores Softmax + CrossEntropyError / '
+                                      'SuperclassCrossEntropyError classifiers only')
         if any(getattr(nd, 'keep', 1.0) != 1.0 for nd in eng.nodes):
             # the reference applies Dropout in every mode: an 'ev' pass through it is random, and this walk has no mask
             raise NotImplementedError('compacted evaluation does not cover Dropout(λ < 1) blocks')
-        root = eng.nodes[0]
-        if root.kind != 'pyr' or getattr(root, 'lln', None) is not None:
-            raise NotImplementedError('compacted evaluation starts from a ToPyramid root without MultiscaleLLN')
         self.eng, self.L, self.B = eng, eng.L, int(batch)
         self.plan = plan = eng._plan(self.B, False, False)      # buffers, packed operands, BN constants
         self.n_cls = eng.net.hypers.y_shape[0]
+        # columns of predict's prob: a superclass leaf writes its n_out softmax outputs, zero-filled to this width
+        self.n_prob = max([self.n_cls] + [plan.reg[nd.idx].n for nd in eng.regs])
+        self.sce = [plan.reg[nd.idx] for nd in eng.regs if nd.loss == 'sce']
         B = self.B
         dev = eng.dev
         self.dyn_k = eng.dynamic and bool(eng.net.hypers.dyn_k_cpt)
@@ -130,7 +142,7 @@ class CompactEvaluator:
         # (hi | mid | lo) split planes, the only form of the input its convs read)
         self.cin = {}
         for nd in eng.nodes:
-            if nd.kind == 'rcm' and len(eng.nodes[nd.parent].kids) > 1:
+            if nd.kind == 'rcm' and nd.parent is not None and len(eng.nodes[nd.parent].kids) > 1:
                 st = plan.node[nd.idx]
                 self.cin[nd.idx] = [plan.zeros((3 * s.C // 8, s.geo.P, 8), torch.bfloat16) if eng.split
                                     else plan.planes(s.C, s.geo) for s in st.pin]
@@ -201,21 +213,33 @@ class CompactEvaluator:
     def _walk(self, live, leaf, split):
         """run the loaded chunk down the tree on the current stream.  live: its (launch batch, device count), (n, None)
         or (B, count of the chunk); leaf: the leaf action; split: the switch step"""
-        eng, plan = self.eng, self.plan
+        eng, plan, L = self.eng, self.plan, self.L
         H0, W0, C0 = eng.net.hypers.x0_shape
         stream = torch.cuda.current_stream(eng.dev)
         S = ctypes.c_void_p(stream.cuda_stream)
-        for i, slot in enumerate(plan.node[0].out):
-            g = slot.geo
-            self.L.pack_input_counted(_vp(plan.x0), live[0], H0, W0, C0, 2 ** i, _vp(slot.t),
-                                      min(slot.C, (C0 + 7) // 8 * 8), g.G, g.P, eng.dtype, _vp(live[1]), S)
-            if eng.split:
-                self.L.split_planes3_counted(_vp(slot.t), slot.C, live[0], g.H, g.W, g.G, g.P, _vp(slot.split),
-                                             _vp(live[1]), S)
         root = eng.nodes[0]
-        leaf.visit(root, live[0])
+        pyr = root.kind == 'pyr'
+        # the pyramid's scales, or the image a Conv chain at the root reads (the dense plan's _image_slot)
+        lln = getattr(root, 'lln', None)
+        for i, slot in enumerate(plan.node[0].out if pyr else plan._image_slot().out):
+            g = slot.geo
+            src, H, W, step = plan.x0, H0, W0, 2 ** i
+            if lln is not None:                     # MultiscaleLLN: normalise the scale, then pack the fp32 result
+                L.lln_counted(_vp(plan.x0), live[0], H0, W0, C0, step, float(lln.hypers.σ), float(lln.hypers.ϵ),
+                              _vp(slot.lln), _vp(live[1]), S)
+                src, H, W, step = slot.lln, g.H, g.W, 1
+            L.pack_input_counted(_vp(src), live[0], H, W, C0, step, _vp(slot.t), min(slot.C, (C0 + 7) // 8 * 8),
+                                 g.G, g.P, eng.dtype, _vp(live[1]), S)
+            if eng.split:
+                L.split_planes3_counted(_vp(slot.t), slot.C, live[0], g.H, g.W, g.G, g.P, _vp(slot.split),
+                                        _vp(live[1]), S)
         if live[0] == 0:                            # run_batch of no examples
+            leaf.visit(root, 0)
             return
+        if not pyr:                                 # a Conv chain at the root: an ordinary node
+            self._node(root, live, live, None, None, live[1], stream, leaf, split)
+            return
+        leaf.visit(root, live[0])
         for k in root.kids:
             self._node(eng.nodes[k], live, live, None, None, live[1], stream, leaf, split)
 
@@ -234,6 +258,8 @@ class CompactEvaluator:
                 self._prepare()
             y = eng._to_dev(y, (n,) + tuple(eng.net.hypers.y_shape), 'y')
             plan.y[:n].copy_(y, non_blocking=True)
+            for r in self.sce if n else ():         # a superclass leaf is scored against y @ w_cls of these labels
+                self.L.superclass_targets(_vp(plan.y), _vp(r.w_cls), n, self.n_cls, r.n, _vp(r.y), self._S())
             self.n_seen += n
             self._load(x0, n, kf)
             self._walk((n, None), _LeafStats(self), self._host_split)
@@ -250,7 +276,7 @@ class CompactEvaluator:
         eng = self.eng
         n = self._check_x0(x0)
         kf = self._k_feature(k_cpt, n)
-        nc = self.n_cls
+        nc = self.n_prob
         # one byte buffer holds the four outputs, so that one device-to-host copy returns them
         o_prob = 8 * n
         o_cls = o_prob + 4 * n * nc
@@ -300,7 +326,7 @@ class CompactEvaluator:
                 r = plan.reg[nd.idx]
                 # logits of the parent's compact batch (rows of the examples that exit here are read through pos)
                 L.fc_fwd_counted(_vp(pst.feat), pst.F, plan.Balloc, par[0], eng.tptr(r.fc.params.w),
-                                 eng.tptr(r.fc.params.b), None, self.n_cls, _vp(r.Zbuf), dt, _vp(par[1]), S)
+                                 eng.tptr(r.fc.params.b), None, r.n, _vp(r.Zbuf), dt, _vp(par[1]), S)
             leaf(nd, n, orig, pos, sink_cnt, S)
             return
         st = plan.node[nd.idx]
@@ -338,6 +364,10 @@ class CompactEvaluator:
                         q = sc.geo_p
                         L.split_planes3_counted(_vp(sc.pooled), sc.N, n, q.H, q.W, q.G, q.P, _vp(sc.pooled_split),
                                                 _vp(cnt), S)
+            # (Dropout(λ = 1) is the identity, and an ActivityError cost enters the training objective only)
+            if getattr(nd, 'gmp', False):           # the GlobalMaxPool classifier's features, without the argmax
+                L.global_maxpool_fwd_counted(_vp(sc.act), sc.N, n, g.H, g.W, g.G, g.P, _vp(st.feat), None, plan.Balloc,
+                                             dt, _vp(cnt), S)
         if not nd.kids:
             return
         if plan.umma_heads and nd.idx in plan.heads:
@@ -401,7 +431,7 @@ class RoutedPredictor:
         self.ev, eng = ev, ev.eng
         self.B = ev.B
         dev = eng.dev
-        B, nc = ev.B, ev.n_cls
+        B, nc = ev.B, ev.n_prob
         self.n_dev = torch.zeros(1, dtype=torch.int32, device=dev)
         self.cls = torch.zeros(B, dtype=torch.int32, device=dev)
         self.prob = torch.zeros((B, nc), dtype=torch.float32, device=dev)

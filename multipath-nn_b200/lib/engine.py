@@ -1125,7 +1125,7 @@ class _Plan:
                     st.out.append(_slot(t, cpad, C0, geo))
                     if getattr(nd, 'lln', None) is not None:
                         # MultiscaleLLN behind ToPyramid: normalise the scale in fp32 NHWC, then pack that
-                        tmp = self.f32(B, geo.H, geo.W, C0)
+                        tmp = st.out[-1].lln = self.f32(B, geo.H, geo.W, C0)
 
                         def lln(i=i, tmp=tmp, hy=nd.lln.hypers):
                             L.lln(_vp(self.x0), B, H0, W0, C0, 2 ** i, float(hy.σ), float(hy.ϵ), _vp(tmp), S())
@@ -1169,7 +1169,7 @@ class _Plan:
                 if nd.loss == 'sce':
                     # SuperclassCrossEntropyError (lib/layer_types.py:274-285): the targets are y @ w_cls, refreshed
                     # with the labels at the head of every step
-                    w_cls = torch.tensor(nd.w_cls, dtype=torch.float32, device=eng.dev)
+                    w_cls = r.w_cls = torch.tensor(nd.w_cls, dtype=torch.float32, device=eng.dev)
                     r.y = self.f32(B, n_out)
                     self.keep.append(w_cls)
                     self.pack_ops.append(lambda r=r, w_cls=w_cls, n_out=n_out: L.superclass_targets(

@@ -143,9 +143,12 @@ class Net:
         path in 'ev' mode, in chunks of `batch` on the cached `compact_evaluator(batch)`.  No labels.  Returns
         Ns of numpy arrays:
             cls  int32 (n,)            predicted class (first argmax of prob)
-            prob float32 (n, n_cls)    softmax of the classifier the example exits at
+            prob float32 (n, n_prob)   softmax of the classifier the example exits at
             exit int32 (n,)            that classifier's index in list(net.leaves)
             ops  float64 (n,)          ops of the nodes and routers on the example's path (the dense `moc`)
+        n_prob = max(n_cls, widest classifier), which is n_cls unless a SuperclassCrossEntropyError classifier has
+        more superclasses than the net has classes.  For an example that exits at a superclass classifier, prob is
+        the softmax over that classifier's superclasses (zero-filled to n_prob columns) and cls is the superclass.
         k_cpt: required for nets with a per-example k_cpt (dyn_k_cpt) -- a scalar, one value or n values --
         and None for the others.  The weights are packed and the BatchNorm moments finalised on every call, so a
         call between training steps sees the current parameters."""
@@ -154,7 +157,7 @@ class Net:
     def predictor(self, batch=4096):
         """Routed inference replayed as one CUDA graph (lib/compact_eval.py, RoutedPredictor), cached per capacity.
         `p = net.predictor(batch)`; `p(x0, k_cpt=None)` takes n <= batch examples (host or device) and returns the
-        Ns(cls, prob, exit, ops) of `predict` as DEVICE torch tensors -- views [:n] of the predictor's output buffers,
+        Ns(cls, prob, exit, ops) of `predict` (the same widths and superclass meaning) as DEVICE torch tensors -- views [:n] of the predictor's output buffers,
         overwritten by the next call.  With device inputs a call does not synchronise the host.  The checks, the
         refused compositions and the use of the current parameters are those of `predict`; n > batch raises
         ValueError.  The graph is captured on the first call with n > 0."""
