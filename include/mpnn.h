@@ -375,10 +375,9 @@ int mpnn_route_fwd(const int* parent, const int* sink_idx, const int* n_sinks,
                    const float* floor_, const int* sw, int n_nodes,
                    const float* const* R, const float* hyp, int B,
                    float* p_tr, float* p_ev, int* dec, void* stream);
-/* Actor (critic=0): gradient of c_tot wrt router logits and per-leaf CE
- * coefficients (net_types.py:167-177):
- *   coef[slot][b] = p_tr[leaf][b]
+/* Actor (critic=0): gradient of c_tot wrt router logits (net_types.py:167-177):
  *   dR[slot][b][i] = d/dR of mean_b( sum_l p_tr(c_err + k_cpt ops) + sg(p_tr) k_dec |R|^2 )
+ * (the per-leaf loss coefficients are the p_tr rows of mpnn_route_fwd; this call writes none)
  * Critic (critic=1; net_types.py:201-243,275-280): also computes c_ev/c_opt
  * bottom-up and dR = p_tr/B * 2 k_cre (R_i + target_i).
  *   c_err: table of per-leaf [B] arrays; d_cor likewise (use_cls_err).

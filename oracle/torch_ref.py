@@ -91,7 +91,7 @@ def tf_resize_legacy(x, h, w):
 def first_argmax(x, dim):
     """tf.argmax: index of the FIRST maximal element."""
     m = x.max(dim, keepdim=True).values
-    idx = torch.arange(x.shape[dim]).reshape(
+    idx = torch.arange(x.shape[dim], device=x.device).reshape(
         [-1 if d == dim % x.dim() else 1 for d in range(x.dim())])
     big = x.shape[dim]
     return torch.where(x == m, idx, big).min(dim).values

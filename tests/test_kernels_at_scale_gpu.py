@@ -7,13 +7,16 @@ At these sizes the grid-stride loops run their second and later passes, the BN s
 of times longer than in test_kernels_gpu.py.  Tolerances are derived in each docstring; u = 2^-24 is the fp32
 unit roundoff.  Run with -s to see the measured errors."""
 import ctypes
+import functools
 import math
 
+import numpy as np
 import pytest
 import torch
 import torch.nn.functional as Fn
 
-from util import Geo, dropout_mask_t, from_feat_t, from_planes_t, to_feat_t, to_planes_t
+from util import (Geo, dropout_mask_t, from_feat_t, from_planes_t, pad_tree, random_tree, route_ref, to_feat_t,
+                  to_planes_t, tree_tables)
 
 pytestmark = pytest.mark.gpu
 
@@ -785,3 +788,554 @@ def test_bn_statistics_with_large_channel_means_bn_fwd_small(dt, B, H, C):
                      vp(act), None, 0, dt, None)
     torch.cuda.synchronize()
     _check_stats('bn_fwd_small %s B=%d H=%d' % ('fp32' if dt == F32 else 'bf16', B, H), mr[0], mr[1], lin.double(), plan)
+
+
+# --------------------------------------------------------------------------- #
+# the routing walks: mpnn_route_fwd / mpnn_route_bwd
+# --------------------------------------------------------------------------- #
+RT_STAGED_MAX = 32      # csrc/route.cu: trees up to this size run the staged walk, larger ones the global one
+
+
+@functools.lru_cache(None)
+def _plan_of(name):
+    """(routing tables, n_theta, segment tables) of a dry-run plan of a full-size net (lib/engine.py)"""
+    import arch_and_hypers as ah
+    from lib import engine as E
+    eng = E.Engine(getattr(ah, name)(k_cpt=4e-9)((32, 32, 3), (10,)), precision='fp32', impl=0, dry_run=True)
+    plan = eng._plan(128, True, True)
+    seg = {k: getattr(eng, k).clone() for k in ('seg_start', 'seg_node', 'seg_mult', 'seg_l2')}
+    return tree_tables(plan), eng.n_theta, len(eng.nodes), seg
+
+
+def tree_of(spec):
+    if isinstance(spec, str):
+        return _plan_of(spec)[0]
+    n, ns = spec
+    return random_tree(np.random.default_rng(31 * n + ns), n, ns)
+
+
+def _ptrs(ts):
+    return torch.tensor([x.data_ptr() for x in ts] or [0], dtype=torch.int64, device='cuda')
+
+
+def route_launch(t, R, tau, eps, B, c_err=None, d_cor=None, k_cpt=None, critic=0, k_dec=0.0, k_cre=0.0,
+                 optimistic=0, use_cls_err=0, kc=4e-9, bwd=True):
+    """mpnn_route_fwd (+ mpnn_route_bwd) on tables t (NumPy) and device logits R[slot]; outputs start as NaN / -1
+    so that an unwritten element cannot pass"""
+    T = {k: torch.from_numpy(np.ascontiguousarray(v)).cuda() for k, v in t.items()}
+    n = len(t['parent'])
+    hyp = torch.zeros(8, device='cuda')
+    hyp[2], hyp[3], hyp[4] = tau, eps, kc
+    Rt = _ptrs(R)
+    o = dict(p_tr=torch.full((n, B), math.nan, device='cuda'), p_ev=torch.full((n, B), math.nan, device='cuda'),
+             dec=torch.full((max(len(R), 1), B), -1, dtype=torch.int32, device='cuda'))
+    L().route_fwd(vp(T['parent']), vp(T['sink_idx']), vp(T['n_sinks']), vp(T['floor']), vp(T['sw']), n, vp(Rt),
+                  vp(hyp), B, vp(o['p_tr']), vp(o['p_ev']), vp(o['dec']), None)
+    if bwd:
+        o['dR'] = [torch.full_like(r, math.nan) for r in R]
+        o['c_data'] = torch.full((B,), math.nan, device='cuda')
+        scratch = torch.zeros(3 * n * B, device='cuda')
+        ce_t, dc_t, dR_t = _ptrs(c_err), _ptrs(d_cor), _ptrs(o['dR'])
+        L().route_bwd(vp(T['parent']), vp(T['sink_idx']), vp(T['n_sinks']), vp(T['child']), vp(T['floor']),
+                      vp(T['sw']), vp(T['ops']), vp(T['err']), n, vp(Rt), vp(hyp), B, vp(o['p_tr']), vp(o['p_ev']),
+                      vp(ce_t), vp(dc_t), vp(k_cpt), critic, k_dec, k_cre, optimistic, use_cls_err, vp(dR_t),
+                      vp(scratch), vp(o['c_data']), None)
+    torch.cuda.synchronize()
+    return o
+
+
+LOGITS = {'normal': 0.6, 'integer': 1.0, 'sharp': 0.1}       # logits kind -> tau
+
+
+def route_inputs(t, B, kind, seed):
+    g = gen(seed)
+    n_err = int((t['err'] >= 0).sum())
+    R = []
+    for i in range(len(t['parent'])):
+        ns = int(t['n_sinks'][i])
+        if ns < 2:
+            continue
+        if kind == 'normal':
+            r = 2 * torch.randn((B, ns), generator=g, device='cuda')
+        elif kind == 'integer':                  # ties: the first maximum decides dec and p_ev
+            r = torch.randint(-2, 3, (B, ns), generator=g, device='cuda').float()
+        else:                                    # about +-50 at tau = 0.1 (the tau_cr schedule): exponents to 1000
+            r = (25 * torch.randn((B, ns), generator=g, device='cuda')).clamp(-50, 50)
+        R.append(r)
+    ce = [3 * torch.rand(B, generator=g, device='cuda') for _ in range(n_err)]
+    dc = [(torch.rand(B, generator=g, device='cuda') < 0.6).float() for _ in range(n_err)]
+    kv = 1e-8 * torch.rand(B, generator=g, device='cuda')
+    return R, ce, dc, kv
+
+
+MODES = {'actor k_dec': dict(critic=0, k_dec=0.01), 'actor k_cpt vector': dict(critic=0, k_dec=0.01, vec=True),
+         'critic': dict(critic=1, k_cre=1e-3), 'critic optimistic': dict(critic=1, k_cre=1e-3, optimistic=1),
+         'critic use_cls_err': dict(critic=1, k_cre=1e-3, use_cls_err=1, vec=True)}
+
+
+def p_tr_bound(t, ref, tau, eps, X):
+    """First-order bound on |p_tr(fp32) - p_tr| per node and example, propagated down the tree.  A softmax
+    probability in fp32 carries a relative error kappa <= (8X + 14) u: the exponent x_j - max x, with x = R / tau
+    rounded and |x| <= X, is off by <= 4X u in absolute terms, expf adds 2 ulp, the sum of <= 8 terms 8u, the
+    reciprocal and product 2u.  Then p_tr[i] = q p + eps fl[i] with q = p_tr[par] - eps fl[par] gives
+      E[i] = p (E[par] + u eps fl[par] + u q) + q p (kappa + u) + u eps fl[i] + u p_tr[i]."""
+    kappa = (8 * X + 14) * U
+    eps32, n = float(np.float32(eps)), len(t['parent'])
+    E = [torch.zeros_like(ref['p_tr'][0])] * n
+    for i in range(1, n):
+        par = int(t['parent'][i])
+        if t['n_sinks'][par] < 2:
+            E[i] = E[par]
+            continue
+        p = ref['sm'][int(t['sw'][par])][:, int(t['sink_idx'][i])]
+        fp, fi = eps32 * float(t['floor'][par]), eps32 * float(t['floor'][i])
+        q = ref['p_tr'][par] - fp
+        E[i] = p * (E[par] + U * fp + U * q) + q * p * (kappa + U) + U * fi + U * ref['p_tr'][i]
+    return torch.stack(E), kappa
+
+
+def _depth(t):
+    d = [0] * len(t['parent'])
+    for i in range(1, len(d)):
+        par = int(t['parent'][i])
+        d[i] = d[par] + (1 if t['n_sinks'][par] >= 2 else 0)
+    return max(d)
+
+
+def route_bounds(t, ref, mode, tau, eps, R, E, kappa):
+    """Bounds on dR (per element) and c_data (per example), from the float64 intermediates of route_ref:
+      * actor: gs_j = g[child_j] (p_tr - eps fl) and dR_j = sm_j (gs_j - sum_k sm_k gs_k) / tau + 2 k_dec p_tr R_j / B.
+        g (sums of <= n products of <= D probabilities, all terms >= 0) is good to K_g u = (D kappa / u + n + 4) u
+        relative, so |d dR_j| <= (K_g + kappa / u + 8) u sm_j (|gs_j| + sum_k sm_k |gs_k|) / tau
+        + sm_j (|g_j| + sum_k sm_k |g_k|) (E + 2u p_tr) / tau + |k_dec term| (E / p_tr + 6u);
+      * critic: the target (a sum of <= n terms >= 0) is good to (n + 2) u relative, so
+        |d dR_j| <= 2 k_cre p_tr / B ((n + 3) u (|R_j| + target_j)) + |dR_j| (E / p_tr + 6u);
+      * c_data = sum_i p_tr w_i: |d| <= sum_i (E w_i + p_tr dw_i) + (n + 4) u sum_i p_tr w_i, with dw the bound of
+        each weight (local cost: 3u; k_dec |R|^2: 12u; critic regression: 2 (n + 4) u k_cre sum_j (|R_j| + t_j)^2)."""
+    n, D = len(t['parent']), _depth(t)
+    tau32, B = float(np.float32(tau)), R[0].shape[0] if R else 1
+    Kg = D * kappa / U + n + 4
+    k_dec, k_cre = float(np.float32(mode.get('k_dec', 0.0))), float(np.float32(mode.get('k_cre', 0.0)))
+    eps32 = float(np.float32(eps))
+    bdR, terms, dterms = [None] * len(R), [], []
+    p = ref['p_tr']
+    for i in range(n):
+        ns = int(t['n_sinks'][i])
+        if ns < 2:
+            continue
+        s, ks = int(t['sw'][i]), list(t['child'][i, :ns])
+        r = R[s].double()
+        pt, Ei = p[i][:, None], E[i][:, None]
+        if not mode['critic']:
+            sm = ref['sm'][s]
+            gc = ref['g'][ks].T
+            gs = gc * (pt - eps32 * float(t['floor'][i]))
+            a1 = sm * (gs.abs() + (sm * gs.abs()).sum(1, keepdim=True)) / tau32
+            a2 = sm * (gc.abs() + (sm * gc.abs()).sum(1, keepdim=True)) / tau32
+            kd = (2 * k_dec * pt * r / B).abs()
+            bdR[s] = (Kg + kappa / U + 8) * U * a1 + a2 * (Ei + 2 * U * pt) + kd * (Ei / pt + 6 * U)
+            terms.append(k_dec * p[i] * (r ** 2).sum(1)); dterms.append(E[i] * k_dec * (r ** 2).sum(1) + 12 * U * terms[-1])
+        else:
+            tg = ref['tgt'][s]
+            bdR[s] = 2 * k_cre * pt / B * (n + 3) * U * (r.abs() + tg) + ref['dR'][s].abs() * (Ei / pt + 6 * U)
+            w = k_cre * ((r.abs() + tg) ** 2).sum(1)
+            terms.append(p[i] * w); dterms.append(E[i] * w + p[i] * 2 * (n + 4) * U * w)
+    return bdR, terms, dterms
+
+
+def c_data_bound(t, ref, mode, ce, kc, E, terms, dterms):
+    n = len(t['parent'])
+    ops = torch.tensor(t['ops'], dtype=torch.float64, device='cuda')
+    tot, dtot = list(terms), list(dterms)
+    for i in range(n):
+        e = ce[int(t['err'][i])].double() if t['err'][i] >= 0 else 0.0
+        w = e + (0.0 if mode['critic'] else kc * ops[i])
+        w = w if torch.is_tensor(w) else torch.full_like(ref['p_tr'][i], w)
+        tot.append(ref['p_tr'][i] * w); dtot.append(E[i] * w + 3 * U * ref['p_tr'][i] * w)
+    return sum(dtot) + (n + 4) * U * sum(tot)
+
+
+def _ratio(got, ref, bound):
+    return float(((got.double() - ref).abs() / bound.clamp_min(1e-300)).max())
+
+
+@pytest.mark.parametrize('B', BATCHES)
+@pytest.mark.parametrize('logits', list(LOGITS))
+@pytest.mark.parametrize('tree', [(11, 2), (11, 4), (11, 8), (32, 2), (32, 4), (32, 8), (33, 2), (33, 4), (33, 8),
+                                  'ac_tree', 'cr_tree'])
+def test_route_walks_at_scale(tree, logits, B):
+    """mpnn_route_fwd / _bwd on random trees of 11, 32 (staged walk) and 33 nodes (global walk) whose widest switch
+    has 2, 4 or 8 sinks (every NS instantiation of the staged walk), and on the 95-node tables of the full-size
+    ac_tree and cr_tree (global walk), against route_ref: actor with k_dec, actor with a per-example k_cpt,
+    critic plain, optimistic and use_cls_err; random logits (tau 0.6), integer logits (ties, tau 1) and logits of
+    about +-50 at tau = 0.1; eps = 1e-6 and 0.1 (at 1e-6 the floor terms are below every tolerance, at 0.1 they are
+    not).  p_ev and dec are exact; p_tr, dR and c_data are held to the bounds of p_tr_bound and route_bounds,
+    which scale with X = max |R| / tau (2 ulp of a softmax exponent of 1000 is 1e-4 relative)."""
+    t = tree_of(tree)
+    n = len(t['parent'])
+    assert (n > RT_STAGED_MAX) == (tree == 'ac_tree' or tree == 'cr_tree' or tree[0] > 32)
+    tau = LOGITS[logits]
+    R, ce, dc, kv = route_inputs(t, B, logits, 7100 + n + B + len(logits))
+    X = max(float(r.abs().max()) for r in R) / float(np.float32(tau))
+    worst = {}
+    for eps in (1e-6, 0.1):
+        for name, m in MODES.items():
+            k_cpt = kv if m.get('vec') else None
+            got = route_launch(t, R, tau, eps, B, ce, dc, k_cpt, m['critic'], m.get('k_dec', 0.0), m.get('k_cre', 0.0),
+                               m.get('optimistic', 0), m.get('use_cls_err', 0))
+            ref = route_ref(t, R, tau, eps, c_err=ce, d_cor=dc, k_cpt=kv if m.get('vec') else 4e-9,
+                            critic=bool(m['critic']), k_dec=m.get('k_dec', 0.0), k_cre=m.get('k_cre', 0.0),
+                            optimistic=bool(m.get('optimistic')), use_cls_err=bool(m.get('use_cls_err')))
+            assert torch.equal(got['p_ev'].double(), ref['p_ev']), name
+            assert torch.equal(got['dec'][:len(R)].long(), ref['dec']), name
+            E, kappa = p_tr_bound(t, ref, tau, eps, X)
+            bdR, terms, dterms = route_bounds(t, ref, m, tau, eps, R, E, kappa)
+            kc = kv.double() if m.get('vec') else float(np.float32(4e-9))
+            bc = c_data_bound(t, ref, m, ce, kc, E, terms, dterms)
+            r = dict(p_tr=_ratio(got['p_tr'], ref['p_tr'], E + 1e-300),
+                     dR=max(_ratio(a, b, c) for a, b, c in zip(got['dR'], ref['dR'], bdR)),
+                     c_data=_ratio(got['c_data'], ref['c_data'], bc))
+            for k, v in r.items():
+                worst[k] = max(worst.get(k, 0.0), v)
+            assert max(r.values()) <= 1.0, (name, eps, r)
+    print('route %s n=%d B=%d %s (X = %.0f): worst |err| / bound over 2 eps x 5 modes: p_tr %.2f, dR %.2f, '
+          'c_data %.2f (tol 1 each); p_ev, dec exact' % (tree, n, B, logits, X, worst['p_tr'], worst['dR'],
+                                                        worst['c_data']))
+
+
+@pytest.mark.parametrize('tree', [(11, 2), (11, 4), (11, 8), (32, 2), (32, 4), (32, 8), 'ac_chain'])
+@pytest.mark.parametrize('logits', ['normal', 'sharp'])
+def test_staged_walk_equals_global_walk_bit_for_bit(tree, logits):
+    """A tree of <= 32 nodes runs the staged walk; the same tree padded past 32 nodes with a chain of 1-sink
+    nodes below its last node (ops 0, err -1) runs the global walk.  The padding changes no original node's
+    values and only adds exact zeros to c_data, and the two walks do the same arithmetic in the same order, so
+    p_tr, p_ev, dec, dR and c_data must agree bit for bit, in every mode and at both eps."""
+    B = 4097
+    t = tree_of(tree)
+    n = len(t['parent'])
+    assert n <= RT_STAGED_MAX
+    tp = pad_tree(t, 40)
+    tau = LOGITS[logits]
+    R, ce, dc, kv = route_inputs(t, B, logits, 7300 + n)
+    for eps in (1e-6, 0.1):
+        for name, m in MODES.items():
+            a = [route_launch(x, R, tau, eps, B, ce, dc, kv if m.get('vec') else None, m['critic'],
+                              m.get('k_dec', 0.0), m.get('k_cre', 0.0), m.get('optimistic', 0),
+                              m.get('use_cls_err', 0)) for x in (t, tp)]
+            st, gl = a
+            for k in ('p_tr', 'p_ev'):
+                assert torch.equal(st[k], gl[k][:n]), (name, eps, k)
+                assert torch.equal(gl[k][n:], gl[k][n - 1:n].expand(40 - n, B)), (name, eps, k)
+            assert torch.equal(st['dec'], gl['dec']), (name, eps)
+            assert torch.equal(st['c_data'], gl['c_data']), (name, eps)
+            for x, y in zip(st['dR'], gl['dR']):
+                assert torch.equal(x, y), (name, eps)
+    print('staged vs global walk %s %s: p_tr, p_ev, dec, dR, c_data bit-identical (2 eps x 5 modes)' % (tree, logits))
+
+
+def test_first_argmax_on_the_device():
+    from oracle.torch_ref import first_argmax
+    x = torch.tensor([[0., 0., 0.], [1., 3., 3.], [2., 1., 2.]], device='cuda')
+    assert first_argmax(x, 1).tolist() == [0, 1, 0]
+
+
+# --------------------------------------------------------------------------- #
+# node moments and path compaction on the 95-node walk
+# --------------------------------------------------------------------------- #
+@pytest.mark.parametrize('B', [1, 127] + list(BATCHES) + [BIG])
+def test_node_moments_and_compact_paths_on_the_tree_walk(B):
+    """p_tr and p_ev of the global walk on the ac_tree tables (random logits, eps 0.1) into mpnn_node_moments and
+    mpnn_compact_paths.  Moments: each thread sums ceil(B / 256) terms, then 5 shuffle levels and 8 warp partials,
+    all terms >= 0, so |d sum| <= (ceil(B / 256) + 13) u sum (+ u for p^2, + u for the division by B), against
+    float64 sums of the same fp32 p_tr.  Index lists and counts: exact, ascending."""
+    t = tree_of('ac_tree')
+    n = len(t['parent'])
+    R, _, _, _ = route_inputs(t, B, 'normal', 7500 + B)
+    o = route_launch(t, R, 0.6, 0.1, B, bwd=False)
+    stats = torch.full((n, 2), math.nan, device='cuda')
+    L().node_moments(vp(o['p_tr']), n, B, vp(stats), None)
+    idx = torch.full((n, B), -1, dtype=torch.int32, device='cuda')
+    cnt = torch.full((n,), -1, dtype=torch.int32, device='cuda')
+    L().compact_paths(vp(o['p_ev']), n, B, vp(idx), vp(cnt), None)
+    torch.cuda.synchronize()
+    p = o['p_tr'].double()
+    ref = torch.stack([(p ** 2).mean(1), p.mean(1)], 1)
+    k = -(-B // 256) + 13
+    tol = torch.tensor([k + 3, k + 2], dtype=torch.float64, device='cuda') * U
+    e = ((stats.double() - ref).abs() / ref).max(0).values
+    print('node_moments B=%d: mean p^2 %.2e (tol %.1e), mean p %.2e (tol %.1e); compaction exact'
+          % (B, e[0], tol[0], e[1], tol[1]))
+    assert bool((e <= tol).all())
+    assert int(o['p_ev'][0].sum()) == B
+    for i in range(n):
+        want = torch.nonzero(o['p_ev'][i] > 0.5).flatten()
+        assert int(cnt[i]) == want.numel()
+        assert torch.equal(idx[i, :want.numel()].long(), want)
+
+
+
+# --------------------------------------------------------------------------- #
+# error layers: softmax + cross-entropy, squared error, superclass targets
+# --------------------------------------------------------------------------- #
+def logits_rows(g, B, n, ldz):
+    """[B][ldz] logits (columns >= n hold garbage the kernels must not read): normal * 3, every 16th row all equal
+    (ties to the first class), every 16th row (offset 5) of +-80 values; one-hot labels [B][n]"""
+    Z = 3 * torch.randn((B, ldz), generator=g, device='cuda')
+    Z[:, n:] = 1e30
+    Z[::16, :n] = 0.25
+    s = torch.randint(0, 2, (B, n), generator=g, device='cuda').float() * 160 - 80
+    Z[5::16, :n] = s[5::16]
+    y = Fn.one_hot(torch.randint(0, n, (B,), generator=g, device='cuda'), n).float()
+    return Z.contiguous(), y
+
+
+def planes_with_sentinel(B, Balloc):
+    """two bf16 planes [2][Balloc][8]: rows < B hold 7 (every one must be written), rows B .. Balloc zero, as the
+    engine allocates them (the kernels leave those rows alone, and the head GEMMs read them as zero rows)"""
+    t = torch.zeros((2, Balloc, 8), dtype=torch.bfloat16, device='cuda')
+    t[:, :B] = 7.0
+    return t
+
+
+def softmax_ce_ref(z, y, eps, n):
+    """float64 softmax and c_err of fp32 operands (eps and eps / n as the kernel rounds them)"""
+    p = torch.softmax(z, 1)
+    a = float(np.float32(np.float32(eps) / np.float32(n))) + float(np.float32(1 - np.float32(eps))) * p
+    return p, -(y.double() * torch.log(a)).sum(1)
+
+
+@pytest.mark.parametrize('B', list(BATCHES) + [BIG])
+@pytest.mark.parametrize('n', [2, 10, 16, 17, 32])
+@pytest.mark.parametrize('ldz', ['n', 32])
+def test_softmax_ce_at_scale(B, n, ldz):
+    """mpnn_softmax_ce_fwd / _bwd with 16 (n <= 16) and 32 lanes per example, row stride n or 32 (the head GEMM's
+    row), eps 1e-6 and 0.1, a per-example coef.  With m = max_j |z_j - max z| of a row, every fp32 probability of
+    the row is good to kappa = (m + n + 5) u relative (exponent rounding m u, expf 2 ulp, sum n u, reciprocal and
+    product 2u), so
+      prob:  |d p_j| <= kappa p_j (+ 2^-126 for results in the subnormal range);
+      c_err: -log(eps/n + (1-eps) p_y): |d| <= kappa + 4u + u |c_err|;
+      d_cor: exact, the reference argmax taken from the kernel's own prob (checked above);
+      dZ:    k p_j (g_j - sum_k p_k g_k), g = dc/dp: |d| <= (3 kappa + (n + 12) u) k p_j (|g_j| + |sum_k p_k g_k|),
+             against float64 autograd of sum_b k_b c_err_b from the logits;
+      dZp:   the bf16 rounding of the kernel's own dZ, exactly, columns n .. 16 zero, rows B .. Balloc still zero;
+      dbias: float atomics of ~B / 8 CTA partial sums (each of 8 rows): |d| <= sum_b |d dZ| + (B / 8 + 8) u
+             sum_b |dZ|."""
+    ldz = n if ldz == 'n' else ldz
+    g = gen(8100 + B + n + ldz)
+    Balloc = ru(B, 128)
+    Z, y = logits_rows(g, B, n, ldz)
+    coef = torch.rand(B, generator=g, device='cuda')
+    worst = {}
+    for eps in (1e-6, 0.1):
+        prob = torch.full((B, n), math.nan, device='cuda')
+        ce = torch.full((B,), math.nan, device='cuda'); dc = torch.full((B,), math.nan, device='cuda')
+        L().softmax_ce_fwd(vp(Z), ldz, vp(y), B, n, eps, vp(prob), vp(ce), vp(dc), None)
+        dZ = torch.full((B, n), math.nan, device='cuda')
+        dZp = planes_with_sentinel(B, Balloc) if n <= 16 else None
+        dbias = torch.zeros(n, device='cuda') if n <= 16 else None
+        L().softmax_ce_bwd(vp(prob), vp(y), B, n, eps, vp(coef), 1.0 / B, vp(dZ), vp(dZp), Balloc, vp(dbias), None)
+        torch.cuda.synchronize()
+        z = Z[:, :n].double().requires_grad_(True)
+        p, c = softmax_ce_ref(z, y, eps, n)
+        k = coef.double() * float(np.float32(1.0 / B))
+        (c * k).sum().backward()
+        zd = z.detach()
+        kappa = ((zd - zd.max(1, keepdim=True).values).abs().max(1, keepdim=True).values + n + 5) * U
+        e_p = _ratio(prob, p.detach(), kappa * p.detach() + 2.0 ** -126)
+        e_c = _ratio(ce, c.detach(), kappa[:, 0] + 4 * U + U * c.detach().abs())
+        from oracle.torch_ref import first_argmax
+        assert torch.equal(dc, (first_argmax(prob, 1) == first_argmax(y, 1)).float())
+        pd = p.detach()
+        a = float(np.float32(np.float32(eps) / np.float32(n))) + float(np.float32(1 - np.float32(eps))) * pd
+        gr = -y.double() * float(np.float32(1 - np.float32(eps))) / a
+        dot = (pd * gr).sum(1, keepdim=True)
+        bz = (3 * kappa + (n + 12) * U) * k[:, None] * pd * (gr.abs() + dot.abs()) + 2.0 ** -126
+        e_z = _ratio(dZ, z.grad, bz)
+        r = dict(prob=e_p, c_err=e_c, dZ=e_z)
+        if n <= 16:
+            assert torch.equal(from_feat_t(dZp, B)[:, :n], dZ.to(torch.bfloat16))
+            assert not from_feat_t(dZp, B)[:, n:].float().any() and not dZp[:, B:].float().any()
+            bb = bz.sum(0) + (B / 8 + 8) * U * z.grad.abs().sum(0)
+            r['dbias'] = _ratio(dbias, z.grad.sum(0), bb)
+        for kk, v in r.items():
+            worst[kk] = max(worst.get(kk, 0.0), v)
+        assert max(r.values()) <= 1.0, (eps, r)
+    print('softmax_ce B=%d n=%d ldz=%d: worst |err| / bound over eps 1e-6, 0.1: %s (tol 1 each); d_cor%s exact'
+          % (B, n, ldz, ', '.join('%s %.2f' % kv for kv in worst.items()), ', dZp' if n <= 16 else ''))
+
+
+@pytest.mark.parametrize('B', list(BATCHES) + [BIG])
+@pytest.mark.parametrize('n', [2, 10, 16, 17, 32])
+@pytest.mark.parametrize('ldz', ['n', 32])
+def test_squared_err_at_scale(B, n, ldz):
+    """mpnn_squared_err_fwd / _bwd on integer-valued x (ties everywhere) and targets with ties (every 4th row of
+    y all zero, every 4th (offset 1) with two ones, the rest one-hot): out an exact copy of x, d_cor exact (first
+    maximum of x against first maximum of y), c_err = sum (x - y)^2 (an fma chain of n terms: (n + 2) u relative,
+    all terms >= 0), dZ = 2 k (x - y) (2u), dZp exact (bf16 of the kernel's dZ), dbias as in test_softmax_ce_at_scale."""
+    ldz = n if ldz == 'n' else ldz
+    g = gen(8300 + B + n + ldz)
+    Balloc = ru(B, 128)
+    Z = ints(g, (B, ldz), -2, 3)
+    Z[:, n:] = 1e30
+    y = Fn.one_hot(torch.randint(0, n, (B,), generator=g, device='cuda'), n).float()
+    y[::4] = 0
+    y[1::4, 0] = 1
+    y[1::4, n - 1] = 1
+    coef = torch.rand(B, generator=g, device='cuda')
+    out = torch.full((B, n), math.nan, device='cuda')
+    ce = torch.full((B,), math.nan, device='cuda'); dc = torch.full((B,), math.nan, device='cuda')
+    L().squared_err_fwd(vp(Z), ldz, vp(y), B, n, vp(out), vp(ce), vp(dc), None)
+    dZ = torch.full((B, n), math.nan, device='cuda')
+    dZp = planes_with_sentinel(B, Balloc) if n <= 16 else None
+    dbias = torch.zeros(n, device='cuda') if n <= 16 else None
+    L().squared_err_bwd(vp(out), vp(y), B, n, vp(coef), 1.0 / B, vp(dZ), vp(dZp), Balloc, vp(dbias), None)
+    torch.cuda.synchronize()
+    from oracle.torch_ref import first_argmax
+    x = Z[:, :n]
+    assert torch.equal(out, x)
+    assert torch.equal(dc, (first_argmax(x, 1) == first_argmax(y, 1)).float())
+    xd = x.double().requires_grad_(True)
+    c = ((xd - y.double()) ** 2).sum(1)
+    k = coef.double() * float(np.float32(1.0 / B))
+    (c * k).sum().backward()
+    e_c = _ratio(ce, c.detach(), (n + 2) * U * c.detach())
+    bz = 4 * U * xd.grad.abs()
+    e_z = _ratio(dZ, xd.grad, bz + 1e-300)
+    r = dict(c_err=e_c, dZ=e_z)
+    if n <= 16:
+        assert torch.equal(from_feat_t(dZp, B)[:, :n], dZ.to(torch.bfloat16))
+        assert not from_feat_t(dZp, B)[:, n:].float().any() and not dZp[:, B:].float().any()
+        r['dbias'] = _ratio(dbias, xd.grad.sum(0), bz.sum(0) + (B / 8 + 8) * U * xd.grad.abs().sum(0))
+    print('squared_err B=%d n=%d ldz=%d: %s (|err| / bound, tol 1 each); out, d_cor%s exact'
+          % (B, n, ldz, ', '.join('%s %.2f' % kv for kv in r.items()), ', dZp' if n <= 16 else ''))
+    assert max(r.values()) <= 1.0, r
+
+
+@pytest.mark.parametrize('B', [4097, BIG])
+@pytest.mark.parametrize('n_cls', [10, 100])
+@pytest.mark.parametrize('n_sup', [2, 5, 20])
+def test_superclass_targets_at_scale(B, n_cls, n_sup):
+    """mpnn_superclass_targets: y_sup = y @ w_cls.  With the 0/1 weights of a class -> superclass map (class j in
+    superclass j mod n_sup) every product is exact and the result must be too; with random weights it is an fma
+    chain of n_cls terms, |d| <= n_cls u sum_j |y_j w_jk|.  Every 7th row of y is a soft target of multiples of 1/8
+(exact sums).  Then chained into mpnn_softmax_ce_fwd with n = n_sup,
+    as the engine runs a SuperclassCrossEntropyError leaf: c_err and d_cor against the float64 restatement on
+    the exact targets (bounds of test_softmax_ce_at_scale)."""
+    g = gen(8500 + B + n_cls + n_sup)
+    y = Fn.one_hot(torch.randint(0, n_cls, (B,), generator=g, device='cuda'), n_cls).float()
+    y[::7] = torch.randint(0, 9, (len(range(0, B, 7)), n_cls), generator=g, device='cuda') / 8.0   # soft rows (dyadic)
+    w01 = torch.eye(n_sup, device='cuda')[torch.arange(n_cls, device='cuda') % n_sup].contiguous()
+    wr = torch.rand((n_cls, n_sup), generator=g, device='cuda')
+    outs = []
+    for w in (w01, wr):
+        ys = torch.full((B, n_sup), math.nan, device='cuda')
+        L().superclass_targets(vp(y), vp(w), B, n_cls, n_sup, vp(ys), None)
+        outs.append(ys)
+    Z, _ = logits_rows(g, B, n_sup, 32)
+    prob = torch.zeros((B, n_sup), device='cuda'); ce = torch.zeros(B, device='cuda'); dc = torch.zeros(B, device='cuda')
+    L().softmax_ce_fwd(vp(Z), 32, vp(outs[0]), B, n_sup, 1e-6, vp(prob), vp(ce), vp(dc), None)
+    torch.cuda.synchronize()
+    ref01 = y.double() @ w01.double()
+    assert torch.equal(outs[0].double(), ref01)
+    refr = y.double() @ wr.double()
+    e = _ratio(outs[1], refr, n_cls * U * (y.double().abs() @ wr.double().abs()))
+    from oracle.torch_ref import first_argmax
+    z = Z[:, :n_sup].double()
+    p, c = softmax_ce_ref(z, ref01, 1e-6, n_sup)
+    kappa = ((z - z.max(1, keepdim=True).values).abs().max(1).values + n_sup + 5) * U
+    # c_err = -sum_k y_k log(a_k) with soft targets: |d| <= sum_k y_k (kappa + 4u + u |log a_k|)
+    a = float(np.float32(np.float32(1e-6) / np.float32(n_sup))) + float(np.float32(1 - np.float32(1e-6))) * p
+    bc = (ref01 * (kappa[:, None] + 4 * U + U * torch.log(a).abs())).sum(1) + n_sup * U * c.abs()
+    e_c = _ratio(ce, c, bc + 1e-300)
+    assert torch.equal(dc, (first_argmax(prob, 1) == first_argmax(outs[0], 1)).float())
+    print('superclass_targets B=%d n_cls=%d n_sup=%d: 0/1 weights exact, random weights %.2f of the bound, '
+          'chained c_err %.2f of the bound, d_cor exact' % (B, n_cls, n_sup, e, e_c))
+    assert e <= 1.0 and e_c <= 1.0
+
+
+
+# --------------------------------------------------------------------------- #
+# compaction copies and the optimiser step
+# --------------------------------------------------------------------------- #
+CAP = 4096
+
+
+@pytest.mark.parametrize('dt', [F32, BF16])
+@pytest.mark.parametrize('H,C', [(32, 16), (16, 32), (8, 64), (4, 128)])
+def test_gather_scatter_images_at_scale(H, C, dt):
+    """mpnn_gather_images / mpnn_scatter_add_images between planes tensors of capacity 4096 at every stage
+    geometry, with counts 0, 1, 4095 and 4096 (at 32x32x16 the capped grid of 148*16 CTAs makes 15 grid-stride
+    passes).  Gather: destination image j is the whole S-row block of source image idx[j], the rest of the
+    destination untouched.  Scatter-add into a destination that is not zero: block idx[j] += block j, one fp32
+    addition rounded once to the storage type, the rest untouched.  All exact."""
+    g = gen(8700 + H + dt)
+    geo = Geo(CAP, H, H)
+    KG, S = C // 8, geo.S
+    src = to_planes_t(rnd(g, (CAP, H, H, C), dt), geo).to(TD[dt])
+    base = to_planes_t(rnd(g, (CAP, H, H, C), dt), geo).to(TD[dt])
+    blk = lambda t: t[:, geo.G:geo.G + CAP * S].view(KG, CAP, S, 8)
+    for count in (0, 1, CAP - 1, CAP):
+        idx = torch.randperm(CAP, generator=g, device='cuda')[:count].sort().values.int()
+        idx_full = torch.zeros(CAP, dtype=torch.int32, device='cuda')
+        idx_full[:count] = idx
+        cnt = torch.tensor([count], dtype=torch.int32, device='cuda')
+        dst = torch.full_like(src, 3.0)
+        L().gather_images(vp(src), CAP, geo.P, vp(idx_full), vp(cnt), vp(dst), CAP, geo.P, C, H, H, geo.G, dt, None)
+        acc = base.clone()
+        L().scatter_add_images(vp(src), CAP, geo.P, vp(idx_full), vp(cnt), vp(acc), CAP, geo.P, C, H, H, geo.G, dt, None)
+        torch.cuda.synchronize()
+        il = idx.long()
+        want = torch.full_like(src, 3.0)
+        blk(want)[:, :count] = blk(src)[:, il]
+        assert torch.equal(dst, want), count
+        want = base.clone()
+        blk(want)[:, il] = (blk(base)[:, il].float() + blk(src)[:, :count].float()).to(TD[dt])
+        assert torch.equal(acc, want), count
+    print('gather / scatter-add %dx%dx%d %s, counts 0, 1, 4095, 4096: exact (tol 0)' % (H, H, C, 'fp32' if dt == F32 else 'bf16'))
+
+
+@pytest.mark.parametrize('net', ['ac_chain', 'ac_tree'])
+@pytest.mark.parametrize('talr,stats', [(0, False), (1, False), (0, True), (1, True)])
+@pytest.mark.parametrize('gscale', [1.0, 0.125])
+def test_talr_momentum_step_at_scale(net, talr, stats, gscale):
+    """mpnn_talr_momentum_step over the parameter buffer of the full-size net (n_theta 680,826 in 178 segments for
+    ac_chain, 5,010,238 in 917 for ac_tree: the grid of 148*8 CTAs of 256 threads makes up to 17 grid-stride
+    passes, and every segment boundary is crossed) against a float64 restatement of csrc/optim.cu element by
+    element:  coef = m1 gs, scale = mult / sqrt(m2 gs) (talr, node stats present), g = (grad gs + 2 l2 coef theta)
+    scale, a = mu a + g, theta -= lr a.  Each fp32 operation rounds once, so |d a| <= 10 u (mu |a| + |g terms|)
+    and |d theta| <= lr (|d a| + 2u |a|) + 2u |theta|: the last rounding alone reaches u |theta| at the bottom of
+    a binade (measured: 0.99 u |theta|), the second u leaves room for everything of second order."""
+    _, n_theta, n_nodes, seg = _plan_of(net)
+    g = gen(8900 + n_theta % 1000 + 10 * talr + int(stats) + int(8 * gscale))
+    seg = {k: v.cuda() for k, v in seg.items()}
+    n_seg = seg['seg_node'].numel()
+    th = torch.randn(n_theta, generator=g, device='cuda')
+    gr = torch.randn(n_theta, generator=g, device='cuda')
+    acc = torch.randn(n_theta, generator=g, device='cuda')
+    m2 = 0.01 + 0.5 * torch.rand(n_nodes, generator=g, device='cuda')
+    m1 = m2.sqrt() + (1 - m2.sqrt()) * torch.rand(n_nodes, generator=g, device='cuda')
+    st = (torch.stack([m2, m1], 1) / gscale).contiguous() if stats else None     # moments ride in the scaled tail
+    hyp = torch.zeros(8, device='cuda')
+    hyp[0], hyp[1], hyp[5] = 0.05, 0.9, gscale
+    TH, A = th.clone(), acc.clone()
+    L().talr_momentum_step(vp(TH), vp(gr), vp(A), n_theta, vp(seg['seg_start']), vp(seg['seg_node']),
+                           vp(seg['seg_mult']), vp(seg['seg_l2']), n_seg, vp(st), talr, vp(hyp), None)
+    torch.cuda.synchronize()
+    sid = torch.repeat_interleave(torch.arange(n_seg, device='cuda'), (seg['seg_start'][1:] - seg['seg_start'][:-1]).long())
+    node = seg['seg_node'].long()[sid]
+    mult, l2 = seg['seg_mult'].double()[sid], seg['seg_l2'].double()[sid]
+    gs, lr, mu = float(np.float32(gscale)), float(np.float32(0.05)), float(np.float32(0.9))
+    if stats:
+        coef = st[:, 1].double()[node] * gs
+        scale = mult / torch.sqrt(st[:, 0].double()[node] * gs) if talr else mult
+    else:
+        coef, scale = torch.ones_like(mult), mult
+    t0, t1 = gr.double() * gs, 2 * l2 * coef * th.double()
+    a = mu * acc.double() + (t0 + t1) * scale
+    thn = th.double() - lr * a
+    ba = 10 * U * (mu * acc.double().abs() + (t0.abs() + t1.abs()) * scale.abs())
+    bt = lr * (ba + 2 * U * a.abs()) + 2 * U * thn.abs()
+    e = (_ratio(A, a, ba + 1e-300), _ratio(TH, thn, bt + 1e-300))
+    print('talr_momentum_step %s n=%d talr=%d stats=%s gscale=%g: accum %.2f, theta %.2f of the bound (tol 1)'
+          % (net, n_theta, talr, stats, gscale, *e))
+    assert max(e) <= 1.0

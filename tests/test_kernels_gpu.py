@@ -1012,7 +1012,6 @@ def test_talr_momentum_step():
                                      ('cr', dict(k_cpt=4e-9)), ('cr', dict(k_cpt=4e-9, optimistic=True))])
 def test_route_fwd_bwd(kind, hy):
     from util import tiny_net
-    from lib.net_types import n_leaves
     B, tau, eps = 50, 0.6, 1e-6
     net = tiny_net(kind, **hy).configure(precision='fp32')
     eng = net._get_engine()
@@ -1034,51 +1033,20 @@ def test_route_fwd_bwd(kind, hy):
     plan.fwd_ops[-1]()          # route_fwd
     plan.bwd_ops[0]()           # route_bwd
     torch.cuda.synchronize()
-    # ---- reference with autograd (float64)
-    Rt = {i: torch.tensor(r, dtype=torch.float64, requires_grad=True) for i, r in Rs.items()}
-    root_leaves = n_leaves(net.root)
-    fl = [eps * n_leaves(nd.layer) / root_leaves for nd in nodes]
-    ops = [nd.layer.n_ops + (nd.router.n_ops if nd.router is not None else 0) for nd in nodes]
-    p_tr = [None] * len(nodes); p_ev = [None] * len(nodes)
-    p_tr[0] = torch.ones(B, dtype=torch.float64); p_ev[0] = torch.ones(B, dtype=torch.float64)
-    for nd in nodes[1:]:
-        par = nodes[nd.parent]
-        if len(par.kids) < 2:
-            p_tr[nd.idx], p_ev[nd.idx] = p_tr[par.idx], p_ev[par.idx]
-        else:
-            r = Rt[par.idx]
-            sm = torch.softmax(r / tau, 1)
-            p_tr[nd.idx] = (p_tr[par.idx] - fl[par.idx]) * sm[:, nd.sink_idx] + fl[nd.idx]
-            p_ev[nd.idx] = p_ev[par.idx] * (torch.tensor(Rs[par.idx]).argmax(1) == nd.sink_idx)
-    k = hy['k_cpt']
-    cerr = lambda nd: torch.tensor(ce[nd.idx], dtype=torch.float64) if nd.idx in ce else torch.zeros(B, dtype=torch.float64)
-    if not critic:
-        tot = sum(p_tr[nd.idx] * (cerr(nd) + k * ops[nd.idx]) for nd in nodes)
-        tot = tot + sum(p_tr[nd.idx].detach() * 0.01 * (Rt[nd.idx] ** 2).sum(1) for nd in eng.switches)
-    else:
-        cev = [None] * len(nodes); cop = [None] * len(nodes); tot = 0
-        for nd in reversed(nodes):
-            base = cerr(nd) + k * ops[nd.idx]
-            if len(nd.kids) < 2:
-                cev[nd.idx] = base + sum(cev[c] for c in nd.kids)
-                cop[nd.idx] = base + sum(cop[c] for c in nd.kids)
-                cre = 0
-            else:
-                dec = torch.tensor(Rs[nd.idx]).argmax(1)
-                cev[nd.idx] = base + sum((dec == j) * cev[c] for j, c in enumerate(nd.kids))
-                cop[nd.idx] = base + torch.stack([cop[c] for c in nd.kids]).min(0).values
-                tg = cop if hy.get('optimistic') else cev
-                cre = 1e-3 * sum((Rt[nd.idx][:, j] + tg[c].detach()) ** 2 for j, c in enumerate(nd.kids))
-            tot = tot + p_tr[nd.idx].detach() * (cerr(nd) + cre)
-    tot.mean().backward()
+    # ---- float64 reference from the plan's tables (actor dR by autograd)
+    from util import route_ref, tree_tables
+    ref = route_ref(tree_tables(plan), [torch.from_numpy(Rs[nd.idx]) for nd in eng.switches], tau, eps,
+                    c_err=[torch.from_numpy(ce[nd.idx]) for nd in eng.regs], k_cpt=hy['k_cpt'], critic=critic,
+                    k_dec=0.0 if critic else 0.01, k_cre=1e-3 if critic else 0.0,
+                    optimistic=bool(hy.get('optimistic')))
     got_ptr = plan.p_tr.cpu().numpy()
     for nd in nodes:
-        np.testing.assert_allclose(got_ptr[nd.idx], p_tr[nd.idx].detach().numpy(), rtol=2e-5, atol=1e-9)
-        np.testing.assert_array_equal(plan.p_ev.cpu().numpy()[nd.idx], p_ev[nd.idx].numpy())
-    np.testing.assert_allclose(plan.c_data.cpu().numpy(), tot.detach().numpy(), rtol=2e-5)
-    for nd in eng.switches:
+        np.testing.assert_allclose(got_ptr[nd.idx], ref['p_tr'][nd.idx].numpy(), rtol=2e-5, atol=1e-9)
+        np.testing.assert_array_equal(plan.p_ev.cpu().numpy()[nd.idx], ref['p_ev'][nd.idx].numpy())
+    np.testing.assert_allclose(plan.c_data.cpu().numpy(), ref['c_data'].numpy(), rtol=2e-5)
+    for s, nd in enumerate(eng.switches):
         got = plan.rtr[nd.idx].dR.cpu().numpy()
-        assert rel_err(got, Rt[nd.idx].grad.numpy()) < 1e-4, nd.idx
+        assert rel_err(got, ref['dR'][s].numpy()) < 1e-4, nd.idx
 
 
 # --------------------------------------------------------------------------- #

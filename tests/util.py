@@ -266,3 +266,174 @@ def from_feat_t(t, B):
 
 def stencil_offsets(Wp):
     return [(t // 3 - 1) * Wp + (t % 3 - 1) for t in range(9)]
+
+
+# ---- routing tree tables (include/mpnn.h, "Tree tables") and a float64 restatement of both walks ---------- #
+RT_MAXS = 8             # sinks per switch (csrc/route.cu)
+
+
+def random_tree(rng, n_nodes, max_sinks):
+    """Random tables for mpnn_route_fwd / _bwd: n_nodes nodes in preorder, a mix of leaves, 1-sink chain nodes and
+    switches of 2 .. max_sinks sinks, at least one switch of exactly max_sinks sinks (the root).  Every leaf is a
+    classifier (err = its leaf slot), switches get slots in preorder, ops are positive, and
+    floor = n_leaves(i) / n_leaves(root) as the engine writes it.  NumPy arrays, keyed by the C argument names."""
+    assert 2 <= max_sinks <= RT_MAXS and n_nodes > max_sinks
+    kids = [[]]
+    open_, left = [0], n_nodes - 1
+    while left:
+        v = open_.pop(len(open_) - 1 - int(rng.integers(min(3, len(open_)))))     # mostly the newest: deep trees
+        if v == 0:
+            ns = max_sinks
+        else:
+            r = rng.random()
+            ns = 0 if r < 0.3 else 1 if r < 0.55 else int(rng.integers(2, max_sinks + 1))
+            ns = min(ns, left)
+            if ns == 0 and not open_:           # the last open node must not close the tree early
+                ns = 1
+        for _ in range(ns):
+            kids.append([])
+            kids[v].append(len(kids) - 1)
+            open_.append(len(kids) - 1)
+        left -= ns
+    order = []                                   # preorder relabelling
+
+    def walk(v):
+        order.append(v)
+        for c in kids[v]:
+            walk(c)
+    walk(0)
+    new = {v: i for i, v in enumerate(order)}
+    n = n_nodes
+    t = dict(parent=np.full(n, -1, np.int32), sink_idx=np.zeros(n, np.int32), n_sinks=np.zeros(n, np.int32),
+             child=np.full((n, RT_MAXS), -1, np.int32), floor=np.zeros(n, np.float32), sw=np.full(n, -1, np.int32),
+             ops=np.zeros(n, np.float32), err=np.full(n, -1, np.int32))
+    for v in order:
+        i = new[v]
+        t['n_sinks'][i] = len(kids[v])
+        for j, c in enumerate(kids[v]):
+            t['parent'][new[c]], t['sink_idx'][new[c]], t['child'][i, j] = i, j, new[c]
+    n_sw = n_err = 0
+    for i in range(n):
+        if t['n_sinks'][i] >= 2:
+            t['sw'][i], n_sw = n_sw, n_sw + 1
+        if t['n_sinks'][i] == 0:
+            t['err'][i], n_err = n_err, n_err + 1
+    leaves = np.zeros(n, np.int64)
+    for i in reversed(range(n)):
+        leaves[i] = 1 if t['n_sinks'][i] == 0 else sum(leaves[c] for c in t['child'][i, :t['n_sinks'][i]])
+    t['floor'][:] = leaves / leaves[0]
+    t['ops'][:] = rng.uniform(1e6, 3e8, n).astype(np.float32)
+    return t
+
+
+def tree_tables(plan):
+    """the routing tables of an engine plan (lib/engine.py _build_routing) as NumPy arrays, keyed as random_tree's"""
+    return {k: getattr(plan, 't_' + a).cpu().numpy() for k, a in (
+        ('parent', 'parent'), ('sink_idx', 'sink'), ('n_sinks', 'nsinks'), ('child', 'child'), ('floor', 'floor'),
+        ('sw', 'sw'), ('ops', 'ops'), ('err', 'err'))}
+
+
+def pad_tree(t, n_total):
+    """t with a chain of 1-sink nodes hung below its last node in preorder (a leaf) up to n_total nodes: ops 0,
+    err -1, so the padding changes no original node's p_tr, p_ev, c_ev or c_opt, and adds exact zeros to c_data.
+    The former last node keeps its err slot."""
+    n = len(t['parent'])
+    assert t['n_sinks'][n - 1] == 0 and n_total > n
+    p = {k: v.copy() for k, v in t.items()}
+    extra = n_total - n
+    for k in ('parent', 'sink_idx', 'n_sinks', 'floor', 'sw', 'ops', 'err'):
+        fill = {'parent': 0, 'sink_idx': 0, 'n_sinks': 1, 'floor': t['floor'][n - 1], 'sw': -1, 'ops': 0, 'err': -1}[k]
+        p[k] = np.concatenate([p[k], np.full(extra, fill, p[k].dtype)])
+    p['child'] = np.concatenate([p['child'], np.full((extra, RT_MAXS), -1, np.int32)])
+    for i in range(n - 1, n_total):
+        if i > n - 1:
+            p['parent'][i] = i - 1
+        if i < n_total - 1:
+            p['n_sinks'][i], p['child'][i, 0] = 1, i + 1
+    p['n_sinks'][n_total - 1] = 0
+    return p
+
+
+def _f32(v):
+    return float(np.float32(v))
+
+
+def route_ref(t, R, tau, eps, c_err=None, d_cor=None, k_cpt=0.0, critic=False, k_dec=0.0, k_cre=0.0,
+              optimistic=False, use_cls_err=False):
+    """Both routing walks of csrc/route.cu (lib/net_types.py:108-131 actor, :193-243 critic) in float64 torch, from
+    the tables alone, on the device of R.  R[slot]: [B][n_sinks] logits of each switch slot; c_err[leaf], d_cor[leaf]:
+    [B]; k_cpt: a number or a [B] vector.  The scalars are rounded to fp32 first, as the kernels receive them.
+      p_tr[i] = (p_tr[par] - eps floor[par]) softmax(R / tau)[sink_idx[i]] + eps floor[i]   below a switch,
+      p_ev[i] = p_ev[par] [first argmax R == sink_idx[i]],   dec[slot] = first argmax R.
+    Actor: c_data = sum_i p_tr (c_err + k_cpt ops) + sum_switches sg(p_tr) k_dec |R|^2, dR = d mean_b(c_data) / dR by
+    autograd; 'g' is the explicit dL/dp_tr of every node (the `gp` of the kernels), for error bounds.
+    Critic: c_ev / c_opt bottom-up (ce = 1 - d_cor with use_cls_err), dR = p_tr / B k_cre 2 (R + target) with
+    target = c_opt (optimistic) or c_ev of each sink, c_data = sum_i p_tr (c_err + k_cre sum_j (R_j + target_j)^2).
+    Returns a dict of p_tr, p_ev [n][B], dec [n_sw][B] (int64), c_data [B], dR [slot] and the intermediates."""
+    from oracle.torch_ref import first_argmax
+    import torch
+    L = {k: (v.tolist() if hasattr(v, 'tolist') else list(v)) for k, v in t.items()}
+    n = len(L['parent'])
+    dev = R[0].device if len(R) else (c_err[0].device if c_err else 'cpu')
+    B = R[0].shape[0] if len(R) else c_err[0].shape[0]
+    dt = torch.float64
+    tau, eps, k_dec, k_cre = _f32(tau), _f32(eps), _f32(k_dec), _f32(k_cre)
+    fl = [eps * _f32(f) for f in L['floor']]
+    ops = [_f32(o) for o in L['ops']]
+    kc = k_cpt.double() if hasattr(k_cpt, 'double') else _f32(k_cpt)
+    Rt = [r.detach().double().requires_grad_(not critic) for r in R]
+    sm = [torch.softmax(r / tau, 1) for r in Rt]
+    dec = [first_argmax(r.detach(), 1) for r in Rt]
+    one = torch.ones(B, dtype=dt, device=dev)
+    zero = torch.zeros(B, dtype=dt, device=dev)
+    p_tr, p_ev = [one] + [None] * (n - 1), [one] + [None] * (n - 1)
+    for i in range(1, n):
+        par = L['parent'][i]
+        if L['n_sinks'][par] >= 2:
+            s, si = L['sw'][par], L['sink_idx'][i]
+            p_tr[i] = (p_tr[par] - fl[par]) * sm[s][:, si] + fl[i]
+            p_ev[i] = p_ev[par] * (dec[s] == si).to(dt)
+        else:
+            p_tr[i], p_ev[i] = p_tr[par], p_ev[par]
+    ce = [c_err[L['err'][i]].double() if L['err'][i] >= 0 else zero for i in range(n)]
+    out = dict(sm=[s.detach() for s in sm], dec=torch.stack(dec) if dec else None)
+    if not critic:
+        local = [ce[i] + kc * ops[i] for i in range(n)]
+        tot = sum(p_tr[i] * local[i] for i in range(n))
+        for i in range(n):
+            if L['n_sinks'][i] >= 2:
+                tot = tot + p_tr[i].detach() * k_dec * (Rt[L['sw'][i]] ** 2).sum(1)
+        if Rt:
+            (tot.sum() / B).backward()
+        with torch.no_grad():
+            g = [(local[i] / B).detach().clone() for i in range(n)]
+            for i in range(n - 1, 0, -1):
+                par = L['parent'][i]
+                w = sm[L['sw'][par]][:, L['sink_idx'][i]].detach() if L['n_sinks'][par] >= 2 else 1.0
+                g[par] = g[par] + g[i] * w
+        out.update(dR=[r.grad for r in Rt], g=torch.stack(g), c_data=tot.detach())
+    else:
+        ce_loss = [(1.0 - d_cor[L['err'][i]].double()) if L['err'][i] >= 0 else zero for i in range(n)] \
+            if use_cls_err else ce
+        cev, cop, dR, tgt = [None] * n, [None] * n, [None] * len(R), [None] * len(R)
+        tot = zero
+        for i in range(n - 1, -1, -1):
+            base = ce_loss[i] + kc * ops[i]
+            ks = L['child'][i][:L['n_sinks'][i]]
+            cre = zero
+            if len(ks) < 2:
+                cev[i] = base + sum((cev[c] for c in ks), zero)
+                cop[i] = base + sum((cop[c] for c in ks), zero)
+            else:
+                s = L['sw'][i]
+                tg = torch.stack([(cop if optimistic else cev)[c] for c in ks], 1)
+                r = Rt[s]
+                dR[s] = p_tr[i][:, None] / B * k_cre * 2 * (r + tg)
+                tgt[s] = tg
+                cre = k_cre * ((r + tg) ** 2).sum(1)
+                cev[i] = base + torch.stack([cev[c] for c in ks], 1).gather(1, dec[s][:, None])[:, 0]
+                cop[i] = base + torch.stack([cop[c] for c in ks], 1).min(1).values
+            tot = tot + p_tr[i] * (ce[i] + cre)
+        out.update(dR=dR, tgt=tgt, c_ev=torch.stack(cev), c_opt=torch.stack(cop), c_data=tot)
+    out.update(p_tr=torch.stack([p.detach() for p in p_tr]), p_ev=torch.stack(p_ev))
+    return out
